@@ -70,7 +70,44 @@ def parse():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-side-tables", action="store_true", help="skip masked / C5 / multi-GPU C3 / C-entry rows")
     ap.add_argument("--no-cpu-big", action="store_true", help="reference arm: skip the extra 256^3 pass")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy (CUDA path)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "cuda":
+        ap.error("--dump-outputs applies to the CUDA path")
+    return args
+
+
+# voxels of the output volume that --dump-outputs writes: 16 MB of float32 values + 32 MB of float64 indices
+DUMP_SAMPLE = 1 << 22
+
+
+def dump_outputs(path, out, z0, shape, threshold, dist, world, rank, dev):
+    """--dump-outputs: what a caller of the timed step receives -- the post-vote score volume and the
+    saliency-cut threshold -- as DIR/out_sample.npy, DIR/out_sample_index.npy and DIR/threshold.npy.  The
+    volume is written at a fixed, seeded set of voxels (all of them when it has at most DUMP_SAMPLE), with
+    their flat z-y-x indices beside the values, so that two builds run with the same arguments can be
+    compared output for output.  `out` holds planes [z0, z0 + len(out)) of this rank."""
+    import torch
+    n = int(np.prod(shape))
+    if n <= DUMP_SAMPLE:
+        idx = np.arange(n, dtype=np.int64)
+    else:
+        idx = np.unique(np.random.default_rng(0).integers(0, n, DUMP_SAMPLE, dtype=np.int64))
+    lo = z0 * shape[1] * shape[2]
+    gidx = torch.from_numpy(idx).to(dev)
+    mine = (gidx >= lo) & (gidx < lo + out.numel())
+    bits = torch.zeros(len(idx), dtype=torch.int32, device=dev)
+    bits[mine] = out.reshape(-1).view(torch.int32)[gidx[mine] - lo]
+    if world > 1:
+        dist.all_reduce(bits)    # every voxel lies on exactly one rank: its bit pattern plus zeros, exact
+    if rank == 0:
+        os.makedirs(path, exist_ok=True)
+        np.save(os.path.join(path, "out_sample.npy"), bits.view(torch.float32).cpu().numpy())
+        np.save(os.path.join(path, "out_sample_index.npy"), idx.astype(np.float64))
+        np.save(os.path.join(path, "threshold.npy"), np.array([threshold], np.float64))
 
 
 class ClockSampler:
@@ -573,12 +610,16 @@ def main():
             dist.barrier()
         torch.cuda.synchronize()
 
+    last = {}
+
     def device_step():
         if world == 1:
             ctx.reset_stage_ms()
-            ctx.membrane(own, SIGMA, RATIO, visfd_b200.DECREASING_EIVALS, TV_BEST, True, TV_SIGMA, 4, SQ2, out=out)
+            r = ctx.membrane(own, SIGMA, RATIO, visfd_b200.DECREASING_EIVALS, TV_BEST, True, TV_SIGMA, 4, SQ2, out=out)
+            last["threshold"] = r["threshold"]
         else:
             pipe.run(own, out=out)
+            last["threshold"] = pipe.threshold
 
     def timed(fn, steps):
         ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -603,6 +644,8 @@ def main():
     ms_step = timed(device_step, args.steps)
     launches = ctx.launch_count() - l0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, out, z0, shape, last["threshold"], dist, world, rank, dev)
     stage = {k: ctx.stage_ms(k) for k in ("gauss", "ridge", "select", "compact", "tv")}   # last step, this rank
     n_voters = ctx.last_voter_count()
     lt = torch.tensor([launches], device=dev, dtype=torch.int64)
@@ -709,7 +752,7 @@ def main():
                 pipe.run(own, out=d_out, out_host=h_out)   # D2H chunk by chunk behind the voting kernels
                 torch.cuda.current_stream().synchronize()
         e2e_step()
-        e2e_ms = timed(e2e_step, max(1, min(args.steps, 2)))
+        e2e_ms = timed(e2e_step, args.steps)
         e2e = {"value": n_vox / (e2e_ms * 1e-3) / 1e9, "unit": "Gvoxel/s", "ms_per_step": e2e_ms,
                "h2d_bytes_per_step": int(4 * n_vox), "d2h_bytes_per_step": int(4 * n_vox),
                "call": "visfd_cuda_membrane(host pointers)" if world == 1 else

@@ -12,9 +12,21 @@ def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a B200 (run with -m gpu on the GPU box)")
 
 
+class GoldenVectors(dict):
+    """Name -> array, with the `files` list of an NpzFile."""
+    @property
+    def files(self):
+        return list(self)
+
+
 @pytest.fixture(scope="session")
 def golden():
-    return np.load(os.path.join(ROOT, "tests", "golden", "reference_vectors.npz"))
+    """tests/golden/reference_vectors*.npz (tests/golden/make_golden.py), kept in parts of less than 1 MB"""
+    out = GoldenVectors()
+    for name in ("reference_vectors.npz", "reference_vectors_blob_lists.npz", "reference_vectors_live.npz"):
+        with np.load(os.path.join(ROOT, "tests", "golden", name)) as part:
+            out.update((k, part[k]) for k in part.files)
+    return out
 
 
 @pytest.fixture(scope="session")

@@ -332,9 +332,55 @@ def main():
             len(nms_in), len(nms_out), len(cli2), len(out["bloblist_nms_sep"]), len(out["bloblist_nms_vol"]),
             len(out["bloblist_nms_inc"])))
 
-    path = os.path.join(HERE, "reference_vectors.npz")
-    np.savez_compressed(path, **out)
-    print("wrote", path, "%.1f KiB" % (os.path.getsize(path) / 1024), len(out), "arrays")
+    # ---- reference_vectors_live.npz: the reference's results for the inputs of the tests that also compare with
+    # oracle/_ref directly (test_*_live, test_*_vs_reference, test_*_is_the_reference, test_live_*); README.md in
+    # this directory says where the committed values came from ------------------------------------------------------
+    import test_blob_lists
+    import test_mrc_io
+    from visfd_b200.blobs import BlobLists
+    from visfd_b200.mrc import open_library
+    h, vox = test_mrc_io.live_case(open_library())
+    with tempfile.TemporaryDirectory() as td:
+        pth = os.path.join(td, "a.mrc")
+        ref_mrc.write(pth, h, vox)
+        out["live_mrc_out"] = np.frombuffer(open(pth, "rb").read(), np.uint8)
+        out["live_mrc_hdr"] = np.frombuffer(ref_mrc.read(pth)[0].as_bytes(), np.uint8)
+    ref_lists = BlobLists(ctypes.CDLL(os.path.join(ROOT, "oracle", "_ref", "libvisfd_ref.so")), "ref_blobs_")
+
+    def rows(src, kept):
+        """row numbers in src of the blobs kept, in their order"""
+        return np.array([np.flatnonzero(np.all(src == r, axis=1))[0] for r in kept], np.int64)
+
+    for n, b, bb, mask in test_blob_lists.live_cases():
+        for k, args in enumerate(test_blob_lists.LIVE_OVERLAP_ARGS):
+            out["live_blobs_%d_overlap%d" % (n, k)] = rows(b, ref_lists.discard_overlapping(b, *args))
+        out["live_blobs_%d_masked" % n] = rows(bb, ref_lists.discard_masked(bb, mask))
+
+    import test_oracle_golden
+    for trial, img, mask, regions in test_oracle_golden.random_draw_cases():
+        for subtract in (False, True):
+            d = ref.draw_regions(img, regions, mask=mask, negative_means_subtract=subtract)
+            out["live_draw_%d_%d" % (trial, subtract)] = np.where(d != img, d, np.float32(np.nan)).astype(np.float32)
+    for k, v in test_oracle_golden.port_live_outputs(ref).items():
+        out["live_port_" + k] = v
+    from util import sha256_of
+    for name, args, kw in test_oracle_golden.restatement_connect_calls(ref, out):
+        res = ref.label_connected(*args, **kw)
+        key = "live_connect_%s_" % name
+        out[key + "labels"], out[key + "n_clusters"] = res[0].astype(np.int16), np.int64(res[1])
+        if kw.get("want_direction"):
+            out[key + "direction_inside"] = res[2][res[0] >= 1]
+            out[key + "direction_sha256"] = np.array(sha256_of(res[2]))
+
+    # files of less than 1 MB each; tests/conftest.py merges them
+    lists = ("bloblist_", "blobfix_", "blobnms_")
+    parts = {"reference_vectors_blob_lists.npz": {k: v for k, v in out.items() if k.startswith(lists)},
+             "reference_vectors_live.npz": {k: v for k, v in out.items() if k.startswith("live_")},
+             "reference_vectors.npz": {k: v for k, v in out.items() if not k.startswith(lists + ("live_",))}}
+    for name, arrays in parts.items():
+        path = os.path.join(HERE, name)
+        np.savez_compressed(path, **arrays)
+        print("wrote", path, "%.1f KiB" % (os.path.getsize(path) / 1024), len(arrays), "arrays")
 
 
 if __name__ == "__main__":

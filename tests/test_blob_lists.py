@@ -66,24 +66,27 @@ def test_nms_properties(lists):
     assert len(inner) > 100 and np.all(d >= rsum * (1 - 1e-6))
 
 
-def test_live_against_reference_build(lists, golden):
-    import ctypes
-    import os
-    ref_so = os.path.join(os.path.dirname(__file__), "..", "oracle", "_ref", "libvisfd_ref.so")
-    if not os.path.exists(ref_so):
-        pytest.skip("oracle/_ref not present")
-    lib = ctypes.CDLL(ref_so)
-    if not hasattr(lib, "ref_blobs_sort"):
-        pytest.skip("oracle/_ref predates the blob list shim")
-    ref = vblobs.BlobLists(lib, "ref_blobs_")
+# DiscardOverlappingBlobs arguments of live_cases: separation, large and small overlap ratios, sort criterion
+LIVE_OVERLAP_ARGS = ((1.0, np.inf, np.inf, 3), (0.5, 0.2, 0.9, 3), (0.0, 0.5, 0.5, 1), (1.3, np.inf, np.inf, 4))
+
+
+def live_cases():
+    """random lists of 1, 7 and 400 blobs -> (n, blobs, blobs clipped to a 150 x 150 x 60 image, a random mask)"""
     g = np.random.default_rng(11)
     for n in (1, 7, 400):
         b = np.stack([g.uniform(0, 150, n), g.uniform(0, 150, n), g.uniform(0, 60, n), g.uniform(3, 40, n),
                       g.standard_normal(n) * 10], axis=1).astype(np.float32)
-        for sep, large, small, crit in ((1.0, np.inf, np.inf, 3), (0.5, 0.2, 0.9, 3), (0.0, 0.5, 0.5, 1), (1.3, np.inf, np.inf, 4)):
-            assert np.array_equal(lists.discard_overlapping(b, sep, large, small, crit),
-                                  ref.discard_overlapping(b, sep, large, small, crit)), (n, sep, large, small, crit)
         mask = (g.uniform(size=(60, 150, 150)) > 0.3).astype(np.float32)
         bb = b.copy()
         bb[:, :3] = np.clip(bb[:, :3], 0, [149, 149, 59])
-        assert np.array_equal(lists.discard_masked(bb, mask), ref.discard_masked(bb, mask))
+        yield n, b, bb, mask
+
+
+def test_live_against_reference_build(lists, golden):
+    """live_cases through DiscardOverlappingBlobs and DiscardMaskedBlobs: the blobs the reference kept, in its order
+    (stored as row numbers of the input; tests/golden/README.md)"""
+    for n, b, bb, mask in live_cases():
+        for k, (sep, large, small, crit) in enumerate(LIVE_OVERLAP_ARGS):
+            want = b[golden["live_blobs_%d_overlap%d" % (n, k)]]
+            assert np.array_equal(lists.discard_overlapping(b, sep, large, small, crit), want), (n, sep, large, small, crit)
+        assert np.array_equal(lists.discard_masked(bb, mask), bb[golden["live_blobs_%d_masked" % n]])

@@ -1,8 +1,6 @@
 """MRC/REC file I/O (include/visfd_mrc.h, SURVEY 8f rank 2) against the reference's MrcSimple:
 golden files in every mode, what MrcSimple::Read made of them, the bytes MrcSimple::Write
 produced (tests/golden/make_golden.py).  Host code: no GPU needed."""
-import os
-
 import numpy as np
 import pytest
 
@@ -36,16 +34,8 @@ def test_read_and_write_match_the_reference(io, golden, tmp_path):
         assert hdr2.mode == 2 and np.array_equal(vox2, vox), name
 
 
-def test_live_against_reference_build(io, golden, tmp_path):
-    """the same through oracle/_ref where it has been built (dev container, GPU box)"""
-    import ctypes
-    ref_so = os.path.join(os.path.dirname(__file__), "..", "oracle", "_ref", "libvisfd_ref.so")
-    if not os.path.exists(ref_so):
-        pytest.skip("oracle/_ref not present")
-    lib = ctypes.CDLL(ref_so)
-    if not hasattr(lib, "ref_mrc_read"):
-        pytest.skip("oracle/_ref predates the MRC shim")
-    ref = vmrc.MrcIO(lib, "ref_mrc_")
+def live_case(io):
+    """a header from visfd_mrc_header_init with a shape and a cell set, random float voxels"""
     rng = np.random.default_rng(9)
     vox = rng.standard_normal((9, 4, 11)).astype(np.float32)
     h = vmrc.MrcHeader()
@@ -53,14 +43,18 @@ def test_live_against_reference_build(io, golden, tmp_path):
     h.nvoxels[:] = (11, 4, 9)
     h.mvoxels[:] = (11, 4, 9)
     h.cellA[:] = (22.0, 8.0, 18.0)
-    ours, theirs = tmp_path / "a.mrc", tmp_path / "b.mrc"
-    h2 = vmrc.MrcHeader.from_buffer_copy(h.as_bytes())
+    return h, vox
+
+
+def test_live_against_reference_build(io, golden, tmp_path):
+    """live_case written and read back: the bytes the reference's MrcSimple::Write produced for it and the header
+    its MrcSimple::Read made of the file (tests/golden/README.md)"""
+    h, vox = live_case(io)
+    ours = tmp_path / "a.mrc"
     io.write(ours, h, vox)
-    ref.write(theirs, h2, vox)
-    assert ours.read_bytes() == theirs.read_bytes()
+    assert ours.read_bytes() == golden["live_mrc_out"].tobytes()
     ho, vo = io.read(ours)
-    hr, vr = ref.read(ours)
-    assert ho.as_bytes() == hr.as_bytes() and np.array_equal(vo, vr) and np.array_equal(vo, vox)
+    assert ho.as_bytes() == golden["live_mrc_hdr"].tobytes() and np.array_equal(vo, vox)
 
 
 def ctypes_byref(x):

@@ -135,20 +135,35 @@ def test_c1_reference_fixture(oracle, golden):
     assert (m0["out"] != 0).sum() == 27
 
 
-def test_port_matches_reference_live(oracle, ref_oracle):
-    """Where oracle/_ref exists: fresh seeded inputs, every stage, bit for bit."""
+def port_live_outputs(o):
+    """Every stage of the path on a seeded 15 x 18 x 21 tomogram with a random mask, through checker `o`:
+    name -> array"""
     from visfd_b200 import synth
     vol = synth.tomogram((15, 18, 21), seed=11)
     rng = np.random.default_rng(2)
     mask = (rng.random(vol.shape) > 0.2).astype(np.float32)
-    for kw in (dict(), dict(mask=mask), dict(normalize=False)):
-        eq(oracle.apply_gauss(vol, 1.7, 4, **kw)[0], ref_oracle.apply_gauss(vol, 1.7, 4, **kw)[0])
-    eq(oracle.apply_log(vol, 2.0, 0.02, 2.6482)[0], ref_oracle.apply_log(vol, 2.0, 0.02, 2.6482)[0])
-    a = oracle.membrane(vol, 1.2, 2.6482, 1, 0.1, True, 3.0, 4, SQ2, mask=mask)
-    b = ref_oracle.membrane(vol, 1.2, 2.6482, 1, 0.1, True, 3.0, 4, SQ2, mask=mask)
+    out = {}
+    for name, kw in (("gauss", dict()), ("gauss_masked", dict(mask=mask)), ("gauss_nonorm", dict(normalize=False))):
+        out[name] = o.apply_gauss(vol, 1.7, 4, **kw)[0]
+    out["log"] = o.apply_log(vol, 2.0, 0.02, 2.6482)[0]
+    m = o.membrane(vol, 1.2, 2.6482, 1, 0.1, True, 3.0, 4, SQ2, mask=mask)
     for k in ("hess_saliency", "direction", "tensor", "out"):
-        eq(a[k], b[k])
-    assert a["threshold"] == b["threshold"]
+        out["membrane_" + k] = m[k]
+    out["membrane_threshold"] = np.float32(m["threshold"])
+    return out
+
+
+def test_port_matches_reference_live(oracle, golden):
+    """Fresh seeded inputs, every stage, bit for bit: against the reference's outputs stored in
+    tests/golden/reference_vectors_live.npz (tests/golden/README.md), and against oracle/_ref itself where it
+    has been built."""
+    from oracle.pyoracle import Oracle, have
+    got = port_live_outputs(oracle)
+    for k, v in got.items():
+        eq(v, golden["live_port_" + k])
+    if have("reference"):
+        for k, v in port_live_outputs(Oracle("reference")).items():
+            eq(got[k], v)
 
 
 def test_binning_matches_reference(golden, oracle):
@@ -194,7 +209,9 @@ def test_draw_regions(oracle, golden):
     assert np.array_equal(golden["draw_empty"], draw_cases()["empty"][0])
 
 
-def test_draw_regions_vs_reference(oracle, ref_oracle):
+def random_draw_cases():
+    """20 random sets of 1 to 6 spheres and boxes, half of them on a zero image, a third of them masked
+    -> (trial, image, mask, regions)"""
     rng = np.random.default_rng(5)
     shape = (17, 19, 23)
     for trial in range(20):
@@ -209,9 +226,17 @@ def test_draw_regions_vs_reference(oracle, ref_oracle):
                 regions.append(("rect", lo[0], hi[0], lo[1], hi[1], lo[2], hi[2], v))
         img = np.zeros(shape, np.float32) if trial % 2 else rng.standard_normal(shape).astype(np.float32)
         mask = None if trial % 3 else (rng.random(shape) > 0.4).astype(np.float32)
+        yield trial, img, mask, regions
+
+
+def test_draw_regions_vs_reference(oracle, golden):
+    """random_draw_cases: the reference's images, stored as the voxels it changed, NaN elsewhere
+    (tests/golden/reference_vectors_live.npz, tests/golden/README.md)"""
+    for trial, img, mask, regions in random_draw_cases():
         for subtract in (False, True):
+            changed = golden["live_draw_%d_%d" % (trial, subtract)]
             eq(oracle.draw_regions(img, regions, mask=mask, negative_means_subtract=subtract),
-               ref_oracle.draw_regions(img, regions, mask=mask, negative_means_subtract=subtract))
+               np.where(np.isnan(changed), img, changed))
 
 
 def test_c1_pass2_known_answer(golden):
@@ -255,31 +280,47 @@ def _random_connect_case(oracle, seed, shape=(18, 20, 22)):
     return sal, T.astype(np.float32), mask, float(np.quantile(sal, 0.6))
 
 
-def test_label_connected_restatement_is_the_reference(oracle, ref_oracle, golden):
+def restatement_connect_calls(o, golden):
+    """The LabelConnected calls of test_label_connected_restatement_is_the_reference: (name, args, kwargs) for the C1
+    pipeline output of checker `o`, random fields with masks, plateaus, rejected seeds and merges, and one field
+    with the direction thresholds disabled"""
+    sigma, ratio, tv_sigma, expo, cutoff, best = [float(v) for v in golden["c1_params"]]
+    r = o.membrane(golden["c1_in_binned"], sigma, ratio, 1, best, True, tv_sigma, int(expo), cutoff)
+    yield "c1", (r["out"], r["tensor"], 1e9), dict(angle_deg=30.0, want_direction=True)
+    for seed in range(6):
+        sal, T, mask, thr = _random_connect_case(o, seed)
+        for angle in (25.0, 60.0):
+            yield "random_%d_%g" % (seed, angle), (sal, T, thr), dict(angle_deg=angle, mask=mask, want_direction=True)
+    sal, T, mask, thr = _random_connect_case(o, 2)
+    yield "thresholds_disabled", (sal, T, 6.0), dict(thresholds=(-np.inf,) * 4)
+
+
+def test_label_connected_restatement_is_the_reference(oracle, golden):
     """oracle/visfd_oracle.cpp::vo_label_connected == the unmodified LabelConnected (lib/visfd/connect.hpp:171) behind
     HandleTV's arguments, label for label and direction for direction (bit-identical: same compiler, same libm), on
-    the C1 pipeline output and on random fields with masks, plateaus, rejected seeds and merges."""
-    sigma, ratio, tv_sigma, expo, cutoff, best = [float(v) for v in golden["c1_params"]]
-    r = ref_oracle.membrane(golden["c1_in_binned"], sigma, ratio, 1, best, True, tv_sigma, int(expo), cutoff)
-    a = oracle.label_connected(r["out"], r["tensor"], 1e9, angle_deg=30.0, want_direction=True)
-    b = ref_oracle.label_connected(r["out"], r["tensor"], 1e9, angle_deg=30.0, want_direction=True)
-    assert a[1] == b[1] == 1 and np.array_equal(a[0], b[0]) and np.array_equal(a[2], b[2])
+    restatement_connect_calls: against the reference's labels, stored directions of the clustered voxels and a SHA-256
+    of the whole direction field (tests/golden/reference_vectors_live.npz, tests/golden/README.md), and against
+    oracle/_ref itself where it has been built."""
+    from oracle.pyoracle import Oracle, have
+    from util import sha256_of
+    ref = Oracle("reference") if have("reference") else None
     total = 0
-    for seed in range(6):
-        sal, T, mask, thr = _random_connect_case(oracle, seed)
-        for angle in (25.0, 60.0):
-            a = oracle.label_connected(sal, T, thr, angle_deg=angle, mask=mask, want_direction=True)
-            b = ref_oracle.label_connected(sal, T, thr, angle_deg=angle, mask=mask, want_direction=True)
-            assert a[1] == b[1]
-            assert np.array_equal(a[0], b[0])
-            assert np.array_equal(a[2], b[2])
-            total += a[1]
-    assert total > 20
-    ninf = -np.inf
-    sal, T, mask, thr = _random_connect_case(oracle, 2)
-    a = oracle.label_connected(sal, T, 6.0, thresholds=(ninf,) * 4)
-    b = ref_oracle.label_connected(sal, T, 6.0, thresholds=(ninf,) * 4)
-    assert a[1] == b[1] > 1 and np.array_equal(a[0], b[0])
+    for name, args, kw in restatement_connect_calls(oracle, golden):
+        key = "live_connect_%s_" % name
+        a = oracle.label_connected(*args, **kw)
+        assert a[1] == int(golden[key + "n_clusters"]), name
+        assert np.array_equal(a[0], golden[key + "labels"]), name
+        if kw.get("want_direction"):
+            eq(a[2][a[0] >= 1], golden[key + "direction_inside"])
+            assert sha256_of(a[2]) == str(golden[key + "direction_sha256"]), name
+        if ref is not None:
+            b = ref.label_connected(*args, **kw)
+            assert a[1] == b[1] and np.array_equal(a[0], b[0]), name
+            if kw.get("want_direction"):
+                assert np.array_equal(a[2], b[2]), name
+        total += a[1] if name.startswith("random") else 0
+    assert int(golden["live_connect_c1_n_clusters"]) == 1
+    assert total > 20 and int(golden["live_connect_thresholds_disabled_n_clusters"]) > 1
 
 
 def test_label_connected_restatement_c1_known_answer(oracle, golden):

@@ -1,4 +1,6 @@
 """Parity metrics shared by the tests (tolerances from BASELINE.json:north_star)."""
+import hashlib
+
 import numpy as np
 
 TOL_GAUSS = 1e-5      # Gaussian / DoG / LoG outputs
@@ -91,3 +93,15 @@ def draw_cases():
         "negative_first_nonzero": (noisy, None, [("sphere", 9.0, 9.0, 9.0, 5.0, -1.0)], True),
         "empty": (noisy, None, [], True),
     }
+
+
+def sha256_of(*arrays):
+    """SHA-256 (hex) of the bytes, shapes and dtypes of the arrays, None skipped: a stored check that the inputs or
+    outputs of a test are, bit for bit, those some stored vectors were made from."""
+    h = hashlib.sha256()
+    for a in arrays:
+        if a is not None:
+            a = np.ascontiguousarray(a)
+            h.update(("%s%s" % (a.dtype.str, a.shape)).encode())
+            h.update(a.tobytes())
+    return h.hexdigest()
