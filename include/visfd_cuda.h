@@ -270,13 +270,14 @@ int visfd_cuda_vote_slab_host(visfd_ctx *ctx, int64_t nx, int64_t ny, int64_t nz
                               float *out_host);
 
 /* ---- the same pipeline on several GPUs of one node, one call (SURVEY 8b / 8e) ------------------ */
-/* visfd_cuda_membrane with HOST arrays, spread over `ndev` devices as Z-slabs (one worker thread per device, no
+/* visfd_cuda_membrane with HOST arrays, spread over `ndev` devices as Z-slabs (one host thread per device, no
  * process per GPU, no MPI): the drop-in a C++ host such as filter_mrc links.  devices[] may name a device more than
  * once.  Each device uploads its slab (own planes + halo of raw source, halo = tv_halfwidth + 1 + gauss_halfwidth)
  * straight from src_host; the `-tv-best` cut is a global radix select (histograms summed on the host, handlers.cpp:
  * 1766-1782); every device writes its planes of the result into out_host behind its voting kernels.  The result is
  * bit-identical to visfd_cuda_membrane on one GPU.  mask_host may be NULL.  device_ms (ndev doubles or NULL): device
- * time of each worker, first upload to last download.  Contexts are created on first use and kept. */
+ * time of each worker, first upload to last download.  The call keeps one context per entry of devices[], created
+ * on first use and kept for later calls; concurrent calls are therefore serialised (one runs at a time). */
 int visfd_cuda_membrane_multi(int ndev, const int *devices, int64_t nx, int64_t ny, int64_t nz,
                               const float *src_host, const float *mask_host, const visfd_membrane_params *p,
                               float *out_host, float *threshold_out, double *device_ms);

@@ -583,7 +583,8 @@ float vo_saliency_cut(i64 N, float *sal, const float *mask, float cut,
       if (!(mask && mask[i] == 0)) v.push_back(sal[i]);
     std::sort(v.begin(), v.end(), std::greater<float>());
     size_t n = v.size();
-    size_t k = (size_t)floorf((float)n * cut);
+    // fraction >= 1 indexes past the end in the reference; clamped to the last element, as the library does
+    size_t k = std::min((size_t)floorf((float)n * cut), n - 1);
     thr = v[k];
   }
   for (i64 i = 0; i < N; i++)

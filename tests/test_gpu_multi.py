@@ -11,8 +11,9 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 @pytest.mark.gpu
 def test_multi_device_c_entry_equals_one_gpu():
     """visfd_cuda_membrane_multi (one C call, one worker thread per device; tests/cpp/multi_check.cpp) == the one-GPU
-    result bit for bit for 1, 2, 3, 4 and 8 workers -- on as many devices as the box has (a one-GPU box lists the same
-    device several times, which runs the same slab logic)."""
+    result bit for bit for 1, 2, 3, 4 and 8 workers and for two calls made at once -- on as many devices as the box has
+    (a one-GPU box lists the same device several times, which runs the same slab logic).  Calls that fail (no
+    un-masked voxel, a voting radius above the maximum, a missing device) return their error."""
     exe = os.path.join(ROOT, "tests", "cpp", "multi_check")
     if not os.path.exists(exe):
         subprocess.check_call(["make", "-s", "-C", os.path.dirname(exe)])

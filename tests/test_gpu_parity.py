@@ -368,7 +368,8 @@ def test_saliency_cut_bit_exact(ctx, oracle, golden):
     assert np.array_equal(out, golden["cut_frac0.1"])
 
 
-@pytest.mark.parametrize("n,frac", [(1, 0.05), (37, 0.5), (100003, 0.05), (1 << 20, 0.013), (300007, 0.999)])
+@pytest.mark.parametrize("n,frac", [(1, 0.05), (37, 0.5), (37, 1.0), (1000, 0.0), (100003, 0.05),
+                                    (1 << 20, 0.013), (300007, 0.999)])
 def test_radix_select_matches_sort(ctx, oracle, n, frac):
     rng = np.random.default_rng(n)
     v = (rng.standard_normal(n) ** 2 * 1e9).astype(np.float32)

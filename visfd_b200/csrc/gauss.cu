@@ -46,18 +46,16 @@ namespace visfd_cuda {
 // everything outside the volume, and an mbarrier per chunk tells the CTA when it landed.
 // ---------------------------------------------------------------------------------
 static PFN_cuTensorMapEncodeTiled tensor_map_encoder() {
-  static PFN_cuTensorMapEncodeTiled fn = nullptr;
-  static bool tried = false;
-  if (!tried) {
-    tried = true;
+  // resolved once; the initialisation of a function-local static is thread-safe (several host threads filter at once)
+  static const PFN_cuTensorMapEncodeTiled fn = [] {
     void *p = nullptr;
     cudaDriverEntryPointQueryResult q;
     if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess &&
         q == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<PFN_cuTensorMapEncodeTiled>(p);
-    else
-      cudaGetLastError();
-  }
+      return reinterpret_cast<PFN_cuTensorMapEncodeTiled>(p);
+    cudaGetLastError();
+    return PFN_cuTensorMapEncodeTiled(nullptr);
+  }();
   return fn;
 }
 

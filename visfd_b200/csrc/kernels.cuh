@@ -2,6 +2,8 @@
 // Everything here works on DEVICE memory of ctx's GPU and enqueues on ctx->stream;
 // the extern "C" layer in api.cu adds host staging, argument checks and timing.
 #pragma once
+#include <functional>
+
 #include "common.cuh"
 
 namespace visfd_cuda {
@@ -41,14 +43,19 @@ void tensor_score_device(visfd_ctx *ctx, i64 n, const float *tensor, const float
                          float *eivals, float *direction);
 
 // ---- select.cu --------------------------------------------------------------------
+constexpr int HIST_BINS = 2048;
 void select_hist_device(visfd_ctx *ctx, i64 n, const float *sal, const float *mask,
-                        uint32_t prefix, int prefix_bits, uint64_t *hist_host /*2048*/);
+                        uint32_t prefix, int prefix_bits, uint64_t *hist_host /*HIST_BINS*/);
 int select_step_host(const uint64_t *hist, uint32_t *prefix, int *prefix_bits, uint64_t *rank);
 uint32_t float_to_key(float f);
 float key_to_float(uint32_t k);
 // count of un-masked voxels
 i64 count_unmasked_device(visfd_ctx *ctx, i64 n, const float *mask);
-// threshold such that the reference's cut (handlers.cpp:1751-1797) is reproduced
+// Threshold such that the reference's cut (handlers.cpp:1751-1797) is reproduced, by a radix select over
+// histograms that summed_hist fills: the HIST_BINS-bin histogram of the keys that match the prefix, summed
+// over every part of the volume (select_hist_device on each part).
+float select_threshold(float fraction,
+                       const std::function<void(uint32_t prefix, int prefix_bits, uint64_t *hist)> &summed_hist);
 float select_threshold_device(visfd_ctx *ctx, i64 n, const float *sal, const float *mask,
                               float fraction);
 void apply_cut_device(visfd_ctx *ctx, i64 n, float *sal, float thr);

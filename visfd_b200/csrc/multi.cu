@@ -3,21 +3,24 @@
 //
 //   visfd_cuda_membrane_multi(ndev, devices, nx, ny, nz, src_host, mask_host, params, out_host, &threshold)
 //
-// One worker thread per device.  The volume is cut into Z-slabs exactly as visfd_b200/slab.py does for the
+// One slab per device.  The volume is cut into Z-slabs exactly as visfd_b200/slab.py does for the
 // process-per-GPU driver (rank boundaries on multiples of 8 planes, slabs widened by a halo of RAW SOURCE planes,
 // halo = tv_halfwidth + 1 + gauss_halfwidth, slab start rounded down to a multiple of 8), so every stage is
 // slab-local and the result is bit-identical to the one-GPU result.  Because the source lives in host memory, each
 // device uploads its slab -- halo included -- straight from the caller's array over its own PCIe link: there is no
-// device-to-device halo traffic at all.  The only exchange is the radix select of the `-tv-best` cut: three rounds of
-// 2048-bin histograms, summed by the host between two thread barriers (the cut must be a GLOBAL order statistic,
-// bin/filter_mrc/handlers.cpp:1766-1782).  Each device delivers its planes of the result into the caller's array
-// chunk by chunk behind its voting kernels (visfd_cuda_vote_slab_host).
+// device-to-device halo traffic at all.
+//
+// The call runs in phases.  A phase runs every slab at once (slab 0 on the calling thread, the others on threads of
+// their own) and is joined on the host before the next one starts, so a slab that fails cannot leave the others
+// waiting for it: (1) upload + ridge saliency; (2) for the `-tv-best` cut, one phase per round of the radix select
+// (select_threshold), in which every slab histograms its own planes into 2048 bins and the calling thread sums them
+// (the cut must be a GLOBAL order statistic, bin/filter_mrc/handlers.cpp:1766-1782); (3) voting, each device
+// delivering its planes of the result into the caller's array chunk by chunk behind its voting kernels
+// (visfd_cuda_vote_slab_host).
 //
 // The same device may be listed several times (two slabs on one GPU): that is how the one-GPU test box exercises
 // the slab logic.
-#include <atomic>
-#include <condition_variable>
-#include <cstring>
+#include <algorithm>
 #include <mutex>
 #include <thread>
 
@@ -27,27 +30,6 @@
 using namespace visfd_cuda;
 
 namespace {
-
-class Barrier {   // C++17: no std::barrier
-  std::mutex m;
-  std::condition_variable cv;
-  const int n;
-  int waiting = 0;
-  uint64_t generation = 0;
- public:
-  explicit Barrier(int count) : n(count) {}
-  void wait() {
-    std::unique_lock<std::mutex> lk(m);
-    const uint64_t g = generation;
-    if (++waiting == n) {
-      waiting = 0;
-      generation++;
-      cv.notify_all();
-    } else {
-      cv.wait(lk, [&] { return generation != g; });
-    }
-  }
-};
 
 struct SlabPlan {
   int64_t own0, own1;     // global planes this worker delivers
@@ -76,12 +58,11 @@ std::vector<SlabPlan> make_plans(int64_t nz, int world, int gauss_hw, int tv_hw)
   return plans;
 }
 
-// contexts are kept between calls: one per (slot, device)
-std::mutex g_ctx_mutex;
+// One call at a time: the contexts are kept between calls, one per (slot, device), and a call uses them throughout.
+std::mutex g_call_mutex;
 std::vector<std::pair<int, visfd_ctx *> > g_ctx;   // index = slot
 
 visfd_ctx *context_for(int slot, int device) {
-  std::lock_guard<std::mutex> lk(g_ctx_mutex);
   if ((int)g_ctx.size() <= slot) g_ctx.resize((size_t)slot + 1, {-1, nullptr});
   auto &e = g_ctx[(size_t)slot];
   if (e.second && e.first != device) {
@@ -94,6 +75,50 @@ visfd_ctx *context_for(int slot, int device) {
     e = {device, c};
   }
   return e.second;
+}
+
+// What a slab keeps on its device from one phase to the next.
+struct Slab {
+  visfd_ctx *ctx = nullptr;
+  SlabPlan plan;
+  Scratch<float> mask, smoothed, saliency;
+  cudaEvent_t start = nullptr, stop = nullptr;   // device time: first upload to last download
+  double ms = 0.0;
+  uint64_t hist[HIST_BINS];
+  ~Slab() {
+    if (start) cudaEventDestroy(start);
+    if (stop) cudaEventDestroy(stop);
+  }
+};
+
+// Runs fn(slab) for every slab at once, slab 0 on the calling thread and the others on threads of their own, each
+// on its slab's device.  Returns when all of them have finished, and then throws the error of the first slab that
+// failed.
+template <typename Fn>
+void for_each_slab(std::vector<Slab> &slabs, const Fn &fn) {
+  std::vector<std::string> errors(slabs.size());
+  auto run = [&](size_t r) {
+    try {
+      VCK(cudaSetDevice(slabs[r].ctx->device));
+      fn(slabs[r]);
+    } catch (const std::exception &ex) {
+      errors[r] = ex.what();
+    }
+  };
+  std::vector<std::thread> threads;
+  for (size_t r = 1; r < slabs.size(); r++) {
+    try {
+      threads.emplace_back(run, r);
+    } catch (const std::exception &ex) {   // no thread for this slab; the others still run and are joined
+      errors[r] = ex.what();
+    }
+  }
+  run(0);
+  for (std::thread &t : threads) t.join();
+  for (size_t r = 0; r < slabs.size(); r++)
+    if (!errors[r].empty())
+      throw Error("visfd_cuda_membrane_multi, slab " + std::to_string(r) + " on device " +
+                  std::to_string(slabs[r].ctx->device) + ": " + errors[r]);
 }
 
 }  // namespace
@@ -113,129 +138,69 @@ extern "C" int visfd_cuda_membrane_multi(int ndev, const int *devices, int64_t n
     const std::vector<SlabPlan> plans = make_plans(nz, world, gauss_hw, tv_hw);
     const size_t plane = (size_t)nx * (size_t)ny;
 
-    std::vector<visfd_ctx *> ctxs((size_t)world);
-    for (int r = 0; r < world; r++) ctxs[(size_t)r] = context_for(r, devices[r]);
+    std::lock_guard<std::mutex> lock(g_call_mutex);
+    std::vector<Slab> slabs((size_t)world);
+    for (int r = 0; r < world; r++) {
+      slabs[(size_t)r].ctx = context_for(r, devices[r]);
+      slabs[(size_t)r].plan = plans[(size_t)r];
+    }
 
-    Barrier barrier(world);
-    std::vector<std::string> errors((size_t)world);
-    std::vector<std::vector<uint64_t> > hists((size_t)world, std::vector<uint64_t>(2048));
-    // state of the distributed radix select, written by worker 0 between barriers
-    uint32_t prefix = 0;
-    int prefix_bits = 0;
-    uint64_t rank_k = 0;
+    // ---- upload the slab, halo included, and compute its ridge saliency ----
+    for_each_slab(slabs, [&](Slab &s) {
+      const SlabPlan &pl = s.plan;
+      const size_t n = (size_t)(pl.slab1 - pl.slab0) * plane;
+      VCK(cudaEventCreate(&s.start));
+      VCK(cudaEventCreate(&s.stop));
+      VCK(cudaEventRecord(s.start, s.ctx->stream));
+      Scratch<float> src(s.ctx, n);   // the raw slab is not needed after this phase
+      s.smoothed.reset(s.ctx, n);
+      s.saliency.reset(s.ctx, n);
+      VCK(cudaMemcpyAsync(src.get(), src_host + (size_t)pl.slab0 * plane, n * sizeof(float), cudaMemcpyHostToDevice,
+                          s.ctx->stream));
+      if (mask_host) {
+        s.mask.reset(s.ctx, n);
+        VCK(cudaMemcpyAsync(s.mask.get(), mask_host + (size_t)pl.slab0 * plane, n * sizeof(float),
+                            cudaMemcpyHostToDevice, s.ctx->stream));
+      }
+      if (visfd_cuda_ridge_saliency_slab(s.ctx, nx, ny, pl.slab1 - pl.slab0, pl.slab0, nz, src.get(), s.mask.get(),
+                                         p->sigma, p->truncate_ratio, p->eival_order, VISFD_SCORE_PLANAR,
+                                         s.smoothed.get(), s.saliency.get()) != 0)
+        throw Error(visfd_cuda_last_error());
+    });
+
+    // ---- global cut: radix select over the slabs' own planes ----
     float threshold = p->cut;
-    std::atomic<bool> failed{false};
-    std::mutex fail_mutex;
-    std::vector<double> ms((size_t)world, 0.0);
+    if (p->cut_is_fraction)
+      threshold = select_threshold(p->cut, [&](uint32_t prefix, int prefix_bits, uint64_t *hist) {
+        for_each_slab(slabs, [&](Slab &s) {
+          const size_t own = (size_t)(s.plan.own0 - s.plan.slab0) * plane;
+          select_hist_device(s.ctx, (i64)((s.plan.own1 - s.plan.own0) * (int64_t)plane), s.saliency.get() + own,
+                             mask_host ? s.mask.get() + own : nullptr, prefix, prefix_bits, s.hist);
+        });
+        std::fill(hist, hist + HIST_BINS, 0);
+        for (const Slab &s : slabs)
+          for (int b = 0; b < HIST_BINS; b++) hist[b] += s.hist[b];
+      });
 
-    auto worker = [&](int r) {
-      visfd_ctx *ctx = ctxs[(size_t)r];
-      const SlabPlan &pl = plans[(size_t)r];
-      const int64_t nzl = pl.slab1 - pl.slab0;
-      auto fail = [&](const std::string &m) {
-        std::lock_guard<std::mutex> lk(fail_mutex);
-        errors[(size_t)r] = m;
-        failed = true;
-      };
-      // stages run under try/catch individually: a worker that failed still meets the others at every barrier
-      Scratch<float> src, mask, smoothed, saliency, out;
-      cudaEvent_t e0 = nullptr, e1 = nullptr;
-      try {
-        VCK(cudaSetDevice(ctx->device));
-        VCK(cudaEventCreate(&e0));
-        VCK(cudaEventCreate(&e1));
-        VCK(cudaEventRecord(e0, ctx->stream));
-        src.reset(ctx, (size_t)nzl * plane);
-        smoothed.reset(ctx, (size_t)nzl * plane);
-        saliency.reset(ctx, (size_t)nzl * plane);
-        VCK(cudaMemcpyAsync(src.get(), src_host + (size_t)pl.slab0 * plane, (size_t)nzl * plane * sizeof(float),
-                            cudaMemcpyHostToDevice, ctx->stream));
-        if (mask_host) {
-          mask.reset(ctx, (size_t)nzl * plane);
-          VCK(cudaMemcpyAsync(mask.get(), mask_host + (size_t)pl.slab0 * plane, (size_t)nzl * plane * sizeof(float),
-                              cudaMemcpyHostToDevice, ctx->stream));
-        }
-        if (visfd_cuda_ridge_saliency_slab(ctx, nx, ny, nzl, pl.slab0, nz, src.get(), mask.get(), p->sigma,
-                                           p->truncate_ratio, p->eival_order, VISFD_SCORE_PLANAR, smoothed.get(),
-                                           saliency.get()) != 0)
-          throw Error(visfd_cuda_last_error());
-        src.free();   // the raw slab is not needed any more
-      } catch (const std::exception &ex) {
-        fail(ex.what());
-      }
-      // ---- global cut: radix select over the workers' own planes ----
-      if (p->cut_is_fraction) {
-        bool first = true;
-        for (;;) {
-          barrier.wait();                    // prefix / prefix_bits of this round are final
-          if (failed || prefix_bits >= 32) break;
-          try {
-            VCK(cudaSetDevice(ctx->device));
-            select_hist_device(ctx, (i64)((pl.own1 - pl.own0) * (int64_t)plane),
-                               saliency.get() + (size_t)(pl.own0 - pl.slab0) * plane,
-                               mask_host ? mask.get() + (size_t)(pl.own0 - pl.slab0) * plane : nullptr, prefix,
-                               prefix_bits, hists[(size_t)r].data());
-            VCK(cudaStreamSynchronize(ctx->stream));
-          } catch (const std::exception &ex) {
-            fail(ex.what());
-          }
-          barrier.wait();                    // all histograms are in
-          if (r == 0 && !failed) {
-            std::vector<uint64_t> sum(2048, 0);
-            for (int q = 0; q < world; q++)
-              for (int b = 0; b < 2048; b++) sum[(size_t)b] += hists[(size_t)q][(size_t)b];
-            if (first) {
-              uint64_t total = 0;
-              for (uint64_t v : sum) total += v;
-              if (total == 0) {
-                fail("saliency cut: no un-masked voxels");
-              } else {
-                // i = floor(n_voxels * fraction) in float, as handlers.cpp:1779-1782; clamped to the last element
-                const uint64_t k = (uint64_t)std::max(0.0f, floorf((float)total * p->cut));
-                rank_k = std::min(k, total - 1);
-              }
-            }
-            if (!failed) select_step_host(sum.data(), &prefix, &prefix_bits, &rank_k);
-          }
-          first = false;
-        }
-        if (r == 0 && !failed) threshold = key_to_float(prefix);
-        barrier.wait();                      // threshold is final
-      }
-      // ---- voting on the own planes, delivered into the caller's array ----
-      if (!failed) {
-        try {
-          VCK(cudaSetDevice(ctx->device));
-          out.reset(ctx, (size_t)(pl.own1 - pl.own0) * plane);
-          if (visfd_cuda_vote_slab_host(ctx, nx, ny, nzl, pl.slab0, nz, pl.own0 - pl.slab0, pl.own1 - pl.slab0,
-                                        pl.vote0 - pl.slab0, pl.vote1 - pl.slab0, saliency.get(), smoothed.get(),
-                                        mask_host ? mask.get() : nullptr, threshold, p, out.get(), nullptr,
-                                        out_host + (size_t)pl.own0 * plane) != 0)
-            throw Error(visfd_cuda_last_error());
-          VCK(cudaEventRecord(e1, ctx->stream));
-          VCK(cudaEventSynchronize(e1));
-          float t = 0;
-          VCK(cudaEventElapsedTime(&t, e0, e1));
-          ms[(size_t)r] = t;
-        } catch (const std::exception &ex) {
-          fail(ex.what());
-        }
-      }
-      if (e0) cudaEventDestroy(e0);
-      if (e1) cudaEventDestroy(e1);
-    };
+    // ---- voting on the own planes, delivered into the caller's array ----
+    for_each_slab(slabs, [&](Slab &s) {
+      const SlabPlan &pl = s.plan;
+      Scratch<float> out(s.ctx, (size_t)(pl.own1 - pl.own0) * plane);
+      if (visfd_cuda_vote_slab_host(s.ctx, nx, ny, pl.slab1 - pl.slab0, pl.slab0, nz, pl.own0 - pl.slab0,
+                                    pl.own1 - pl.slab0, pl.vote0 - pl.slab0, pl.vote1 - pl.slab0, s.saliency.get(),
+                                    s.smoothed.get(), s.mask.get(), threshold, p, out.get(), nullptr,
+                                    out_host + (size_t)pl.own0 * plane) != 0)
+        throw Error(visfd_cuda_last_error());
+      VCK(cudaEventRecord(s.stop, s.ctx->stream));
+      VCK(cudaEventSynchronize(s.stop));
+      float t = 0;
+      VCK(cudaEventElapsedTime(&t, s.start, s.stop));
+      s.ms = t;
+    });
 
-    std::vector<std::thread> threads;
-    for (int r = 1; r < world; r++) threads.emplace_back(worker, r);
-    worker(0);
-    for (auto &t : threads) t.join();
-    for (int r = 0; r < world; r++)
-      if (!errors[(size_t)r].empty())
-        throw Error("visfd_cuda_membrane_multi, slab " + std::to_string(r) + " on device " +
-                    std::to_string(devices[r]) + ": " + errors[(size_t)r]);
     if (threshold_out) *threshold_out = threshold;
     if (device_ms)
-      for (int r = 0; r < ndev; r++) device_ms[r] = r < world ? ms[(size_t)r] : 0.0;
+      for (int r = 0; r < ndev; r++) device_ms[r] = r < world ? slabs[(size_t)r].ms : 0.0;
     return 0;
   } catch (const std::exception &ex) {
     set_last_error(ex.what());

@@ -25,8 +25,6 @@ float key_to_float(uint32_t k) {
   return f;
 }
 
-constexpr int HIST_BINS = 2048;
-
 __device__ __forceinline__ void hist_add(unsigned int *sh, bool valid, uint32_t bin) {
   // warp-uniform bins (long runs of equal saliency, e.g. zeros) cost one atomic
   const unsigned full = 0xffffffffu;
@@ -147,15 +145,15 @@ int select_step_host(const uint64_t *hist, uint32_t *prefix, int *prefix_bits, u
   return 1;  // rank beyond the population
 }
 
-float select_threshold_device(visfd_ctx *ctx, i64 n, const float *sal, const float *mask,
-                              float fraction) {
+float select_threshold(float fraction,
+                       const std::function<void(uint32_t prefix, int prefix_bits, uint64_t *hist)> &summed_hist) {
   uint64_t hist[HIST_BINS];
   uint32_t prefix = 0;
   int prefix_bits = 0;
   uint64_t rank = 0;
   bool first = true;
   while (prefix_bits < 32) {
-    select_hist_device(ctx, n, sal, mask, prefix, prefix_bits, hist);
+    summed_hist(prefix, prefix_bits, hist);
     if (first) {
       uint64_t total = 0;
       for (int b = 0; b < HIST_BINS; b++) total += hist[b];
@@ -172,6 +170,13 @@ float select_threshold_device(visfd_ctx *ctx, i64 n, const float *sal, const flo
     VREQUIRE(rc == 0, "saliency cut: rank outside the population");
   }
   return key_to_float(prefix);
+}
+
+float select_threshold_device(visfd_ctx *ctx, i64 n, const float *sal, const float *mask,
+                              float fraction) {
+  return select_threshold(fraction, [&](uint32_t prefix, int prefix_bits, uint64_t *hist) {
+    select_hist_device(ctx, n, sal, mask, prefix, prefix_bits, hist);
+  });
 }
 
 __global__ void cut_kernel(float *__restrict__ sal, float thr, i64 n) {
