@@ -336,10 +336,11 @@ void visfd_cuda_set_timing(visfd_ctx *ctx, int enabled);
 int64_t visfd_cuda_last_voter_count(visfd_ctx *ctx);
 /* Which voting kernel the most recent voting call ran: 0 = tv_gather_kernel (radial decay by MUFU; every
  * parameter set), 1 / 2 = tv_gather_lut_kernel (decay and 1/r^2 from a shared-memory table indexed by the integer
- * r^2; exponent 4, positive weights, radius <= 24; 2 = the table ends at the support and the index is clamped).
- * Environment switches read by the voting call, for tests and tuning only: VISFD_CUDA_NO_LUT=1 forces kernel 0,
- * VISFD_CUDA_LUT_MODE=2 forces the clamped table, VISFD_CUDA_CHUNK_WAVES=n sets the smallest receiver chunk of the
- * overlapped download (default 64 waves of CTAs); visfd_cuda_membrane also reads VISFD_CUDA_UPLOAD_CHUNK=planes. */
+ * r^2; exponent 4, positive weights, radius <= 24; 2 = the table ends at the support and the index is clamped,
+ * used when the full table does not fit in shared memory: radii 21-24 on a B200).  The inputs alone decide.
+ * Environment switch read by the voting call, for tests and tuning only: VISFD_CUDA_CHUNK_WAVES=n sets the smallest
+ * receiver chunk of the overlapped download (default 64 waves of CTAs); visfd_cuda_membrane also reads
+ * VISFD_CUDA_UPLOAD_CHUNK=planes. */
 int visfd_cuda_last_tv_kernel(visfd_ctx *ctx);
 /* Number of (receiver, voter) pairs the reference's TVReceiveStickVotes would evaluate
  * past its skip tests (feature.hpp:2251-2270) for this input: voters as above, receivers

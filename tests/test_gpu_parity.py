@@ -399,19 +399,47 @@ def test_tv_golden(ctx, golden):
     assert np.all(got[tm == 0] == 0)
 
 
-@pytest.mark.parametrize("sigma_tv,shape", [(2.9, (20, 24, 28)), (7.08, (30, 33, 41)), (14.2, (44, 48, 50))])
+# The voting kernel each radius of test_tv_radii takes (exponent 4, positive weights): the table kernel up to
+# radius 24, with the full table (1) while it fits in the B200's 227 KB of shared memory beside the voter rings
+# (radius <= 20), else the table clamped at the support (2); the MUFU kernel (0) beyond.
+TV_RADII_KERNEL = {2.9: 1, 7.08: 1, 14.2: 1, 15.6: 2, 18.5: 0}
+
+
+@pytest.mark.parametrize("sigma_tv,shape", [(2.9, (20, 24, 28)), (7.08, (30, 33, 41)), (14.2, (44, 48, 50)),
+                                            (15.6, (32, 36, 40)), (18.5, (32, 36, 40))])
 def test_tv_radii(ctx, oracle, sigma_tv, shape):
-    """vote radii 4, 10 and 20 (hw = floor(sigma*sqrt2)); includes the lattice points that
+    """vote radii 4, 10, 20, 22 and 26 (hw = floor(sigma*sqrt2)); includes the lattice points that
     sit exactly on the support shell r^2 == hw^2"""
     vol = synth.tomogram(shape, seed=13)
     m = oracle.membrane(vol, 1.5, 2.6482, 1, 0.05, True, 0.0, 4, SQ2)
     sal, dire = m["hess_saliency"], m["direction"]
     want = oracle.tv_dense_stick(sal, dire, sigma_tv, 4, SQ2)
     got = ctx.tv_dense_stick(sal, dire, sigma_tv, 4, SQ2)
+    assert ctx.last_tv_kernel() == TV_RADII_KERNEL[sigma_tv]
     assert tensor_rel_err(got, want) <= TOL_SALIENCY
     hw = vb.tv_halfwidth(sigma_tv, SQ2)
     pairs = ctx.tv_count_pairs(sal, -np.inf, hw)
     assert pairs > 0
+
+
+def test_tv_nonpositive_weights_and_no_voters(ctx, oracle):
+    """a voter with negative saliency (thr = -inf) leaves the table kernel for the MUFU kernel without
+    the sqrt(weight) form; no voters at all: MUFU kernel, all-zero tensor"""
+    vol = synth.tomogram((20, 24, 28), seed=13)
+    m = oracle.membrane(vol, 1.5, 2.6482, 1, 0.05, True, 0.0, 4, SQ2)
+    sal, dire = m["hess_saliency"].copy(), m["direction"]
+    # negative voters at x < 10, positive ones at x >= 18: the radius is 4, so no receiver adds votes of
+    # both signs (a cancelling sum would be judged against its own small size)
+    sal[:, :, :10] *= -1.0
+    sal[:, :, 10:18] = 0.0
+    assert (sal < 0).any() and (sal > 0).any()
+    want = oracle.tv_dense_stick(sal, dire, 2.9, 4, SQ2)
+    got = ctx.tv_dense_stick(sal, dire, 2.9, 4, SQ2)
+    assert ctx.last_tv_kernel() == 0
+    assert tensor_rel_err(got, want) <= TOL_SALIENCY
+    got = ctx.tv_dense_stick(np.zeros_like(sal), dire, 2.9, 4, SQ2)
+    assert ctx.last_voter_count() == 0 and ctx.last_tv_kernel() == 0
+    assert not got.any()
 
 
 def test_tv_single_voter_support(ctx, oracle):

@@ -307,9 +307,10 @@ __device__ __forceinline__ void voter_direction(const DirSrc &d, int nx, int ny,
   n[2] = (float)e0[2];
 }
 
-// Pass 1 of the fill: positions and weights in brick order, voxels of a brick in (z, y, x) order.
+// Pass 1 of the fill: positions and weights in brick order, voxels of a brick in (z, y, x) order.  The records it
+// writes are the same for both gather kernels; voter_direction_kernel puts them in the chosen kernel's form.
 __global__ void __launch_bounds__(32 * VL_WARPS)
-voter_fill_kernel(VoterSrc v, const uint32_t *__restrict__ off, float inv_total, bool lut,
+voter_fill_kernel(VoterSrc v, const uint32_t *__restrict__ off, float inv_total,
                   VoterRec *__restrict__ rec, uint32_t *__restrict__ nonpos_flag) {
   const int lane = threadIdx.x & 31;
   const int bx0 = (blockIdx.x * VL_WARPS + (threadIdx.x >> 5)) * 8;
@@ -332,9 +333,7 @@ voter_fill_kernel(VoterSrc v, const uint32_t *__restrict__ off, float inv_total,
       // (a logarithm, a sixth root) are computed by voter_direction_kernel, where every lane has a voter -- here
       // ~5 % of the lanes do, and a warp would run the libm sequence for them at that lane efficiency
       VoterRec *q = rec + base + rank + __popc(nib & below);
-      const float px = -(float)x, py = -(float)(by * VBR + (r & 3)), pz = -(float)(bz * VBR + (r >> 2));
-      const float cs = lut ? pow2f(LUT_RHO_LOG2) : 1.0f;
-      q->a = make_float4(px * cs, py * cs, pz * cs, 0.0f);
+      q->a = make_float4(-(float)x, -(float)(by * VBR + (r & 3)), -(float)(bz * VBR + (r >> 2)), 0.0f);
       q->c.w = 4.0f * wgt;
     }
     rank += __popc(nib);
@@ -342,14 +341,14 @@ voter_fill_kernel(VoterSrc v, const uint32_t *__restrict__ off, float inv_total,
 }
 
 // Pass 2: one THREAD per voter (dense lanes -- in the brick pass only ~5 % of the lanes are
-// voters and the double-precision eigenvector would run at that lane efficiency).
+// voters and the double-precision eigenvector would run at that lane efficiency).  Finishes each
+// record for the gather kernel the host chose: lut = the table kernel.
 __global__ void __launch_bounds__(256)
 voter_direction_kernel(DirSrc d, int nx, int ny, uint32_t n_voters, bool lut, VoterRec *__restrict__ rec) {
   const uint32_t i = blockIdx.x * 256u + threadIdx.x;
   if (i >= n_voters) return;
   VoterRec *r = rec + i;
-  float4 a = r->a;
-  if (lut) { const float un = pow2f(-LUT_RHO_LOG2); a.x *= un; a.y *= un; a.z *= un; }
+  const float4 a = r->a;
   float n[3];
   voter_direction(d, nx, ny, (int)(-a.x), (int)(-a.y), (i64)(-a.z), n);
   // the weight w4 = 4 * saliency * mask weight / table total in the three forms vote() / vote_lut() use
@@ -358,7 +357,8 @@ voter_direction_kernel(DirSrc d, int nx, int ny, uint32_t n_voters, bool lut, Vo
   if (lut) {   // only used when every weight is positive (checked by the host before the launch)
     const float lam = (float)pow((double)fmaxf(w4, 0.0f), 1.0 / 6.0);
     sb = lam * pow2f(LUT_BETA_LOG2); sc = lam * pow2f(LUT_BETA2_LOG2);
-    r->a.w = lam * lam * pow2f(LUT_K_LOG2);
+    const float rho = pow2f(LUT_RHO_LOG2);   // the table kernel's position scale (exact: a power of two)
+    r->a = make_float4(a.x * rho, a.y * rho, a.z * rho, lam * lam * pow2f(LUT_K_LOG2));
     r->b.w = lam;
     r->c.w = 0.0f;
   } else {
@@ -916,6 +916,132 @@ __global__ void __launch_bounds__(32 * LUT_WARPS, 1) tv_gather_lut_kernel(Gather
 // ---------------------------------------------------------------------------------
 // host driver
 // ---------------------------------------------------------------------------------
+// Count, scan, fill: the voter list in brick order (off = the list's offset of every brick), its records in the
+// form voter_fill_kernel leaves them.  Returns the number of voters; nonpos: some voter's weight is <= 0.
+static uint32_t build_voter_list(visfd_ctx *ctx, const VoterSrc &vs, float inv_total, Scratch<uint32_t> &off,
+                                 Scratch<VoterRec> &rec, bool &nonpos) {
+  const i64 n_bricks = (i64)vs.vbx * vs.vby * vs.vbz;
+  const dim3 grid((unsigned)div_up(vs.vbx, 8 * VL_WARPS), (unsigned)vs.vby, (unsigned)vs.vbz);
+  Scratch<uint32_t> counts(ctx, n_bricks);
+  off.reset(ctx, n_bricks + 1);
+  const i64 n_scan_blocks = (n_bricks + SCAN_B - 1) / SCAN_B;
+  Scratch<uint32_t> sums(ctx, n_scan_blocks + 2);   // block sums, [n] = total, [n+1] = non-positive-weight flag
+  uint32_t *total = sums.get() + n_scan_blocks, *flag = total + 1;
+  voter_count_kernel<<<grid, 32 * VL_WARPS, 0, ctx->stream>>>(vs, counts.get());
+  VCK(cudaGetLastError());
+  scan_local_kernel<<<(unsigned)n_scan_blocks, SCAN_T, 0, ctx->stream>>>(counts.get(), off.get(), sums.get(), n_bricks);
+  VCK(cudaGetLastError());
+  scan_sums_kernel<<<1, SCAN_T, 0, ctx->stream>>>(sums.get(), n_scan_blocks, total);
+  VCK(cudaGetLastError());
+  scan_add_kernel<<<(unsigned)n_scan_blocks, SCAN_T, 0, ctx->stream>>>(off.get(), sums.get(), n_bricks, total);
+  VCK(cudaGetLastError());
+  ctx->count_launch(4);
+  uint32_t n_voters = 0, nonpos_flag = 0;
+  VCK(cudaMemcpyAsync(&n_voters, total, sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
+  VCK(cudaStreamSynchronize(ctx->stream));
+  // (a 32-bit voter count: 4.29e9 voters would need 137 GB of voter records anyway)
+  rec.reset(ctx, std::max<size_t>(n_voters, 1));
+  if (n_voters > 0) {
+    VCK(cudaMemsetAsync(flag, 0, sizeof(uint32_t), ctx->stream));
+    voter_fill_kernel<<<grid, 32 * VL_WARPS, 0, ctx->stream>>>(vs, off.get(), inv_total, rec.get(), flag);
+    VCK(cudaGetLastError());
+    ctx->count_launch();
+    VCK(cudaMemcpyAsync(&nonpos_flag, flag, sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
+    VCK(cudaStreamSynchronize(ctx->stream));
+  }
+  nonpos = nonpos_flag != 0;
+  return n_voters;
+}
+
+// Which gather kernel runs, and with what arguments.
+struct GatherPlan {
+  int kernel = 0;           // 0: tv_gather_kernel, 1: tv_gather_lut_kernel, 2: the same with a clamped table index
+  int expo;                 // tv_gather_kernel<EXPO, CURVES, POSW, SHELL>: EXPO 2 or 4, 0 for any other exponent
+  bool curves, posw, shell;
+  float lim_in, lim_pass;   // GatherArgs::lim_in / lim_pass
+  int row_cap;              // GatherArgs::row_cap
+  int n_lut = 0;            // table rows (kernels 1 and 2)
+  size_t smem;              // dynamic shared memory per CTA
+  float neg_c;              // GatherArgs::neg_c
+};
+
+// The table kernel wants exponent 4, positive weights, a support whose shell is all kept or all dropped, and a
+// radius whose table fits beside its 16 voter rings in smem_optin bytes of shared memory.  No voters: kernel 0.
+static GatherPlan plan_gather(const TVParams &p, int hw, const DecayInfo &info, uint32_t n_voters, bool nonpos,
+                              int smem_optin) {
+  GatherPlan pl;
+  // lattice points on the shell r2 == hw^2: all kept / all dropped / mixed (see vote())
+  const bool mixed_shell = info.shell_total != 0 && info.shell_kept != 0 && info.shell_kept != info.shell_total;
+  const bool shell_in = info.shell_total != 0 && info.shell_kept == info.shell_total;
+  const float hw2 = (float)(hw * hw);
+  pl.lim_in = hw2 + ((shell_in && !mixed_shell) ? 0.5f : -0.5f);
+  pl.lim_pass = hw2 + ((shell_in || mixed_shell) ? 0.5f : -0.5f);
+  const int per_axis = ((2 * hw + 3) >> VSH) + 2;
+  pl.row_cap = per_axis * per_axis;
+  const size_t per_warp = (TV_QCAP * sizeof(VoterRec) + (2 * (size_t)pl.row_cap + 4) * sizeof(uint32_t) + 15) & ~(size_t)15;
+  pl.expo = (p.exponent == 2 || p.exponent == 4) ? p.exponent : 0;
+  pl.curves = p.curves != 0;
+  pl.shell = mixed_shell;
+  // POSW: all voter weights > 0 (always true for the planar ridge score), so log2(weight) rides in the decay exponent
+  pl.posw = !mixed_shell && !nonpos;
+  pl.neg_c = (float)(-1.4426950408889634 / ((double)p.sigma * (double)p.sigma));
+  pl.smem = TV_WARPS * per_warp;
+  if (p.exponent == 4 && pl.posw && hw <= LUT_MAX_HW && n_voters > 0) {
+    const size_t budget = (size_t)smem_optin - 1024;   // the kernel's static shared memory (work tickets)
+    // largest r2 between a receiver of a 4x4x4 patch and a voter the cull lets through (gap vector g, |g|^2 < lim_pass)
+    int r2_reach = 27;
+    for (int gz = 0; gz <= hw; gz++)
+      for (int gy = 0; gy <= hw; gy++)
+        for (int gx = 0; gx <= hw; gx++)
+          if ((float)(gx * gx + gy * gy + gz * gz) < pl.lim_pass)
+            r2_reach = std::max(r2_reach, (gx + 3) * (gx + 3) + (gy + 3) * (gy + 3) + (gz + 3) * (gz + 3));
+    const int r2_in = (int)floorf(pl.lim_in);          // largest r2 with a non-zero weight (lim_in = hw^2 +- 0.5)
+    const int n_full = r2_reach + 1, n_clamped = r2_in + 2;
+    if ((size_t)n_full * LUT_ROW + LUT_WARPS * per_warp <= budget) { pl.kernel = 1; pl.n_lut = n_full; }
+    else if ((size_t)n_clamped * LUT_ROW + LUT_WARPS * per_warp <= budget) { pl.kernel = 2; pl.n_lut = n_clamped; }
+    if (pl.kernel) pl.smem = (size_t)pl.n_lut * LUT_ROW + LUT_WARPS * per_warp;
+  }
+  if (!pl.kernel && pl.expo == 4 && pl.posw) pl.neg_c *= 0.5f;   // SQRTW: the decay of sqrt(weight)
+  return pl;
+}
+
+// The table kernel's rows r2 = 0 .. n_lut - 1: {E', ninv'} in the scales of its records (LUT_*).
+static void upload_table(visfd_ctx *ctx, const GatherPlan &pl, float sigma, Scratch<float2> &lut) {
+  std::vector<float2> h(pl.n_lut);
+  for (int r2 = 0; r2 < pl.n_lut; r2++) {
+    const float e = ((float)r2 < pl.lim_in) ? (float)exp(-0.5 * (double)r2 / ((double)sigma * (double)sigma)) : 0.0f;
+    // powers of two: exact
+    h[r2] = make_float2(ldexpf(e, LUT_E_LOG2), r2 ? ldexpf((float)(-1.0 / (double)r2), LUT_TAU_LOG2) : 0.0f);
+  }
+  if (pl.kernel == 2) h[pl.n_lut - 1] = make_float2(0.0f, 0.0f);
+  lut.reset(ctx, h.size());
+  VCK(cudaMemcpyAsync(lut.get(), h.data(), h.size() * sizeof(float2), cudaMemcpyHostToDevice, ctx->stream));
+  VCK(cudaStreamSynchronize(ctx->stream));   // h goes out of scope
+}
+
+typedef void (*GatherKernel)(GatherArgs);
+template <int E, bool C>
+static GatherKernel mufu_kernel(const GatherPlan &pl) {
+  if (pl.shell) return tv_gather_kernel<E, C, false, true>;
+  return pl.posw ? tv_gather_kernel<E, C, true, false> : tv_gather_kernel<E, C, false, false>;
+}
+template <bool C>
+static GatherKernel gather_kernel(const GatherPlan &pl) {
+  if (pl.kernel) return pl.kernel == 2 ? tv_gather_lut_kernel<C, true> : tv_gather_lut_kernel<C, false>;
+  return pl.expo == 2 ? mufu_kernel<2, C>(pl) : pl.expo == 4 ? mufu_kernel<4, C>(pl) : mufu_kernel<0, C>(pl);
+}
+
+// One launch over the 8x8x4 receiver tiles of g: one 4-warp CTA per tile in tv_gather_kernel; the persistent table
+// kernel takes them from g.ticket.
+static void launch_gather(visfd_ctx *ctx, const GatherPlan &pl, const GatherArgs &g, unsigned tiles) {
+  const GatherKernel k = pl.curves ? gather_kernel<true>(pl) : gather_kernel<false>(pl);
+  const unsigned ctas = pl.kernel ? (unsigned)std::min<i64>(ctx->sm_count, ((i64)tiles + LUT_QUADS - 1) / LUT_QUADS) : tiles;
+  VCK(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl.smem));
+  k<<<ctas, pl.kernel ? 32 * LUT_WARPS : TV_THREADS, pl.smem, ctx->stream>>>(g);
+  VCK(cudaGetLastError());
+  ctx->count_launch();
+}
+
 bool tv_device(visfd_ctx *ctx, i64 nx, i64 ny, i64 nz_local, i64 z_offset, i64 nz_global,
                i64 own_z0, i64 own_z1, const float *saliency, float thr, const float *direction,
                const float *smoothed, float ridge_sigma, int eival_order, int score_kind,
@@ -935,60 +1061,30 @@ bool tv_device(visfd_ctx *ctx, i64 nx, i64 ny, i64 nz_local, i64 z_offset, i64 n
 
   const int nbx = (int)div_up(nx, BR), nby = (int)div_up(ny, BR);   // 8x8 receiver tiles per layer
   const int vbx = (int)div_up(nx, VBR), vby = (int)div_up(ny, VBR), vbz = (int)div_up(nz_local, VBR);
-  const i64 n_bricks = (i64)vbx * vby * vbz;
-  VREQUIRE(n_bricks < 2147483647LL, "too many bricks for one launch");
+  VREQUIRE((i64)vbx * vby * vbz < 2147483647LL, "too many bricks for one launch");
   VREQUIRE(vby <= 65535 && vbz <= 65535, "slab too large for the voter list kernels");
-  VoterSrc vs{saliency, mask_src, thr, (int)nx, (int)ny, nz_local, vbx, vby, vbz};
-  const dim3 vl_grid((unsigned)div_up(vbx, 8 * VL_WARPS), (unsigned)vby, (unsigned)vbz);
-
-  Scratch<uint32_t> counts(ctx, n_bricks), off(ctx, n_bricks + 1);
-  const i64 n_scan_blocks = (n_bricks + SCAN_B - 1) / SCAN_B;
-  Scratch<uint32_t> sums(ctx, n_scan_blocks + 2);   // block sums, [n] = total, [n+1] = non-positive-weight flag
-  // which kernel: the table kernel wants exponent 4, positive weights (known after the fill), a support
-  // whose shell is all kept or all dropped, and a radius whose table fits beside the voter rings
-  const bool mixed_shell = info.shell_total != 0 && info.shell_kept != 0 && info.shell_kept != info.shell_total;
-  const bool shell_in = info.shell_total != 0 && info.shell_kept == info.shell_total;
-  const char *no_lut_env = getenv("VISFD_CUDA_NO_LUT");   // tests: force the MUFU kernel
-  bool use_lut = p.exponent == 4 && !mixed_shell && hw <= LUT_MAX_HW && !(no_lut_env && atoi(no_lut_env));
-  uint32_t n_voters = 0, nonpos = 0;
+  int smem_optin = 0;
+  VCK(cudaDeviceGetAttribute(&smem_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, ctx->device));
+  Scratch<uint32_t> off;
   Scratch<VoterRec> rec;
+  uint32_t n_voters = 0;
+  GatherPlan pl;
   {
     StageTimer t(ctx, "compact");
-    voter_count_kernel<<<vl_grid, 32 * VL_WARPS, 0, ctx->stream>>>(vs, counts.get());
-    VCK(cudaGetLastError());
-    scan_local_kernel<<<(unsigned)n_scan_blocks, SCAN_T, 0, ctx->stream>>>(counts.get(), off.get(), sums.get(), n_bricks);
-    VCK(cudaGetLastError());
-    scan_sums_kernel<<<1, SCAN_T, 0, ctx->stream>>>(sums.get(), n_scan_blocks, sums.get() + n_scan_blocks);
-    VCK(cudaGetLastError());
-    scan_add_kernel<<<(unsigned)n_scan_blocks, SCAN_T, 0, ctx->stream>>>(off.get(), sums.get(), n_bricks,
-                                                                        sums.get() + n_scan_blocks);
-    VCK(cudaGetLastError());
-    ctx->count_launch(4);
-    VCK(cudaMemcpyAsync(&n_voters, sums.get() + n_scan_blocks, sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
-    VCK(cudaStreamSynchronize(ctx->stream));
-    // (a 32-bit voter count: 4.29e9 voters would need 137 GB of voter records anyway)
-    rec.reset(ctx, std::max<size_t>(n_voters, 1));
-    if (n_voters > 0) {
+    bool nonpos = false;
+    n_voters = build_voter_list(ctx, VoterSrc{saliency, mask_src, thr, (int)nx, (int)ny, nz_local, vbx, vby, vbz},
+                                1.0f / info.total, off, rec, nonpos);
+    pl = plan_gather(p, hw, info, n_voters, nonpos, smem_optin);
+    if (n_voters > 0) {   // the direction pass
       DirSrc ds{direction, smoothed, ridge_sigma, eival_order, z_offset, nz_global};
-      VCK(cudaMemsetAsync(sums.get() + n_scan_blocks + 1, 0, sizeof(uint32_t), ctx->stream));
-      for (;;) {
-        voter_fill_kernel<<<vl_grid, 32 * VL_WARPS, 0, ctx->stream>>>(vs, off.get(), 1.0f / info.total, use_lut, rec.get(),
-                                                                      sums.get() + n_scan_blocks + 1);
-        VCK(cudaGetLastError());
-        ctx->count_launch();
-        VCK(cudaMemcpyAsync(&nonpos, sums.get() + n_scan_blocks + 1, sizeof(uint32_t), cudaMemcpyDeviceToHost,
-                            ctx->stream));
-        VCK(cudaStreamSynchronize(ctx->stream));
-        if (!(use_lut && nonpos)) break;
-        use_lut = false;   // a weight <= 0 (negative saliency or mask weight): records for the MUFU kernel instead
-      }
-      voter_direction_kernel<<<div_up(n_voters, 256), 256, 0, ctx->stream>>>(ds, (int)nx, (int)ny, n_voters, use_lut,
-                                                                            rec.get());
+      voter_direction_kernel<<<div_up(n_voters, 256), 256, 0, ctx->stream>>>(ds, (int)nx, (int)ny, n_voters,
+                                                                            pl.kernel != 0, rec.get());
       VCK(cudaGetLastError());
       ctx->count_launch();
     }
   }
   ctx->last_voters = n_voters;
+  ctx->last_tv_kernel = pl.kernel;
 
   Scratch<uint32_t> shell(ctx, std::max<size_t>(info.shell_keep.size(), 1));
   if (!info.shell_keep.empty())
@@ -1003,15 +1099,13 @@ bool tv_device(visfd_ctx *ctx, i64 nx, i64 ny, i64 nz_local, i64 z_offset, i64 n
   g.own_z0 = own_z0; g.own_z1 = own_z1;
   g.ntx = nbx; g.nty = nby;
   g.hw = hw; g.hw2 = (float)(hw * hw);
-  { const int per_axis = ((2 * hw + 3) >> VSH) + 2; g.row_cap = per_axis * per_axis; }
-  // lattice points on the shell r2 == hw^2: all kept / all dropped / mixed (see vote())
-  g.lim_in = g.hw2 + ((shell_in && !mixed_shell) ? 0.5f : -0.5f);
-  g.lim_pass = g.hw2 + ((shell_in || mixed_shell) ? 0.5f : -0.5f);
-  g.neg_c = (float)(-1.4426950408889634 / ((double)p.sigma * (double)p.sigma));
+  g.row_cap = pl.row_cap;
+  g.lim_in = pl.lim_in; g.lim_pass = pl.lim_pass;
+  g.neg_c = pl.neg_c;
   g.half_exp = 0.5f * (float)p.exponent;
   g.mask_dst = mask_dst; g.tensor = tensor; g.score = score;
   g.order = eival_order; g.score_kind = score_kind;
-  g.lut = nullptr; g.n_lut = 0; g.n_tiles = 0; g.ticket = nullptr;
+  g.lut = nullptr; g.n_lut = pl.n_lut; g.n_tiles = 0; g.ticket = nullptr;
   // receiver planes in chunks (multiples of the 8-plane tile): one launch each, so that a
   // finished chunk of the result can travel to the host while the next one is computed
   const i64 planes = own_z1 - own_z0;
@@ -1029,120 +1123,31 @@ bool tv_device(visfd_ctx *ctx, i64 nx, i64 ny, i64 nz_local, i64 z_offset, i64 n
            "too many receiver tiles for one launch");
   EventList chunk_events(ctx);
   std::vector<cudaEvent_t> &chunk_done = chunk_events.ev;
-  // ---- table kernel set-up ---------------------------------------------------------------------
-  const size_t per_warp = (TV_QCAP * sizeof(VoterRec) + (2 * (size_t)g.row_cap + 4) * sizeof(uint32_t) + 15) & ~(size_t)15;
   Scratch<float2> lut;
   Scratch<unsigned> tickets;
-  int lut_mode = 0;   // 0: MUFU kernel, 1: table over the whole reach, 2: table up to the support, clamped index
-  size_t lut_smem = 0;
-  if (use_lut && n_voters > 0) {
-    int smem_max = 0;
-    VCK(cudaDeviceGetAttribute(&smem_max, cudaDevAttrMaxSharedMemoryPerBlockOptin, ctx->device));
-    const size_t budget = (size_t)smem_max - 1024;   // the kernel's static shared memory (work tickets)
-    // largest r2 between a receiver of a 4x4x4 patch and a voter the cull lets through (gap vector g, |g|^2 < lim_pass)
-    int r2_reach = 27;
-    for (int gz = 0; gz <= hw; gz++)
-      for (int gy = 0; gy <= hw; gy++)
-        for (int gx = 0; gx <= hw; gx++)
-          if ((float)(gx * gx + gy * gy + gz * gz) < g.lim_pass)
-            r2_reach = std::max(r2_reach, (gx + 3) * (gx + 3) + (gy + 3) * (gy + 3) + (gz + 3) * (gz + 3));
-    const int r2_in = (int)floorf(g.lim_in);          // largest r2 with a non-zero weight (lim_in = hw^2 +- 0.5)
-    const int n_full = r2_reach + 1, n_clamped = r2_in + 2;
-    const char *mode_env = getenv("VISFD_CUDA_LUT_MODE");   // tests / tuning: 1 or 2
-    const int want = mode_env ? atoi(mode_env) : 0;
-    if (want != 2 && (size_t)n_full * LUT_ROW + LUT_WARPS * per_warp <= budget) { lut_mode = 1; g.n_lut = n_full; }
-    else if ((size_t)n_clamped * LUT_ROW + LUT_WARPS * per_warp <= budget) { lut_mode = 2; g.n_lut = n_clamped; }
-    if (lut_mode) {
-      std::vector<float2> h(g.n_lut);
-      for (int r2 = 0; r2 < g.n_lut; r2++) {
-        const float e = ((float)r2 < g.lim_in) ? (float)exp(-0.5 * (double)r2 / ((double)p.sigma * (double)p.sigma)) : 0.0f;
-        // {E', ninv'} in the scales of the table kernel's records (LUT_*); powers of two: exact
-        h[r2] = make_float2(ldexpf(e, LUT_E_LOG2), r2 ? ldexpf((float)(-1.0 / (double)r2), LUT_TAU_LOG2) : 0.0f);
-      }
-      if (lut_mode == 2) h[g.n_lut - 1] = make_float2(0.0f, 0.0f);
-      lut.reset(ctx, h.size());
-      VCK(cudaMemcpyAsync(lut.get(), h.data(), h.size() * sizeof(float2), cudaMemcpyHostToDevice, ctx->stream));
-      VCK(cudaStreamSynchronize(ctx->stream));   // h goes out of scope
-      g.lut = lut.get();
-      lut_smem = (size_t)g.n_lut * LUT_ROW + LUT_WARPS * per_warp;
-    }
-  }
-  if (use_lut && n_voters > 0 && !lut_mode) {
-    // records were written for the table kernel but no table fits: rewrite them for the MUFU kernel
-    voter_fill_kernel<<<vl_grid, 32 * VL_WARPS, 0, ctx->stream>>>(vs, off.get(), 1.0f / info.total, false, rec.get(),
-                                                                  sums.get() + n_scan_blocks + 1);
-    VCK(cudaGetLastError());
-    DirSrc ds{direction, smoothed, ridge_sigma, eival_order, z_offset, nz_global};
-    voter_direction_kernel<<<div_up(n_voters, 256), 256, 0, ctx->stream>>>(ds, (int)nx, (int)ny, n_voters, false, rec.get());
-    VCK(cudaGetLastError());
-    ctx->count_launch(2);
-  }
-  ctx->last_tv_kernel = lut_mode;
-  const GatherArgs g_all = g;
-  if (lut_mode) {
+  if (pl.kernel) {
+    upload_table(ctx, pl, p.sigma, lut);
+    g.lut = lut.get();
     tickets.reset(ctx, (size_t)n_chunks);
     VCK(cudaMemsetAsync(tickets.get(), 0, (size_t)n_chunks * sizeof(unsigned), ctx->stream));
   }
   {
     StageTimer t(ctx, "tv");
-    // POSW: all voter weights > 0 (always true for the planar ridge score), so log2(weight)
-    // rides in the decay exponent
-    const size_t smem = (TV_THREADS / 32) * per_warp;
     for (int c = 0; c < n_chunks; c++) {
-    g = g_all;
-    g.own_z0 = g_all.own_z0 + c * chunk_planes;
-    g.own_z1 = std::min(g_all.own_z1, g.own_z0 + chunk_planes);
-    const size_t chunk_off = (size_t)(g.own_z0 - g_all.own_z0) * (size_t)nx * (size_t)ny;
-    if (g_all.score) g.score = g_all.score + chunk_off;
-    if (g_all.tensor) g.tensor = g_all.tensor + 6 * chunk_off;
-    const unsigned grid = (unsigned)((i64)g.ntx * g.nty * div_up(g.own_z1 - g.own_z0, TV_TILE_Z) * 4 / TV_WARPS);
-    if (lut_mode) {
-      g.n_tiles = grid;   // one 4-warp tile per CTA of the MUFU kernel
-      g.ticket = tickets.get() + c;
-      const unsigned ctas = (unsigned)std::min<i64>(ctx->sm_count, ((i64)grid + LUT_QUADS - 1) / LUT_QUADS);
-#define TV_LUT_LAUNCH(C, K)                                                                                        \
-      do {                                                                                                         \
-        VCK(cudaFuncSetAttribute(tv_gather_lut_kernel<C, K>, cudaFuncAttributeMaxDynamicSharedMemorySize,          \
-                                 (int)lut_smem));                                                                  \
-        tv_gather_lut_kernel<C, K><<<ctas, 32 * LUT_WARPS, lut_smem, ctx->stream>>>(g);                            \
-      } while (0)
-      if (p.curves) { if (lut_mode == 2) TV_LUT_LAUNCH(true, true); else TV_LUT_LAUNCH(true, false); }
-      else { if (lut_mode == 2) TV_LUT_LAUNCH(false, true); else TV_LUT_LAUNCH(false, false); }
-#undef TV_LUT_LAUNCH
-    } else {
-#define TV_LAUNCH1(E, C, P, S)                                                                            \
-    do {                                                                                                  \
-      VCK(cudaFuncSetAttribute(tv_gather_kernel<E, C, P, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
-                               (int)smem));                                                               \
-      tv_gather_kernel<E, C, P, S><<<grid, TV_THREADS, smem, ctx->stream>>>(g);                           \
-    } while (0)
-#define TV_LAUNCH(E, C)                                   \
-    do {                                                  \
-      if (mixed_shell) TV_LAUNCH1(E, C, false, true);     \
-      else if (nonpos) TV_LAUNCH1(E, C, false, false);    \
-      else {                                              \
-        if (E == 4) g.neg_c *= 0.5f;                      \
-        TV_LAUNCH1(E, C, true, false);                    \
-      }                                                   \
-    } while (0)
-    if (p.curves) {
-      if (p.exponent == 2) TV_LAUNCH(2, true);
-      else if (p.exponent == 4) TV_LAUNCH(4, true);
-      else TV_LAUNCH(0, true);
-    } else {
-      if (p.exponent == 2) TV_LAUNCH(2, false);
-      else if (p.exponent == 4) TV_LAUNCH(4, false);
-      else TV_LAUNCH(0, false);
+      GatherArgs gc = g;
+      gc.own_z0 = g.own_z0 + c * chunk_planes;
+      gc.own_z1 = std::min(g.own_z1, gc.own_z0 + chunk_planes);
+      const size_t chunk_off = (size_t)(gc.own_z0 - g.own_z0) * (size_t)nx * (size_t)ny;
+      if (g.score) gc.score = g.score + chunk_off;
+      if (g.tensor) gc.tensor = g.tensor + 6 * chunk_off;
+      const unsigned grid = (unsigned)((i64)gc.ntx * gc.nty * div_up(gc.own_z1 - gc.own_z0, TV_TILE_Z) * 4 / TV_WARPS);
+      if (pl.kernel) {
+        gc.n_tiles = grid;   // one 4-warp tile per CTA of the MUFU kernel
+        gc.ticket = tickets.get() + c;
+      }
+      launch_gather(ctx, pl, gc, grid);
+      if (overlap_d2h) VCK(cudaEventRecord(chunk_events.add(), ctx->stream));
     }
-#undef TV_LAUNCH
-#undef TV_LAUNCH1
-    }
-    VCK(cudaGetLastError());
-    ctx->count_launch();
-    if (overlap_d2h) {
-      VCK(cudaEventRecord(chunk_events.add(), ctx->stream));
-    }
-    }  // chunks
   }
   if (overlap_d2h) {
     // all launches are queued; now the copies, each behind its chunk (with pageable host memory
@@ -1153,7 +1158,7 @@ bool tv_device(visfd_ctx *ctx, i64 nx, i64 ny, i64 nz_local, i64 z_offset, i64 n
       const size_t off = (size_t)c * (size_t)chunk_planes * plane;
       const size_t cnt = (size_t)std::min(chunk_planes, planes - c * chunk_planes) * plane;
       VCK(cudaStreamWaitEvent(ctx->copy_stream, chunk_done[c], 0));
-      VCK(cudaMemcpyAsync(score_host + off, g_all.score + off, cnt * sizeof(float), cudaMemcpyDeviceToHost,
+      VCK(cudaMemcpyAsync(score_host + off, g.score + off, cnt * sizeof(float), cudaMemcpyDeviceToHost,
                           ctx->copy_stream));
     }
     VCK(cudaStreamSynchronize(ctx->copy_stream));
