@@ -74,6 +74,11 @@ void visfd_cuda_set_fast_gauss(visfd_ctx *ctx, int enabled);
 int visfd_cuda_trim(visfd_ctx *ctx);
 /* Number of kernel launches issued by ctx since creation (bench bookkeeping). */
 int64_t visfd_cuda_launch_count(visfd_ctx *ctx);
+/* Bookkeeping (like visfd_cuda_launch_count): the highest number of bytes the context's pool has held from
+ * cudaMalloc (live + cached) since creation or the last reset.  A reset starts from what the pool holds at that
+ * moment (visfd_cuda_trim first to start from zero). */
+int64_t visfd_cuda_peak_reserved_bytes(visfd_ctx *ctx);
+void visfd_cuda_reset_peak_reserved_bytes(visfd_ctx *ctx);
 /* Device milliseconds spent in a named stage since the last visfd_cuda_reset_stage_ms,
  * measured with CUDA events on the context's stream around the stage's kernels:
  * "gauss", "ridge", "select", "compact", "tv", "threshold", "blob_scan", "h2d", "d2h".
@@ -281,6 +286,21 @@ int visfd_cuda_vote_slab_host(visfd_ctx *ctx, int64_t nx, int64_t ny, int64_t nz
 int visfd_cuda_membrane_multi(int ndev, const int *devices, int64_t nx, int64_t ny, int64_t nz,
                               const float *src_host, const float *mask_host, const visfd_membrane_params *p,
                               float *out_host, float *threshold_out, double *device_ms);
+
+/* visfd_cuda_membrane with HOST arrays on ONE device, for volumes whose working set does not fit on it: the volume
+ * is cut into Z-slabs exactly as visfd_cuda_membrane_multi cuts it, and the slabs run one after another on ctx, each
+ * freed before the next.  The device memory the call reserves (the context's pool, cached blocks included) stays at
+ * or below device_bytes; 0 = the free memory the device reports at entry, less a margin.  The result and the
+ * threshold are bit-identical to visfd_cuda_membrane.  *n_slabs_out (may be NULL): slabs used.
+ * The call runs passes over the slabs; in each pass a slab uploads its planes (halo included) and computes its ridge
+ * saliency again.  A fraction cut takes one pass per radix-select round (three); an absolute cut takes one pass
+ * that counts the voters when the budget would otherwise be sized for every voxel voting; the vote pass delivers
+ * each slab's planes into out_host.  The number of slabs is the smallest whose slabs fit device_bytes; the call
+ * fails, naming the bytes needed, when slabs of 8 planes do not fit.  The cache is released on entry, between the
+ * steps of a slab and after every slab, so the call leaves no device memory reserved. */
+int visfd_cuda_membrane_stream(visfd_ctx *ctx, int64_t nx, int64_t ny, int64_t nz, const float *src_host,
+                               const float *mask_host, const visfd_membrane_params *p, int64_t device_bytes,
+                               float *out_host, float *threshold_out, int64_t *n_slabs_out);
 
 /* ---- clustering: LabelConnected ------------------------------------------------------ */
 /* lib/visfd/connect.hpp:171-1432 with the arguments HandleTV passes (bin/filter_mrc/handlers.cpp:1927-2034;

@@ -4,7 +4,8 @@ blob detection hot path behind a C ABI (include/visfd_cuda.h).
   visfd_b200/csrc/        CUDA kernels + the extern "C" layer  -> visfd_b200/libvisfd_cuda.so
   visfd_b200/csrc/visfd_cuda_shim.hpp
                           C++ mirror of the reference's `namespace visfd` entry points
-  visfd_b200/csrc/multi.cu        the pipeline on several GPUs behind one C call (visfd_cuda_membrane_multi)
+  visfd_b200/csrc/multi.cu        the pipeline in Z-slabs behind one C call: on several GPUs (visfd_cuda_membrane_multi),
+                                  or on one GPU slab after slab within a memory budget (visfd_cuda_membrane_stream)
   visfd_b200/csrc/connect.cu      LabelConnected: device predicates + ordered host flood
   visfd_b200/capi.py      ctypes binding (tests, bench, multi-GPU driver)
   visfd_b200/slab.py      Z-slab multi-GPU drivers: membrane pipeline, blob detection, image statistics

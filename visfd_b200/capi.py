@@ -50,6 +50,8 @@ def load_library():
     lib = C.CDLL(LIB_PATH)
     lib.visfd_cuda_last_error.restype = C.c_char_p
     lib.visfd_cuda_launch_count.restype = _i64
+    lib.visfd_cuda_peak_reserved_bytes.restype = _i64
+    lib.visfd_cuda_reset_peak_reserved_bytes.restype = None
     lib.visfd_cuda_last_voter_count.restype = _i64
     lib.visfd_cuda_last_tv_kernel.restype = C.c_int
     lib.visfd_cuda_stage_ms.restype = _d
@@ -235,6 +237,15 @@ class Context:
     # ---- bookkeeping -----------------------------------------------------------------
     def launch_count(self):
         return self.lib.visfd_cuda_launch_count(self.h)
+
+    def peak_reserved_bytes(self):
+        """Highest number of bytes the context's pool has held from cudaMalloc (live + cached) since creation or
+        the last reset_peak_reserved_bytes()."""
+        return self.lib.visfd_cuda_peak_reserved_bytes(self.h)
+
+    def reset_peak_reserved_bytes(self):
+        """Restart the peak from what the pool holds now (trim() first to start from zero)."""
+        self.lib.visfd_cuda_reset_peak_reserved_bytes(self.h)
 
     def stage_ms(self, stage):
         return self.lib.visfd_cuda_stage_ms(self.h, stage.encode())
@@ -486,6 +497,24 @@ class Context:
             self._ck(self.lib.visfd_cuda_membrane(self.h, *self._dims(src.shape), _ptr(src), _ptr(mask), C.byref(p),
                                                   _ptr(res), _ptr(sal), _ptr(dire), _ptr(tensor), C.byref(thr)))
         return dict(out=res, hess_saliency=sal, direction=dire, tensor=tensor, threshold=thr.value)
+
+    def membrane_stream(self, src, sigma, truncate_ratio, order, cut, cut_is_fraction, tv_sigma, tv_exponent,
+                        tv_cutoff_ratio, mask=None, out=None, device_bytes=0):
+        """visfd_cuda_membrane_stream: the fused pipeline on this context's GPU in Z-slabs run one after another,
+        for volumes whose working set does not fit on it; the device memory the call reserves stays within
+        device_bytes (0: the free memory at entry, less a margin).  -> dict(out, threshold, n_slabs).  numpy (host)
+        arrays only; the result is bit-identical to membrane()."""
+        src = np.ascontiguousarray(src, np.float32)
+        mask = None if mask is None else np.ascontiguousarray(mask, np.float32)
+        res = out if out is not None else np.empty(src.shape, np.float32)
+        assert isinstance(res, np.ndarray) and res.dtype == np.float32 and res.flags.c_contiguous and res.shape == src.shape
+        p = MembraneParams(sigma, truncate_ratio, order, cut, int(cut_is_fraction), tv_sigma, tv_exponent,
+                           tv_cutoff_ratio)
+        thr, n_slabs = _f(), _i64()
+        self._ck(self.lib.visfd_cuda_membrane_stream(self.h, *self._dims(src.shape), _ptr(src), _ptr(mask), C.byref(p),
+                                                     _i64(int(device_bytes)), _ptr(res), C.byref(thr),
+                                                     C.byref(n_slabs)))
+        return dict(out=res, threshold=thr.value, n_slabs=n_slabs.value)
 
     # ---- slab stages (device tensors only) -----------------------------------------------------------------
     def ridge_saliency_slab(self, src, z_offset, nz_global, sigma, truncate_ratio, order=DECREASING_EIVALS,

@@ -58,7 +58,11 @@ struct visfd_ctx {
   struct Block { void *p; size_t bytes; };
   std::vector<Block> free_blocks;           // cached, not in use
   std::map<void *, size_t> live_blocks;     // handed out
+  int64_t reserved_bytes = 0;               // held from cudaMalloc: live + cached
+  int64_t peak_reserved_bytes = 0;          // highest reserved_bytes since creation or the last reset
 
+  // What alloc(bytes) takes from the device: requests are rounded up to whole 512-byte units.
+  static size_t block_bytes(size_t bytes) { return ((bytes ? bytes : 16) + 511) & ~size_t(511); }
   void *alloc(size_t bytes);
   void release(void *p);
   void trim();

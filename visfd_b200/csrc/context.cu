@@ -62,8 +62,7 @@ void resolve_stage_times(visfd_ctx *ctx) {
 using namespace visfd_cuda;
 
 void *visfd_ctx::alloc(size_t bytes) {
-  if (bytes == 0) bytes = 16;
-  bytes = (bytes + 511) & ~size_t(511);
+  bytes = block_bytes(bytes);
   // best fit among cached blocks that are not wastefully large
   int best = -1;
   for (int i = 0; i < (int)free_blocks.size(); i++) {
@@ -94,6 +93,8 @@ void *visfd_ctx::alloc(size_t bytes) {
     }
   }
   live_blocks[p] = bytes;
+  reserved_bytes += (int64_t)bytes;
+  peak_reserved_bytes = std::max(peak_reserved_bytes, reserved_bytes);
   return p;
 }
 
@@ -108,7 +109,10 @@ void visfd_ctx::release(void *p) {
 }
 
 void visfd_ctx::trim() {
-  for (auto &b : free_blocks) cudaFree(b.p);
+  for (auto &b : free_blocks) {
+    cudaFree(b.p);
+    reserved_bytes -= (int64_t)b.bytes;
+  }
   free_blocks.clear();
 }
 
@@ -192,6 +196,12 @@ int visfd_cuda_trim(visfd_ctx *ctx) {
 }
 
 int64_t visfd_cuda_launch_count(visfd_ctx *ctx) { return ctx ? ctx->launches : -1; }
+
+int64_t visfd_cuda_peak_reserved_bytes(visfd_ctx *ctx) { return ctx ? ctx->peak_reserved_bytes : -1; }
+
+void visfd_cuda_reset_peak_reserved_bytes(visfd_ctx *ctx) {
+  if (ctx) ctx->peak_reserved_bytes = ctx->reserved_bytes;
+}
 
 void visfd_cuda_set_fast_gauss(visfd_ctx *ctx, int enabled) {
   if (ctx) ctx->fast_gauss = enabled != 0;

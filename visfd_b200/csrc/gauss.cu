@@ -1197,6 +1197,12 @@ float separable_device(visfd_ctx *ctx, i64 nx, i64 ny, i64 nz_local, i64 z_offse
   return taps[0][hw[0]] * taps[1][hw[1]] * taps[2][hw[2]];  // filter3d.hpp:1044-1046
 }
 
+size_t separable_workspace_bytes(i64 nx, i64 ny, i64 nz_local, const int hw[3], bool masked, bool normalize) {
+  const size_t consts = (size_t)(2 * hw[0] + 1 + 2 * hw[1] + 1 + 2 * hw[2] + 1 + nx + ny + nz_local) * sizeof(float);
+  const size_t vol = visfd_ctx::block_bytes((size_t)nx * (size_t)ny * (size_t)nz_local * sizeof(float));
+  return visfd_ctx::block_bytes(consts) + vol * (masked && normalize ? 3 : 1);   // dconst, tmp (+ den, den2)
+}
+
 float gauss_device(visfd_ctx *ctx, i64 nx, i64 ny, i64 nz_local, i64 z_offset, i64 nz_global,
                    const float *src, float *dst, const float *mask, const float sigma[3],
                    const int hw[3], bool normalize, const float *combine_minuend, float combine_scale,

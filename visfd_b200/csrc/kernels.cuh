@@ -14,6 +14,8 @@ float separable_device(visfd_ctx *ctx, i64 nx, i64 ny, i64 nz_local, i64 z_offse
                        const float *src, float *dst, const float *mask, const float *const taps[3],
                        const int hw[3], bool normalize, const float *combine_minuend,
                        float combine_scale, bool z_swept = false /* dst already holds the Z sweep (dog_device) */);
+// Device bytes separable_device (and gauss_device) takes from the pool for a slab of nz_local planes.
+size_t separable_workspace_bytes(i64 nx, i64 ny, i64 nz_local, const int hw[3], bool masked, bool normalize);
 float gauss_device(visfd_ctx *ctx, i64 nx, i64 ny, i64 nz_local, i64 z_offset, i64 nz_global,
                    const float *src, float *dst, const float *mask, const float sigma[3],
                    const int hw[3], bool normalize, const float *combine_minuend,
@@ -53,9 +55,11 @@ float key_to_float(uint32_t k);
 i64 count_unmasked_device(visfd_ctx *ctx, i64 n, const float *mask);
 // Threshold such that the reference's cut (handlers.cpp:1751-1797) is reproduced, by a radix select over
 // histograms that summed_hist fills: the HIST_BINS-bin histogram of the keys that match the prefix, summed
-// over every part of the volume (select_hist_device on each part).
+// over every part of the volume (select_hist_device on each part).  *n_at_or_above (if given): the number of
+// un-masked voxels whose saliency is at or above the threshold, ties included.
 float select_threshold(float fraction,
-                       const std::function<void(uint32_t prefix, int prefix_bits, uint64_t *hist)> &summed_hist);
+                       const std::function<void(uint32_t prefix, int prefix_bits, uint64_t *hist)> &summed_hist,
+                       uint64_t *n_at_or_above = nullptr);
 float select_threshold_device(visfd_ctx *ctx, i64 n, const float *sal, const float *mask,
                               float fraction);
 void apply_cut_device(visfd_ctx *ctx, i64 n, float *sal, float thr);
@@ -83,6 +87,9 @@ bool tv_device(visfd_ctx *ctx, i64 nx, i64 ny, i64 nz_local, i64 z_offset, i64 n
                const float *smoothed, float ridge_sigma, int eival_order, int score_kind,
                const float *mask_src, const float *mask_dst, const TVParams &p, float *tensor,
                float *score, float *score_host = nullptr);
+// Upper bound of the device bytes tv_device takes from the pool for a slab of nz_local voter planes, own_planes
+// receiver planes and at most n_voters voters: the voter list (48 B per voter), its brick offsets and the rest.
+size_t tv_workspace_bytes(i64 nx, i64 ny, i64 nz_local, i64 own_planes, uint64_t n_voters);
 int tv_halfwidth(float sigma, float cutoff_ratio);
 
 // ---- threshold.cu -----------------------------------------------------------------

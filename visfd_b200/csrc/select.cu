@@ -146,13 +146,16 @@ int select_step_host(const uint64_t *hist, uint32_t *prefix, int *prefix_bits, u
 }
 
 float select_threshold(float fraction,
-                       const std::function<void(uint32_t prefix, int prefix_bits, uint64_t *hist)> &summed_hist) {
+                       const std::function<void(uint32_t prefix, int prefix_bits, uint64_t *hist)> &summed_hist,
+                       uint64_t *n_at_or_above) {
   uint64_t hist[HIST_BINS];
   uint32_t prefix = 0;
   int prefix_bits = 0;
   uint64_t rank = 0;
+  uint64_t above = 0, equal = 0;   // keys above the threshold's / equal to it
   bool first = true;
   while (prefix_bits < 32) {
+    const int bin_bits = bits_for_pass(prefix_bits);
     summed_hist(prefix, prefix_bits, hist);
     if (first) {
       uint64_t total = 0;
@@ -166,9 +169,13 @@ float select_threshold(float fraction,
       rank = (fl >= (double)total) ? total - 1 : (uint64_t)fl;
       first = false;
     }
+    const uint64_t skip = rank;
     int rc = select_step_host(hist, &prefix, &prefix_bits, &rank);
     VREQUIRE(rc == 0, "saliency cut: rank outside the population");
+    above += skip - rank;   // the keys of the bins above the chosen one
+    equal = hist[prefix & ((1u << bin_bits) - 1u)];
   }
+  if (n_at_or_above) *n_at_or_above = above + equal;
   return key_to_float(prefix);
 }
 

@@ -1042,6 +1042,18 @@ static void launch_gather(visfd_ctx *ctx, const GatherPlan &pl, const GatherArgs
   ctx->count_launch();
 }
 
+// The pool blocks of tv_device below, each at its largest.
+size_t tv_workspace_bytes(i64 nx, i64 ny, i64 nz_local, i64 own_planes, uint64_t n_voters) {
+  static_assert(sizeof(VoterRec) == 48, "voter record size");
+  const size_t n_bricks = (size_t)div_up(nx, VBR) * (size_t)div_up(ny, VBR) * (size_t)div_up(nz_local, VBR);
+  const size_t n_scan_blocks = (n_bricks + SCAN_B - 1) / SCAN_B;
+  const size_t max_lut = 3 * (LUT_MAX_HW + 3) * (LUT_MAX_HW + 3) + 1;   // plan_gather's r2_reach + 1 at most
+  auto b = visfd_ctx::block_bytes;
+  return b(n_bricks * 4) + b((n_bricks + 1) * 4) + b((n_scan_blocks + 2) * 4) +   // counts, off, sums
+         b(std::max<uint64_t>(n_voters, 1) * sizeof(VoterRec)) + b(TV_MAX_SHELL * 4) +   // rec, shell
+         b(max_lut * sizeof(float2)) + b(std::max<size_t>(div_up(own_planes, BR), 1) * 4);   // lut, tickets
+}
+
 bool tv_device(visfd_ctx *ctx, i64 nx, i64 ny, i64 nz_local, i64 z_offset, i64 nz_global,
                i64 own_z0, i64 own_z1, const float *saliency, float thr, const float *direction,
                const float *smoothed, float ridge_sigma, int eival_order, int score_kind,
