@@ -302,6 +302,26 @@ int visfd_cuda_membrane_stream(visfd_ctx *ctx, int64_t nx, int64_t ny, int64_t n
                                const float *mask_host, const visfd_membrane_params *p, int64_t device_bytes,
                                float *out_host, float *threshold_out, int64_t *n_slabs_out);
 
+/* The two calls above with `-membrane-background`: out and *threshold_out are bit-identical to
+ * visfd_cuda_membrane_background with the same arguments, for any number of slabs, with or without a mask and for
+ * both values of normalize_near_boundaries.  background_sigma == 0 gives exactly what the plain call gives (the
+ * same bits and, for stream, the same *n_slabs_out); background_sigma < 0 or NaN fails.  Everything else is as for
+ * the plain calls: HOST arrays only, errors name the slab (and its device), one multi call runs at a time, and
+ * stream stays within device_bytes or fails naming the bytes it needs.
+ * The raw-source halo of a slab widens to max(1 + gauss_halfwidth, floor(background_sigma * truncate_ratio)), so
+ * that the peak height is exact on every voter plane.  Each slab computes its peak height once per pass, as one
+ * volume held until its vote ends: stream needs one more slab volume per slab than the plain call (and the
+ * background Gaussian's scratch), so the same budget may take more slabs. */
+int visfd_cuda_membrane_multi_background(int ndev, const int *devices, int64_t nx, int64_t ny, int64_t nz,
+                                         const float *src_host, const float *mask_host, const visfd_membrane_params *p,
+                                         float background_sigma, int normalize_near_boundaries, float *out_host,
+                                         float *threshold_out, double *device_ms);
+int visfd_cuda_membrane_stream_background(visfd_ctx *ctx, int64_t nx, int64_t ny, int64_t nz, const float *src_host,
+                                          const float *mask_host, const visfd_membrane_params *p,
+                                          float background_sigma, int normalize_near_boundaries,
+                                          int64_t device_bytes, float *out_host, float *threshold_out,
+                                          int64_t *n_slabs_out);
+
 /* ---- clustering: LabelConnected ------------------------------------------------------ */
 /* lib/visfd/connect.hpp:171-1432 with the arguments HandleTV passes (bin/filter_mrc/handlers.cpp:1927-2034;
  * `-connect`, SURVEY 8f rank 1): connectivity 1, clusters grown from the saliency MAXIMA, the tensor positive

@@ -180,10 +180,11 @@ def tv_halfwidth(sigma, cutoff_ratio):
 
 
 def membrane_multi(devices, src, sigma, truncate_ratio, order, cut, cut_is_fraction, tv_sigma, tv_exponent,
-                   tv_cutoff_ratio, mask=None, out=None, lib=None):
+                   tv_cutoff_ratio, mask=None, out=None, lib=None, background_sigma=0.0, normalize=True):
     """visfd_cuda_membrane_multi: the fused pipeline of HandleTV on several GPUs of this node behind one C call
     (one worker thread per device, Z-slabs, host arrays in and out).  devices: list of CUDA device indices (a device
-    may appear more than once).  -> dict(out, threshold, device_ms).  numpy (host) arrays only."""
+    may appear more than once).  background_sigma > 0: `-membrane-background`
+    (visfd_cuda_membrane_multi_background).  -> dict(out, threshold, device_ms).  numpy (host) arrays only."""
     lib = lib or load_library()
     src = np.ascontiguousarray(src, np.float32)
     mask = None if mask is None else np.ascontiguousarray(mask, np.float32)
@@ -194,8 +195,13 @@ def membrane_multi(devices, src, sigma, truncate_ratio, order, cut, cut_is_fract
     ms = (C.c_double * len(devices))()
     thr = _f()
     nz, ny, nx = src.shape
-    rc = lib.visfd_cuda_membrane_multi(_i(len(devices)), devs, _i64(nx), _i64(ny), _i64(nz), _ptr(src), _ptr(mask),
-                                       C.byref(p), _ptr(res), C.byref(thr), ms)
+    if background_sigma > 0.0:
+        rc = lib.visfd_cuda_membrane_multi_background(_i(len(devices)), devs, _i64(nx), _i64(ny), _i64(nz), _ptr(src),
+                                                      _ptr(mask), C.byref(p), _f(background_sigma),
+                                                      _i(int(normalize)), _ptr(res), C.byref(thr), ms)
+    else:
+        rc = lib.visfd_cuda_membrane_multi(_i(len(devices)), devs, _i64(nx), _i64(ny), _i64(nz), _ptr(src),
+                                           _ptr(mask), C.byref(p), _ptr(res), C.byref(thr), ms)
     if rc != 0:
         raise VisfdCudaError(lib.visfd_cuda_last_error().decode())
     return dict(out=res, threshold=thr.value, device_ms=list(ms))
@@ -499,11 +505,12 @@ class Context:
         return dict(out=res, hess_saliency=sal, direction=dire, tensor=tensor, threshold=thr.value)
 
     def membrane_stream(self, src, sigma, truncate_ratio, order, cut, cut_is_fraction, tv_sigma, tv_exponent,
-                        tv_cutoff_ratio, mask=None, out=None, device_bytes=0):
+                        tv_cutoff_ratio, mask=None, out=None, device_bytes=0, background_sigma=0.0, normalize=True):
         """visfd_cuda_membrane_stream: the fused pipeline on this context's GPU in Z-slabs run one after another,
         for volumes whose working set does not fit on it; the device memory the call reserves stays within
-        device_bytes (0: the free memory at entry, less a margin).  -> dict(out, threshold, n_slabs).  numpy (host)
-        arrays only; the result is bit-identical to membrane()."""
+        device_bytes (0: the free memory at entry, less a margin).  background_sigma > 0: `-membrane-background`
+        (visfd_cuda_membrane_stream_background).  -> dict(out, threshold, n_slabs).  numpy (host) arrays only; the
+        result is bit-identical to membrane() with the same arguments."""
         src = np.ascontiguousarray(src, np.float32)
         mask = None if mask is None else np.ascontiguousarray(mask, np.float32)
         res = out if out is not None else np.empty(src.shape, np.float32)
@@ -511,9 +518,14 @@ class Context:
         p = MembraneParams(sigma, truncate_ratio, order, cut, int(cut_is_fraction), tv_sigma, tv_exponent,
                            tv_cutoff_ratio)
         thr, n_slabs = _f(), _i64()
-        self._ck(self.lib.visfd_cuda_membrane_stream(self.h, *self._dims(src.shape), _ptr(src), _ptr(mask), C.byref(p),
-                                                     _i64(int(device_bytes)), _ptr(res), C.byref(thr),
-                                                     C.byref(n_slabs)))
+        if background_sigma > 0.0:
+            self._ck(self.lib.visfd_cuda_membrane_stream_background(
+                self.h, *self._dims(src.shape), _ptr(src), _ptr(mask), C.byref(p), _f(background_sigma),
+                _i(int(normalize)), _i64(int(device_bytes)), _ptr(res), C.byref(thr), C.byref(n_slabs)))
+        else:
+            self._ck(self.lib.visfd_cuda_membrane_stream(self.h, *self._dims(src.shape), _ptr(src), _ptr(mask),
+                                                         C.byref(p), _i64(int(device_bytes)), _ptr(res), C.byref(thr),
+                                                         C.byref(n_slabs)))
         return dict(out=res, threshold=thr.value, n_slabs=n_slabs.value)
 
     # ---- slab stages (device tensors only) -----------------------------------------------------------------

@@ -446,11 +446,13 @@ int visfd_cuda_ridge_saliency_slab(visfd_ctx *ctx, int64_t nx, int64_t ny, int64
   API_END(ctx)
 }
 
-int visfd_cuda_vote_slab_host(visfd_ctx *ctx, int64_t nx, int64_t ny, int64_t nz_local, int64_t z_offset,
-                              int64_t nz_global, int64_t own_z0, int64_t own_z1, int64_t vote_z0, int64_t vote_z1,
-                              const float *saliency, const float *smoothed, const float *mask, float threshold,
-                              const visfd_membrane_params *p, float *out, float *tensor, float *out_host) {
-  API_BEGIN(ctx)
+}  // extern "C"
+
+namespace visfd_cuda {
+void vote_slab_device(visfd_ctx *ctx, int64_t nx, int64_t ny, int64_t nz_local, int64_t z_offset, int64_t nz_global,
+                      int64_t own_z0, int64_t own_z1, int64_t vote_z0, int64_t vote_z1, const float *saliency,
+                      const float *smoothed, const float *mask, float threshold, const visfd_membrane_params *p,
+                      float *out, float *tensor, float *out_host, const float *peak) {
   VREQUIRE(!out_host || !is_device_pointer(out_host), "out_host must be a host pointer");
   check_dims(nx, ny, nz_local);
   VREQUIRE(saliency && smoothed && p && out, "NULL argument");
@@ -475,7 +477,8 @@ int visfd_cuda_vote_slab_host(visfd_ctx *ctx, int64_t nx, int64_t ny, int64_t nz
     const size_t o = plane * (size_t)v0;
     if (tv_device(ctx, nx, ny, vote_z1 - v0, z_offset + v0, nz_global, own_z0 - v0,
               own_z1 - v0, saliency + o, threshold, nullptr, smoothed + o, p->sigma, p->eival_order,
-              VISFD_SCORE_PLANAR, mask ? mask + o : nullptr, mask ? mask + o : nullptr, tp, tensor, out, out_host))
+              VISFD_SCORE_PLANAR, mask ? mask + o : nullptr, mask ? mask + o : nullptr, tp, tensor, out, out_host,
+              peak ? peak + o : nullptr))
       delivered = true;
   } else {
     VCK(cudaMemcpyAsync(out, saliency + plane * (size_t)own_z0, n_own * sizeof(float), cudaMemcpyDeviceToDevice,
@@ -486,6 +489,18 @@ int visfd_cuda_vote_slab_host(visfd_ctx *ctx, int64_t nx, int64_t ny, int64_t nz
     VCK(cudaMemcpyAsync(out_host, out, n_own * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
     VCK(cudaStreamSynchronize(ctx->stream));
   }
+}
+}  // namespace visfd_cuda
+
+extern "C" {
+
+int visfd_cuda_vote_slab_host(visfd_ctx *ctx, int64_t nx, int64_t ny, int64_t nz_local, int64_t z_offset,
+                              int64_t nz_global, int64_t own_z0, int64_t own_z1, int64_t vote_z0, int64_t vote_z1,
+                              const float *saliency, const float *smoothed, const float *mask, float threshold,
+                              const visfd_membrane_params *p, float *out, float *tensor, float *out_host) {
+  API_BEGIN(ctx)
+  vote_slab_device(ctx, nx, ny, nz_local, z_offset, nz_global, own_z0, own_z1, vote_z0, vote_z1, saliency, smoothed,
+                   mask, threshold, p, out, tensor, out_host, nullptr);
   API_END(ctx)
 }
 

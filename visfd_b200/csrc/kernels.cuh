@@ -63,6 +63,7 @@ float select_threshold(float fraction,
 float select_threshold_device(visfd_ctx *ctx, i64 n, const float *sal, const float *mask,
                               float fraction);
 void apply_cut_device(visfd_ctx *ctx, i64 n, float *sal, float thr);
+// score *= src - background where mask != 0 (mask may be NULL); background == NULL: src is the peak height itself
 void scale_by_peak_device(visfd_ctx *ctx, i64 n, float *score, const float *src, const float *background, const float *mask);
 
 // ---- tv.cu ------------------------------------------------------------------------
@@ -81,16 +82,27 @@ struct TVParams {
 // tensor diagonalised with eival_order.  score_host (optional, HOST pointer of the same
 // size): the receiver planes are voted in up to 8 chunks and every finished chunk of
 // `score` is copied to score_host on a second stream while the next chunk is computed;
-// returns true if score_host has been filled that way.
+// returns true if score_host has been filled that way.  peak (optional, N floats indexed like the slab): the score
+// of every receiver with mask_dst != 0 is multiplied by its peak height (`-membrane-background`), chunk by chunk
+// before the chunk's copy to score_host.
 bool tv_device(visfd_ctx *ctx, i64 nx, i64 ny, i64 nz_local, i64 z_offset, i64 nz_global,
                i64 own_z0, i64 own_z1, const float *saliency, float thr, const float *direction,
                const float *smoothed, float ridge_sigma, int eival_order, int score_kind,
                const float *mask_src, const float *mask_dst, const TVParams &p, float *tensor,
-               float *score, float *score_host = nullptr);
+               float *score, float *score_host = nullptr, const float *peak = nullptr);
 // Upper bound of the device bytes tv_device takes from the pool for a slab of nz_local voter planes, own_planes
 // receiver planes and at most n_voters voters: the voter list (48 B per voter), its brick offsets and the rest.
 size_t tv_workspace_bytes(i64 nx, i64 ny, i64 nz_local, i64 own_planes, uint64_t n_voters);
 int tv_halfwidth(float sigma, float cutoff_ratio);
+
+// ---- api.cu -----------------------------------------------------------------------
+// visfd_cuda_vote_slab_host without its API frame (the slab drivers of multi.cu).  peak (optional, nz_local*ny*nx
+// floats like saliency): the voted score is multiplied by the peak height (tv_device); without voting the saliency
+// is expected to carry it already.
+void vote_slab_device(visfd_ctx *ctx, int64_t nx, int64_t ny, int64_t nz_local, int64_t z_offset, int64_t nz_global,
+                      int64_t own_z0, int64_t own_z1, int64_t vote_z0, int64_t vote_z1, const float *saliency,
+                      const float *smoothed, const float *mask, float threshold, const visfd_membrane_params *p,
+                      float *out, float *tensor, float *out_host, const float *peak);
 
 // ---- threshold.cu -----------------------------------------------------------------
 void threshold_device(visfd_ctx *ctx, i64 n, const float *in, float *out, int kind,

@@ -5,11 +5,14 @@
 //     one slab per device, all slabs at once: every GPU of the node on one volume;
 //   visfd_cuda_membrane_stream(ctx, nx, ny, nz, src_host, mask_host, params, device_bytes, out_host, &threshold)
 //     one device, the slabs one after another within a device-memory budget: volumes whose working set does not fit.
+// Their _background forms add `-membrane-background`: both scores multiplied by the peak height
+// source - Gauss(source, background_sigma), as visfd_cuda_membrane_background does on one GPU.
 //
 // The volume is cut into Z-slabs exactly as visfd_b200/slab.py does for the process-per-GPU driver (rank boundaries
 // on multiples of 8 planes, slabs widened by a halo of RAW SOURCE planes, halo = tv_halfwidth + 1 + gauss_halfwidth,
 // slab start rounded down to a multiple of 8), so every stage is slab-local and the result is bit-identical to the
-// one-GPU result for any number of slabs.  Because the source lives in host memory, each slab uploads its planes --
+// one-GPU result for any number of slabs.  With the background the raw-source part of the halo is
+// max(1 + gauss_halfwidth, background_halfwidth): the peak height must be exact on every voter plane.  Because the source lives in host memory, each slab uploads its planes --
 // halo included -- straight from the caller's array: there is no device-to-device halo traffic at all.
 //
 // A slab always runs the same steps: (1) upload + ridge saliency; (2) for the `-tv-best` cut, per round of the radix
@@ -42,11 +45,13 @@ struct SlabPlan {
   int64_t vote0, vote1;   // global voter planes
 };
 
-// visfd_b200/slab.py: partition() + make_plan()
-std::vector<SlabPlan> make_plans(int64_t nz, int world, int gauss_hw, int tv_hw) {
+// visfd_b200/slab.py: partition() + make_plan().  bg_hw: the half-width of the background Gaussian, 0 without one.
+std::vector<SlabPlan> make_plans(int64_t nz, int world, int gauss_hw, int tv_hw, int bg_hw) {
   const int64_t unit = (nz / 8 >= world) ? 8 : 1;
   const int64_t base = (nz / unit) / world, rem = (nz / unit) % world;
-  const int64_t halo = tv_hw > 0 ? tv_hw + 1 + gauss_hw : 1 + gauss_hw;
+  // the smoothed volume is exact 1 + gauss_hw planes inside the slab, the peak height bg_hw planes inside
+  const int64_t raw = std::max(1 + gauss_hw, bg_hw);
+  const int64_t halo = tv_hw > 0 ? tv_hw + raw : raw;
   std::vector<SlabPlan> plans((size_t)world);
   int64_t z = 0;
   for (int r = 0; r < world; r++) {
@@ -64,6 +69,14 @@ std::vector<SlabPlan> make_plans(int64_t nz, int world, int gauss_hw, int tv_hw)
 }
 
 int max_slabs(int64_t nz) { return (int)std::max<int64_t>(1, nz / 8); }   // at least 8 planes per slab
+
+// `-membrane-background`: sigma > 0 multiplies both scores by the peak height source - Gauss(source, sigma)
+struct Background {
+  float sigma = 0.0f;
+  int hw = 0;               // floor(sigma * truncate_ratio), handlers.cpp:1582-1583
+  bool normalize = true;
+  bool on() const { return sigma > 0.0f; }
+};
 
 // One call at a time: the contexts are kept between calls, one per (slot, device), and a call uses them throughout.
 std::mutex g_call_mutex;
@@ -89,6 +102,7 @@ struct Slab {
   visfd_ctx *ctx = nullptr;
   SlabPlan plan;
   Scratch<float> mask, smoothed, saliency;
+  Scratch<float> peak;   // with the background: the peak height of every plane of the slab, until the vote ends
   cudaEvent_t start = nullptr, stop = nullptr;   // device time: first upload to last download
   double ms = 0.0;
   uint64_t hist[HIST_BINS];
@@ -105,9 +119,10 @@ void make_slabs(std::vector<Slab> &slabs, const std::vector<SlabPlan> &plans, vi
   }
 }
 
-// Step (1): upload the slab, halo included, and compute its ridge saliency.
+// Step (1): upload the slab, halo included, and compute its ridge saliency (times the peak height with the
+// background).
 void upload_and_ridge(Slab &s, int64_t nx, int64_t ny, int64_t nz, const float *src_host, const float *mask_host,
-                      const visfd_membrane_params *p) {
+                      const visfd_membrane_params *p, const Background &bg) {
   const SlabPlan &pl = s.plan;
   const size_t plane = (size_t)nx * (size_t)ny;
   const size_t n = (size_t)(pl.slab1 - pl.slab0) * plane;
@@ -121,10 +136,23 @@ void upload_and_ridge(Slab &s, int64_t nx, int64_t ny, int64_t nz, const float *
     VCK(cudaMemcpyAsync(s.mask.get(), mask_host + (size_t)pl.slab0 * plane, n * sizeof(float), cudaMemcpyHostToDevice,
                         s.ctx->stream));
   }
+  if (bg.on()) {
+    // source - Gauss(source) in one volume, through the filter's minuend epilogue: (src - G(src)) * 1 has the bits
+    // of the one-GPU path's __fsub_rn(src, bg)
+    s.peak.reset(s.ctx, n);
+    const float sg[3] = {bg.sigma, bg.sigma, bg.sigma};
+    const int hw[3] = {bg.hw, bg.hw, bg.hw};
+    gauss_device(s.ctx, nx, ny, pl.slab1 - pl.slab0, pl.slab0, nz, src.get(), s.peak.get(), s.mask.get(), sg, hw,
+                 bg.normalize, src.get(), 1.0f);
+    VCK(cudaStreamSynchronize(s.ctx->stream));
+    resolve_stage_times(s.ctx);   // (the entry point below drops the stage events it finds pending)
+  }
   if (visfd_cuda_ridge_saliency_slab(s.ctx, nx, ny, pl.slab1 - pl.slab0, pl.slab0, nz, src.get(), s.mask.get(),
                                      p->sigma, p->truncate_ratio, p->eival_order, VISFD_SCORE_PLANAR, s.smoothed.get(),
                                      s.saliency.get()) != 0)
     throw Error(visfd_cuda_last_error());
+  // before any histogram: the cut ranks the scaled score (handlers.cpp:1698-1702)
+  if (bg.on()) scale_by_peak_device(s.ctx, (i64)n, s.saliency.get(), s.peak.get(), nullptr, s.mask.get());
 }
 
 // Step (2): the histogram of the slabs' own planes, summed into hist.  run(step) runs step(slab) on every slab.
@@ -142,24 +170,25 @@ void summed_own_hist(std::vector<Slab> &slabs, const Run &run, size_t plane, boo
     for (int b = 0; b < HIST_BINS; b++) hist[b] += s.hist[b];
 }
 
-// Step (3): voting on the own planes, delivered into the caller's array.
+// Step (3): voting on the own planes, delivered into the caller's array (each chunk times its peak height with the
+// background).
 void vote_to_host(Slab &s, int64_t nx, int64_t ny, int64_t nz, float threshold, const visfd_membrane_params *p,
                   float *out_host) {
   const SlabPlan &pl = s.plan;
   const size_t plane = (size_t)nx * (size_t)ny;
   Scratch<float> out(s.ctx, (size_t)(pl.own1 - pl.own0) * plane);
-  if (visfd_cuda_vote_slab_host(s.ctx, nx, ny, pl.slab1 - pl.slab0, pl.slab0, nz, pl.own0 - pl.slab0,
-                                pl.own1 - pl.slab0, pl.vote0 - pl.slab0, pl.vote1 - pl.slab0, s.saliency.get(),
-                                s.smoothed.get(), s.mask.get(), threshold, p, out.get(), nullptr,
-                                out_host + (size_t)pl.own0 * plane) != 0)
-    throw Error(visfd_cuda_last_error());
+  vote_slab_device(s.ctx, nx, ny, pl.slab1 - pl.slab0, pl.slab0, nz, pl.own0 - pl.slab0, pl.own1 - pl.slab0,
+                   pl.vote0 - pl.slab0, pl.vote1 - pl.slab0, s.saliency.get(), s.smoothed.get(), s.mask.get(),
+                   threshold, p, out.get(), nullptr, out_host + (size_t)pl.own0 * plane, s.peak.get());
+  VCK(cudaStreamSynchronize(s.ctx->stream));
+  resolve_stage_times(s.ctx);
 }
 
 // Runs fn(slab) for every slab at once, slab 0 on the calling thread and the others on threads of their own, each
 // on its slab's device.  Returns when all of them have finished, and then throws the error of the first slab that
 // failed.
 template <typename Fn>
-void for_each_slab(std::vector<Slab> &slabs, const Fn &fn) {
+void for_each_slab(const char *name, std::vector<Slab> &slabs, const Fn &fn) {
   std::vector<std::string> errors(slabs.size());
   auto run = [&](size_t r) {
     try {
@@ -181,7 +210,7 @@ void for_each_slab(std::vector<Slab> &slabs, const Fn &fn) {
   for (std::thread &t : threads) t.join();
   for (size_t r = 0; r < slabs.size(); r++)
     if (!errors[r].empty())
-      throw Error("visfd_cuda_membrane_multi, slab " + std::to_string(r) + " on device " +
+      throw Error(std::string(name) + ", slab " + std::to_string(r) + " on device " +
                   std::to_string(slabs[r].ctx->device) + ": " + errors[r]);
 }
 
@@ -190,15 +219,21 @@ void for_each_slab(std::vector<Slab> &slabs, const Fn &fn) {
 // Gaussian's scratch; a cut or count pass (vote == false) adds the select's histogram.  The vote pass releases the
 // step's scratch before step (3), which holds the mask, the smoothed volume and the saliency, the own-plane output
 // and the voting workspace for at most `voters` voters in the whole volume.
+// With the background both steps also hold the slab's whole peak height.  In step (1) the background Gaussian runs
+// first, beside the same volumes; its scratch goes back to the pool, where the smoothing's scratch, which has at least
+// as many volumes, takes them again, so only its block of taps may stay cached next to the smoothing's.
 size_t slab_bytes(const SlabPlan &pl, int64_t nx, int64_t ny, bool masked, const visfd_membrane_params *p,
-                  int gauss_hw, bool vote, uint64_t voters) {
+                  int gauss_hw, const Background &bg, bool vote, uint64_t voters) {
   const size_t plane = (size_t)nx * (size_t)ny;
   const int64_t slab = pl.slab1 - pl.slab0;
   const size_t vol = visfd_ctx::block_bytes((size_t)slab * plane * sizeof(float));
-  const int hw[3] = {gauss_hw, gauss_hw, gauss_hw};
-  const size_t ridge = (masked ? 4 : 3) * vol + separable_workspace_bytes(nx, ny, slab, hw, masked, true);
+  const int hw[3] = {gauss_hw, gauss_hw, gauss_hw}, hw_bg[3] = {bg.hw, bg.hw, bg.hw};
+  const size_t peak = bg.on() ? vol : 0;
+  const size_t bg_taps = bg.on() ? separable_workspace_bytes(nx, ny, slab, hw_bg, false, false) - vol : 0;
+  const size_t ridge = (masked ? 4 : 3) * vol + peak + separable_workspace_bytes(nx, ny, slab, hw, masked, true) + bg_taps;
   if (!vote) return ridge + visfd_ctx::block_bytes(HIST_BINS * sizeof(uint64_t));
-  size_t voting = (masked ? 3 : 2) * vol + visfd_ctx::block_bytes((size_t)(pl.own1 - pl.own0) * plane * sizeof(float));
+  size_t voting = (masked ? 3 : 2) * vol + peak +
+                  visfd_ctx::block_bytes((size_t)(pl.own1 - pl.own0) * plane * sizeof(float));
   if (p->tv_sigma > 0.0f) {
     // visfd_cuda_vote_slab_host widens the voter planes down to a global multiple of 8: up to 7 more planes, whose
     // saliency may be incomplete, so they may add up to 7 planes of voters to the count of the whole volume
@@ -217,34 +252,44 @@ void release_cache(visfd_ctx *ctx) {
   ctx->trim();
 }
 
-}  // namespace
+// The background of a _background entry point, checked; sigma 0: none (the plain entry points).
+Background background(const std::string &who, const visfd_membrane_params *p, float sigma, int normalize) {
+  VREQUIRE(sigma >= 0.0f, who + ": negative background width");   // (NaN fails too)
+  Background bg;
+  bg.sigma = sigma;
+  bg.hw = sigma > 0.0f ? (int)floorf(sigma * p->truncate_ratio) : 0;   // as visfd_cuda_membrane_background
+  bg.normalize = normalize != 0;
+  return bg;
+}
 
-extern "C" int visfd_cuda_membrane_multi(int ndev, const int *devices, int64_t nx, int64_t ny, int64_t nz,
-                                         const float *src_host, const float *mask_host,
-                                         const visfd_membrane_params *p, float *out_host, float *threshold_out,
-                                         double *device_ms /* ndev values or NULL */) {
+int membrane_multi(const char *name, int ndev, const int *devices, int64_t nx, int64_t ny, int64_t nz,
+                   const float *src_host, const float *mask_host, const visfd_membrane_params *p,
+                   float background_sigma, int normalize, float *out_host, float *threshold_out,
+                   double *device_ms) {
   try {
-    VREQUIRE(ndev >= 1 && devices, "visfd_cuda_membrane_multi: need at least one device");
-    VREQUIRE(nx > 0 && ny > 0 && nz > 0 && src_host && p && out_host, "visfd_cuda_membrane_multi: bad arguments");
+    const std::string who(name);
+    VREQUIRE(ndev >= 1 && devices, who + ": need at least one device");
+    VREQUIRE(nx > 0 && ny > 0 && nz > 0 && src_host && p && out_host, who + ": bad arguments");
     VREQUIRE(!is_device_pointer(src_host) && !is_device_pointer(out_host) && !is_device_pointer(mask_host),
-             "visfd_cuda_membrane_multi takes HOST arrays (use the slab entry points for device-resident data)");
+             who + " takes HOST arrays (use the slab entry points for device-resident data)");
+    const Background bg = background(who, p, background_sigma, normalize);
     const int gauss_hw = (int)floor(p->sigma * p->truncate_ratio);
     const int tv_hw = p->tv_sigma > 0.0f ? tv_halfwidth(p->tv_sigma, p->tv_cutoff_ratio) : 0;
     const int world = std::min(ndev, max_slabs(nz));
-    const std::vector<SlabPlan> plans = make_plans(nz, world, gauss_hw, tv_hw);
+    const std::vector<SlabPlan> plans = make_plans(nz, world, gauss_hw, tv_hw, bg.hw);
     const size_t plane = (size_t)nx * (size_t)ny;
 
     std::lock_guard<std::mutex> lock(g_call_mutex);
     std::vector<Slab> slabs((size_t)world);
     make_slabs(slabs, plans, nullptr);
     for (int r = 0; r < world; r++) slabs[(size_t)r].ctx = context_for(r, devices[r]);
-    auto concurrently = [&](const auto &step) { for_each_slab(slabs, step); };
+    auto concurrently = [&](const auto &step) { for_each_slab(name, slabs, step); };
 
-    for_each_slab(slabs, [&](Slab &s) {
+    for_each_slab(name, slabs, [&](Slab &s) {
       VCK(cudaEventCreate(&s.start));
       VCK(cudaEventCreate(&s.stop));
       VCK(cudaEventRecord(s.start, s.ctx->stream));
-      upload_and_ridge(s, nx, ny, nz, src_host, mask_host, p);
+      upload_and_ridge(s, nx, ny, nz, src_host, mask_host, p, bg);
     });
 
     float threshold = p->cut;
@@ -253,7 +298,7 @@ extern "C" int visfd_cuda_membrane_multi(int ndev, const int *devices, int64_t n
         summed_own_hist(slabs, concurrently, plane, mask_host != nullptr, prefix, prefix_bits, hist);
       });
 
-    for_each_slab(slabs, [&](Slab &s) {
+    for_each_slab(name, slabs, [&](Slab &s) {
       vote_to_host(s, nx, ny, nz, threshold, p, out_host);
       VCK(cudaEventRecord(s.stop, s.ctx->stream));
       VCK(cudaEventSynchronize(s.stop));
@@ -272,16 +317,16 @@ extern "C" int visfd_cuda_membrane_multi(int ndev, const int *devices, int64_t n
   }
 }
 
-extern "C" int visfd_cuda_membrane_stream(visfd_ctx *ctx, int64_t nx, int64_t ny, int64_t nz, const float *src_host,
-                                          const float *mask_host, const visfd_membrane_params *p,
-                                          int64_t device_bytes, float *out_host, float *threshold_out,
-                                          int64_t *n_slabs_out) {
+int membrane_stream(const char *name, visfd_ctx *ctx, int64_t nx, int64_t ny, int64_t nz, const float *src_host,
+                    const float *mask_host, const visfd_membrane_params *p, float background_sigma, int normalize,
+                    int64_t device_bytes, float *out_host, float *threshold_out, int64_t *n_slabs_out) {
   try {
-    VREQUIRE(ctx != nullptr, "visfd_cuda_membrane_stream: context is NULL");
-    VREQUIRE(nx > 0 && ny > 0 && nz > 0 && src_host && p && out_host && device_bytes >= 0,
-             "visfd_cuda_membrane_stream: bad arguments");
+    const std::string who(name);
+    VREQUIRE(ctx != nullptr, who + ": context is NULL");
+    VREQUIRE(nx > 0 && ny > 0 && nz > 0 && src_host && p && out_host && device_bytes >= 0, who + ": bad arguments");
     VREQUIRE(!is_device_pointer(src_host) && !is_device_pointer(out_host) && !is_device_pointer(mask_host),
-             "visfd_cuda_membrane_stream takes HOST arrays (use visfd_cuda_membrane for device-resident data)");
+             who + " takes HOST arrays (use visfd_cuda_membrane for device-resident data)");
+    const Background bg = background(who, p, background_sigma, normalize);
     VCK(cudaSetDevice(ctx->device));
     drop_pending_stage_events(ctx);
     release_cache(ctx);   // blocks cached by earlier calls count against the budget
@@ -303,14 +348,14 @@ extern "C" int visfd_cuda_membrane_stream(visfd_ctx *ctx, int64_t nx, int64_t ny
     auto fewest_slabs = [&](bool vote_pass, uint64_t voters, size_t *need) {
       for (int world = 1; world <= max_slabs(nz); world++) {
         *need = 0;
-        for (const SlabPlan &pl : make_plans(nz, world, gauss_hw, tv_hw))
-          *need = std::max(*need, slab_bytes(pl, nx, ny, masked, p, gauss_hw, vote_pass, voters));
+        for (const SlabPlan &pl : make_plans(nz, world, gauss_hw, tv_hw, bg.hw))
+          *need = std::max(*need, slab_bytes(pl, nx, ny, masked, p, gauss_hw, bg, vote_pass, voters));
         if (*need <= (size_t)std::max<int64_t>(budget, 0)) return world;
       }
       return 0;
     };
     auto too_small = [&](const char *pass, size_t need) {
-      return Error("visfd_cuda_membrane_stream: " + std::string(pass) + " needs " + std::to_string(need) +
+      return Error(who + ": " + std::string(pass) + " needs " + std::to_string(need) +
                    " bytes of device memory in slabs of 8 planes; the budget is " + std::to_string(budget) +
                    " bytes");
     };
@@ -319,15 +364,15 @@ extern "C" int visfd_cuda_membrane_stream(visfd_ctx *ctx, int64_t nx, int64_t ny
       for (size_t r = 0; r < slabs.size(); r++) {
         Slab &s = slabs[r];
         try {
-          upload_and_ridge(s, nx, ny, nz, src_host, mask_host, p);
+          upload_and_ridge(s, nx, ny, nz, src_host, mask_host, p, bg);
           step(s);
         } catch (const std::exception &ex) {
-          throw Error("visfd_cuda_membrane_stream, slab " + std::to_string(r) + " of " + std::to_string(slabs.size()) +
-                      ": " + ex.what());
+          throw Error(who + ", slab " + std::to_string(r) + " of " + std::to_string(slabs.size()) + ": " + ex.what());
         }
         s.mask.free();
         s.smoothed.free();
         s.saliency.free();
+        s.peak.free();
         release_cache(ctx);
       }
     };
@@ -341,7 +386,7 @@ extern "C" int visfd_cuda_membrane_stream(visfd_ctx *ctx, int64_t nx, int64_t ny
     uint64_t voters = UINT64_MAX;   // unknown: every voxel of a slab's voter planes may vote
     if (p->cut_is_fraction || (vote && fewest_slabs(true, voters, &need) != n_cut)) {
       std::vector<Slab> slabs((size_t)n_cut);
-      make_slabs(slabs, make_plans(nz, n_cut, gauss_hw, tv_hw), ctx);
+      make_slabs(slabs, make_plans(nz, n_cut, gauss_hw, tv_hw, bg.hw), ctx);
       auto in_turn = [&](const auto &step) { one_by_one(slabs, step); };
       if (p->cut_is_fraction) {
         threshold = select_threshold(p->cut, [&](uint32_t prefix, int prefix_bits, uint64_t *hist) {
@@ -359,7 +404,7 @@ extern "C" int visfd_cuda_membrane_stream(visfd_ctx *ctx, int64_t nx, int64_t ny
     const int n_vote = fewest_slabs(true, voters, &need);
     if (n_vote == 0) throw too_small("the vote pass", need);
     std::vector<Slab> slabs((size_t)n_vote);
-    make_slabs(slabs, make_plans(nz, n_vote, gauss_hw, tv_hw), ctx);
+    make_slabs(slabs, make_plans(nz, n_vote, gauss_hw, tv_hw, bg.hw), ctx);
     one_by_one(slabs, [&](Slab &s) {
       release_cache(ctx);   // the ridge step's scratch
       vote_to_host(s, nx, ny, nz, threshold, p, out_host);
@@ -377,4 +422,41 @@ extern "C" int visfd_cuda_membrane_stream(visfd_ctx *ctx, int64_t nx, int64_t ny
     }
     return 1;
   }
+}
+
+}  // namespace
+
+extern "C" int visfd_cuda_membrane_multi(int ndev, const int *devices, int64_t nx, int64_t ny, int64_t nz,
+                                         const float *src_host, const float *mask_host,
+                                         const visfd_membrane_params *p, float *out_host, float *threshold_out,
+                                         double *device_ms /* ndev values or NULL */) {
+  return membrane_multi("visfd_cuda_membrane_multi", ndev, devices, nx, ny, nz, src_host, mask_host, p, 0.0f, 1,
+                        out_host, threshold_out, device_ms);
+}
+
+extern "C" int visfd_cuda_membrane_multi_background(int ndev, const int *devices, int64_t nx, int64_t ny, int64_t nz,
+                                                    const float *src_host, const float *mask_host,
+                                                    const visfd_membrane_params *p, float background_sigma,
+                                                    int normalize_near_boundaries, float *out_host,
+                                                    float *threshold_out, double *device_ms) {
+  return membrane_multi("visfd_cuda_membrane_multi_background", ndev, devices, nx, ny, nz, src_host, mask_host, p,
+                        background_sigma, normalize_near_boundaries, out_host, threshold_out, device_ms);
+}
+
+extern "C" int visfd_cuda_membrane_stream(visfd_ctx *ctx, int64_t nx, int64_t ny, int64_t nz, const float *src_host,
+                                          const float *mask_host, const visfd_membrane_params *p,
+                                          int64_t device_bytes, float *out_host, float *threshold_out,
+                                          int64_t *n_slabs_out) {
+  return membrane_stream("visfd_cuda_membrane_stream", ctx, nx, ny, nz, src_host, mask_host, p, 0.0f, 1,
+                         device_bytes, out_host, threshold_out, n_slabs_out);
+}
+
+extern "C" int visfd_cuda_membrane_stream_background(visfd_ctx *ctx, int64_t nx, int64_t ny, int64_t nz,
+                                                     const float *src_host, const float *mask_host,
+                                                     const visfd_membrane_params *p, float background_sigma,
+                                                     int normalize_near_boundaries, int64_t device_bytes,
+                                                     float *out_host, float *threshold_out, int64_t *n_slabs_out) {
+  return membrane_stream("visfd_cuda_membrane_stream_background", ctx, nx, ny, nz, src_host, mask_host, p,
+                         background_sigma, normalize_near_boundaries, device_bytes, out_host, threshold_out,
+                         n_slabs_out);
 }

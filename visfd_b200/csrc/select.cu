@@ -205,14 +205,15 @@ void apply_cut_device(visfd_ctx *ctx, i64 n, float *sal, float thr) {
 }
 
 // peak_height of `-membrane-background` (handlers.cpp:1698-1702, :1883-1887): score *= source - background, for the
-// voxels the reference visits (mask != 0)
+// voxels the reference visits (mask != 0).  bg == NULL: src already holds the peak height.
 __global__ void scale_by_peak_kernel(float *__restrict__ score, const float *__restrict__ src, const float *__restrict__ bg,
                                      const float *__restrict__ mask, i64 n) {
   i64 i = (i64)blockIdx.x * blockDim.x + threadIdx.x;
   i64 stride = (i64)gridDim.x * blockDim.x;
   for (; i < n; i += stride) {
     if (mask && __ldg(mask + i) == 0.0f) continue;
-    score[i] = __fmul_rn(score[i], __fsub_rn(__ldg(src + i), __ldg(bg + i)));
+    const float peak = bg ? __fsub_rn(__ldg(src + i), __ldg(bg + i)) : __ldg(src + i);
+    score[i] = __fmul_rn(score[i], peak);
   }
 }
 

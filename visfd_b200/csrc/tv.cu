@@ -1058,8 +1058,9 @@ bool tv_device(visfd_ctx *ctx, i64 nx, i64 ny, i64 nz_local, i64 z_offset, i64 n
                i64 own_z0, i64 own_z1, const float *saliency, float thr, const float *direction,
                const float *smoothed, float ridge_sigma, int eival_order, int score_kind,
                const float *mask_src, const float *mask_dst, const TVParams &p, float *tensor,
-               float *score, float *score_host) {
+               float *score, float *score_host, const float *peak) {
   VREQUIRE(nx > 0 && ny > 0 && nz_local > 0, "empty volume");
+  VREQUIRE(!peak || score, "the peak height scales the score: score must be given");
   VREQUIRE(own_z0 >= 0 && own_z1 <= nz_local && own_z0 <= own_z1, "receiver planes outside the slab");
   VREQUIRE(p.sigma > 0.0f, "tensor-voting sigma must be positive");
   VREQUIRE(p.exponent >= 1, "tensor-voting angle exponent must be >= 1");
@@ -1133,6 +1134,12 @@ bool tv_device(visfd_ctx *ctx, i64 nx, i64 ny, i64 nz_local, i64 z_offset, i64 n
   const int n_chunks = (int)((planes + chunk_planes - 1) / chunk_planes);
   VREQUIRE((i64)g.ntx * g.nty * div_up(chunk_planes, TV_TILE_Z) * 4 / TV_WARPS < 2147483647LL,
            "too many receiver tiles for one launch");
+  // score planes [z0, z1) of the slab *= their peak height, where mask_dst != 0
+  auto scale_own_planes = [&](i64 z0, i64 z1, float *s) {
+    const size_t o = (size_t)z0 * (size_t)nx * (size_t)ny;
+    scale_by_peak_device(ctx, (i64)((size_t)(z1 - z0) * (size_t)nx * (size_t)ny), s, peak + o, nullptr,
+                         mask_dst ? mask_dst + o : nullptr);
+  };
   EventList chunk_events(ctx);
   std::vector<cudaEvent_t> &chunk_done = chunk_events.ev;
   Scratch<float2> lut;
@@ -1158,9 +1165,13 @@ bool tv_device(visfd_ctx *ctx, i64 nx, i64 ny, i64 nz_local, i64 z_offset, i64 n
         gc.ticket = tickets.get() + c;
       }
       launch_gather(ctx, pl, gc, grid);
-      if (overlap_d2h) VCK(cudaEventRecord(chunk_events.add(), ctx->stream));
+      if (overlap_d2h) {
+        if (peak) scale_own_planes(gc.own_z0, gc.own_z1, gc.score);   // before the chunk's copy is queued
+        VCK(cudaEventRecord(chunk_events.add(), ctx->stream));
+      }
     }
   }
+  if (peak && !overlap_d2h) scale_own_planes(own_z0, own_z1, score);
   if (overlap_d2h) {
     // all launches are queued; now the copies, each behind its chunk (with pageable host memory
     // cudaMemcpyAsync blocks the host, which no longer delays any launch)
