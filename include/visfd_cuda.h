@@ -492,6 +492,41 @@ int visfd_cuda_blob_finalize(float minima_threshold, float maxima_threshold, int
                              float *min_sigma, float *min_score, int64_t *n_minima, float *max_crds,
                              float *max_sigma, float *max_score, int64_t *n_maxima);
 
+/* visfd_cuda_blob_dog with HOST arrays, in Z-slabs: on several GPUs of one node (multi) or on one GPU slab after slab
+ * within a device-memory budget (stream).  The lists -- rows, their order (scale, z, y, x) and the counts -- are
+ * bit-identical to what visfd_cuda_blob_dog returns for the same arguments, for any number of slabs, with or without
+ * a mask and in both threshold modes; rows beyond `capacity` are not stored and the counts are still the full counts.
+ * src_host, mask_host (may be NULL) and the six list buffers must be HOST arrays: a device pointer fails (use
+ * visfd_cuda_blob_dog_slab for device-resident data).
+ * The volume is cut as visfd_cuda_membrane_multi cuts it, with a halo of (largest LoG half-width + 1) planes of raw
+ * source, which each slab uploads straight from src_host.  A slab scans its own planes at every scale; no slab waits
+ * for another until the end, where the lists are concatenated per scale in slab order, the best scores of the whole
+ * image are taken (min / max over the slabs) and the final score filter runs once.  One pass, unlike the membrane
+ * stream.
+ * multi: one slab per entry of devices[] (a device may be listed more than once).  It shares its per-entry contexts
+ * with visfd_cuda_membrane_multi, and one multi call of either kind runs at a time.  device_ms (ndev doubles or
+ * NULL): device time of each slab, first upload to last scan.  An error names the slab and its device.
+ * stream: the fewest slabs whose every slab fits device_bytes (0 = the free memory at entry, less a margin); the
+ * context's pool never holds more, and every slab is released before the next.  A slab holds its source and mask,
+ * the three LoG volumes of the scan, the Gaussians' scratch (two volumes, four with a mask) and two candidate lists
+ * sized so that they cannot overflow (one row per 2x2x2 voxels of its own planes): about one volume more than
+ * visfd_cuda_blob_dog.  The call fails, naming the bytes it needs, when slabs of 8 planes do not fit; the context
+ * stays usable after any failure.  *n_slabs_out (may be NULL): slabs used. */
+int visfd_cuda_blob_dog_multi(int ndev, const int *devices, int64_t nx, int64_t ny, int64_t nz,
+                              const float *src_host, const float *mask_host, const float *sigmas, int n_sigmas,
+                              float delta, float truncate_ratio, float minima_threshold, float maxima_threshold,
+                              int use_threshold_ratios, int64_t capacity,
+                              float *min_crds, float *min_sigma, float *min_score, int64_t *n_minima,
+                              float *max_crds, float *max_sigma, float *max_score, int64_t *n_maxima,
+                              double *device_ms);
+int visfd_cuda_blob_dog_stream(visfd_ctx *ctx, int64_t nx, int64_t ny, int64_t nz,
+                               const float *src_host, const float *mask_host, const float *sigmas, int n_sigmas,
+                               float delta, float truncate_ratio, float minima_threshold, float maxima_threshold,
+                               int use_threshold_ratios, int64_t device_bytes, int64_t capacity,
+                               float *min_crds, float *min_sigma, float *min_score, int64_t *n_minima,
+                               float *max_crds, float *max_sigma, float *max_score, int64_t *n_maxima,
+                               int64_t *n_slabs_out);
+
 #ifdef __cplusplus
 }
 #endif

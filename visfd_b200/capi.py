@@ -207,6 +207,51 @@ def membrane_multi(devices, src, sigma, truncate_ratio, order, cut, cut_is_fract
     return dict(out=res, threshold=thr.value, device_ms=list(ms))
 
 
+def _blob_buffers(capacity):
+    return [np.zeros((capacity, 3), np.float32), np.zeros(capacity, np.float32), np.zeros(capacity, np.float32),
+            np.zeros((capacity, 3), np.float32), np.zeros(capacity, np.float32), np.zeros(capacity, np.float32)]
+
+
+def _host_blob_args(who, src, mask, sigmas):
+    """numpy host arrays for the blob slab drivers (which refuse device memory)."""
+    if _is_torch(src) or _is_torch(mask):
+        raise VisfdCudaError(f"{who} takes numpy (host) arrays")
+    src = np.ascontiguousarray(src, np.float32)
+    mask = None if mask is None else np.ascontiguousarray(mask, np.float32)
+    return src, mask, np.ascontiguousarray(np.asarray(sigmas), np.float32)
+
+
+def _blob_lists(who, bufs, nmin, nmax, capacity):
+    if nmin.value > capacity or nmax.value > capacity:
+        raise VisfdCudaError("%s: %d minima / %d maxima exceed the capacity of %d rows; call again with a "
+                             "larger capacity" % (who, nmin.value, nmax.value, capacity))
+    return (_pack_blobs(bufs[0], bufs[1], bufs[2], nmin.value),
+            _pack_blobs(bufs[3], bufs[4], bufs[5], nmax.value))
+
+
+def blob_dog_multi(devices, src, sigmas, delta=0.02, truncate_ratio=2.5, mask=None, minima_threshold=np.inf,
+                   maxima_threshold=-np.inf, use_threshold_ratios=False, capacity=1 << 20, lib=None):
+    """visfd_cuda_blob_dog_multi: BlobDog (lib/visfd/feature.hpp:56-427) on several GPUs of this node behind one C
+    call, one Z-slab per entry of devices (a device may appear more than once).  numpy (host) arrays only.
+    -> dict(minima, maxima, device_ms): rows of x,y,z,sigma,score equal to Context.blob_dog's."""
+    lib = lib or load_library()
+    src, mask, sg = _host_blob_args("blob_dog_multi", src, mask, sigmas)
+    devs = (C.c_int * len(devices))(*[int(d) for d in devices])
+    ms = (C.c_double * len(devices))()
+    bufs = _blob_buffers(capacity)
+    nmin, nmax = _i64(), _i64()
+    nz, ny, nx = src.shape
+    rc = lib.visfd_cuda_blob_dog_multi(_i(len(devices)), devs, _i64(nx), _i64(ny), _i64(nz), _ptr(src), _ptr(mask),
+                                       _ptr(sg), _i(len(sg)), _f(delta), _f(truncate_ratio), _f(minima_threshold),
+                                       _f(maxima_threshold), _i(int(use_threshold_ratios)), _i64(capacity),
+                                       _ptr(bufs[0]), _ptr(bufs[1]), _ptr(bufs[2]), C.byref(nmin),
+                                       _ptr(bufs[3]), _ptr(bufs[4]), _ptr(bufs[5]), C.byref(nmax), ms)
+    if rc != 0:
+        raise VisfdCudaError(lib.visfd_cuda_last_error().decode())
+    minima, maxima = _blob_lists("blob_dog_multi", bufs, nmin, nmax, capacity)
+    return dict(minima=minima, maxima=maxima, device_ms=list(ms))
+
+
 class Context:
     """One context per GPU (visfd_cuda_init)."""
 
@@ -644,6 +689,24 @@ class Context:
                                  "larger capacity" % (nmin.value, nmax.value, capacity))
         return (_pack_blobs(bufs[0], bufs[1], bufs[2], nmin.value),
                 _pack_blobs(bufs[3], bufs[4], bufs[5], nmax.value))
+
+    def blob_dog_stream(self, src, sigmas, delta=0.02, truncate_ratio=2.5, mask=None, minima_threshold=np.inf,
+                        maxima_threshold=-np.inf, use_threshold_ratios=False, capacity=1 << 20, device_bytes=0):
+        """visfd_cuda_blob_dog_stream: BlobDog on this context's GPU in Z-slabs run one after another, for volumes
+        whose working set does not fit on it; the device memory the call reserves stays within device_bytes (0: the
+        free memory at entry, less a margin).  numpy (host) arrays only.
+        -> dict(minima, maxima, n_slabs): rows of x,y,z,sigma,score equal to blob_dog's."""
+        src, mask, sg = _host_blob_args("blob_dog_stream", src, mask, sigmas)
+        bufs = _blob_buffers(capacity)
+        nmin, nmax, n_slabs = _i64(), _i64(), _i64()
+        self._ck(self.lib.visfd_cuda_blob_dog_stream(self.h, *self._dims(src.shape), _ptr(src), _ptr(mask), _ptr(sg),
+                                                     _i(len(sg)), _f(delta), _f(truncate_ratio), _f(minima_threshold),
+                                                     _f(maxima_threshold), _i(int(use_threshold_ratios)),
+                                                     _i64(int(device_bytes)), _i64(capacity), _ptr(bufs[0]),
+                                                     _ptr(bufs[1]), _ptr(bufs[2]), C.byref(nmin), _ptr(bufs[3]),
+                                                     _ptr(bufs[4]), _ptr(bufs[5]), C.byref(nmax), C.byref(n_slabs)))
+        minima, maxima = _blob_lists("blob_dog_stream", bufs, nmin, nmax, capacity)
+        return dict(minima=minima, maxima=maxima, n_slabs=n_slabs.value)
 
     def blob_dog_slab(self, src, z_offset, nz_global, own, sigmas, delta=0.02, truncate_ratio=2.5, mask=None,
                       minima_threshold=np.inf, maxima_threshold=-np.inf, use_threshold_ratios=False,

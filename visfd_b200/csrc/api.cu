@@ -34,7 +34,7 @@ static void check_dims(int64_t nx, int64_t ny, int64_t nz) {
 
 static bool on_host(const void *p) { return p != nullptr && !is_device_pointer(p); }
 
-static void emit_blob_list(const BlobList &l, int64_t capacity, float *crds, float *sg, float *sc, int64_t *cnt) {
+void visfd_cuda::emit_blob_list(const BlobList &l, int64_t capacity, float *crds, float *sg, float *sc, int64_t *cnt) {
   int64_t n = (int64_t)l.score.size();
   if (cnt) *cnt = n;
   int64_t k = std::min(n, capacity);

@@ -267,12 +267,13 @@ void blob_final_filter(BlobList &minima, BlobList &maxima, float minima_threshol
 // Slab form: the slab holds image planes [z_offset, z_offset + nz); candidates are produced for the
 // slab-local planes [own_z0, own_z1) with z reported as the IMAGE plane.  best[0] / best[1] receive the
 // best minimum / maximum score found (1 / -1 if none, feature.hpp:122-123).  finalize = false leaves out
-// the final filter, which needs the best scores of the whole image (blob_final_filter).
+// the final filter, which needs the best scores of the whole image (blob_final_filter).  capacity: rows of each
+// device candidate list (0: N / 32, at least 65536); a scale that overflows them is scanned again into larger lists.
 void blob_dog_device(visfd_ctx *ctx, i64 nx, i64 ny, i64 nz, i64 z_offset, i64 nz_global, i64 own_z0, i64 own_z1,
                      const float *src, const float *mask,
                      const float *sigmas, int n_sigmas, float delta, float truncate_ratio,
                      float minima_threshold, float maxima_threshold, int use_threshold_ratios,
-                     BlobList &minima, BlobList &maxima, bool finalize, float best[2]) {
+                     BlobList &minima, BlobList &maxima, bool finalize, float best[2], i64 capacity_rows) {
   VREQUIRE(nx > 0 && ny > 0 && nz > 0, "empty volume");
   VREQUIRE(z_offset >= 0 && z_offset + nz <= nz_global && 0 <= own_z0 && own_z0 <= own_z1 && own_z1 <= nz,
            "slab / receiver planes outside the image");
@@ -282,12 +283,14 @@ void blob_dog_device(visfd_ctx *ctx, i64 nx, i64 ny, i64 nz, i64 z_offset, i64 n
   const float INF = std::numeric_limits<float>::infinity();
   Scratch<float> ring[3];
   for (int k = 0; k < 3; k++) ring[k].reset(ctx, N);
-  unsigned long long capacity = (unsigned long long)std::max<i64>(1 << 16, N / 32);
+  unsigned long long capacity =
+      (unsigned long long)(capacity_rows > 0 ? capacity_rows : std::max<i64>(1 << 16, N / 32));
   Scratch<BlobCand> dmins(ctx, capacity), dmaxs(ctx, capacity);
   Scratch<unsigned long long> counters(ctx, 2);
 
   std::vector<BlobCand> mins, maxs;
   std::vector<float> min_sig, max_sig;
+  std::vector<i64> min_rows(n_sigmas, 0), max_rows(n_sigmas, 0);
   float gmin = 1.0f, gmax = -1.0f;  // feature.hpp:122-123 ("impossible" initial values)
 
   for (int ir = 0; ir < n_sigmas; ir++) {
@@ -349,6 +352,8 @@ void blob_dog_device(visfd_ctx *ctx, i64 nx, i64 ny, i64 nz, i64 z_offset, i64 n
       sort_raster(lx);
       for (auto &c : lm) { mins.push_back(c); min_sig.push_back(sigmas[ir - 1]); gmin = std::min(gmin, c.score); }
       for (auto &c : lx) { maxs.push_back(c); max_sig.push_back(sigmas[ir - 1]); gmax = std::max(gmax, c.score); }
+      min_rows[ir - 1] = (i64)lm.size();
+      max_rows[ir - 1] = (i64)lx.size();
       break;
     }
   }
@@ -365,6 +370,8 @@ void blob_dog_device(visfd_ctx *ctx, i64 nx, i64 ny, i64 nz, i64 z_offset, i64 n
     maxima.sigma.push_back(max_sig[i]);
     maxima.score.push_back(maxs[i].score);
   }
+  minima.scale_rows = std::move(min_rows);
+  maxima.scale_rows = std::move(max_rows);
   if (best) { best[0] = gmin; best[1] = gmax; }
   if (finalize) blob_final_filter(minima, maxima, minima_threshold, maxima_threshold, use_threshold_ratios, gmin, gmax);
 }

@@ -63,6 +63,8 @@ struct visfd_ctx {
 
   // What alloc(bytes) takes from the device: requests are rounded up to whole 512-byte units.
   static size_t block_bytes(size_t bytes) { return ((bytes ? bytes : 16) + 511) & ~size_t(511); }
+  // Whether alloc serves a request of `bytes` (block_bytes) from a cached block of `cached` bytes.
+  static bool reuses(size_t cached, size_t bytes) { return cached >= bytes && cached <= bytes + bytes / 4 + (1 << 20); }
   void *alloc(size_t bytes);
   void release(void *p);
   void trim();

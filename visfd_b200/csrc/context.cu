@@ -67,7 +67,7 @@ void *visfd_ctx::alloc(size_t bytes) {
   int best = -1;
   for (int i = 0; i < (int)free_blocks.size(); i++) {
     size_t b = free_blocks[i].bytes;
-    if (b >= bytes && b <= bytes + bytes / 4 + (1 << 20)) {
+    if (reuses(b, bytes)) {
       if (best < 0 || b < free_blocks[best].bytes) best = i;
     }
   }

@@ -128,15 +128,19 @@ void draw_regions_device(visfd_ctx *ctx, i64 nx, i64 ny, i64 nz, float *img, con
 // ---- blob.cu ----------------------------------------------------------------------
 struct BlobList {
   std::vector<float> crds, sigma, score;  // crds: 3 per entry (x,y,z)
+  std::vector<i64> scale_rows;            // blob_dog_device: rows of each scale (n_sigmas entries), in list order
 };
-// slab form (whole image: z_offset 0, nz_global = nz, own planes [0, nz), finalize true); best: NULL or 2 floats
+// slab form (whole image: z_offset 0, nz_global = nz, own planes [0, nz), finalize true); best: NULL or 2 floats.
+// capacity_rows: rows of each device candidate list, 0 for the default (N / 32, at least 65536).
 void blob_dog_device(visfd_ctx *ctx, i64 nx, i64 ny, i64 nz, i64 z_offset, i64 nz_global, i64 own_z0, i64 own_z1,
                      const float *src, const float *mask,
                      const float *sigmas, int n_sigmas, float delta, float truncate_ratio,
                      float minima_threshold, float maxima_threshold, int use_threshold_ratios,
-                     BlobList &minima, BlobList &maxima, bool finalize, float best[2]);
+                     BlobList &minima, BlobList &maxima, bool finalize, float best[2], i64 capacity_rows = 0);
 void blob_final_filter(BlobList &minima, BlobList &maxima, float minima_threshold, float maxima_threshold,
                        int use_threshold_ratios, float gmin, float gmax);
+// (api.cu) the first `capacity` rows of l into the caller's HOST buffers (any may be NULL); *cnt: all rows.
+void emit_blob_list(const BlobList &l, int64_t capacity, float *crds, float *sg, float *sc, int64_t *cnt);
 
 // ---- util.cu ----------------------------------------------------------------------
 i64 tv_count_pairs_device(visfd_ctx *ctx, i64 nx, i64 ny, i64 nz, const float *sal, float thr,

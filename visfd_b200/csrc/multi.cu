@@ -7,6 +7,7 @@
 //     one device, the slabs one after another within a device-memory budget: volumes whose working set does not fit.
 // Their _background forms add `-membrane-background`: both scores multiplied by the peak height
 // source - Gauss(source, background_sigma), as visfd_cuda_membrane_background does on one GPU.
+// visfd_cuda_blob_dog_multi / visfd_cuda_blob_dog_stream do the same for BlobDog, in one pass (see below).
 //
 // The volume is cut into Z-slabs exactly as visfd_b200/slab.py does for the process-per-GPU driver (rank boundaries
 // on multiples of 8 planes, slabs widened by a halo of RAW SOURCE planes, halo = tv_halfwidth + 1 + gauss_halfwidth,
@@ -82,7 +83,7 @@ struct Background {
 std::mutex g_call_mutex;
 std::vector<std::pair<int, visfd_ctx *> > g_ctx;   // index = slot
 
-visfd_ctx *context_for(int slot, int device) {
+visfd_ctx *context_for(const char *name, int slot, int device) {
   if ((int)g_ctx.size() <= slot) g_ctx.resize((size_t)slot + 1, {-1, nullptr});
   auto &e = g_ctx[(size_t)slot];
   if (e.second && e.first != device) {
@@ -91,11 +92,33 @@ visfd_ctx *context_for(int slot, int device) {
   }
   if (!e.second) {
     visfd_ctx *c = nullptr;
-    if (visfd_cuda_init(device, &c) != 0) throw Error(std::string("visfd_cuda_membrane_multi: ") + visfd_cuda_last_error());
+    if (visfd_cuda_init(device, &c) != 0) throw Error(std::string(name) + ": " + visfd_cuda_last_error());
     e = {device, c};
   }
   return e.second;
 }
+
+// The device time of a multi worker, first upload to last download.
+struct DeviceClock {
+  cudaEvent_t start = nullptr, stop = nullptr;
+  double ms = 0.0;
+  void begin(cudaStream_t s) {
+    VCK(cudaEventCreate(&start));
+    VCK(cudaEventCreate(&stop));
+    VCK(cudaEventRecord(start, s));
+  }
+  void end(cudaStream_t s) {
+    VCK(cudaEventRecord(stop, s));
+    VCK(cudaEventSynchronize(stop));
+    float t = 0;
+    VCK(cudaEventElapsedTime(&t, start, stop));
+    ms = t;
+  }
+  ~DeviceClock() {
+    if (start) cudaEventDestroy(start);
+    if (stop) cudaEventDestroy(stop);
+  }
+};
 
 // What a slab keeps on its device from one step to the next.
 struct Slab {
@@ -103,13 +126,8 @@ struct Slab {
   SlabPlan plan;
   Scratch<float> mask, smoothed, saliency;
   Scratch<float> peak;   // with the background: the peak height of every plane of the slab, until the vote ends
-  cudaEvent_t start = nullptr, stop = nullptr;   // device time: first upload to last download
-  double ms = 0.0;
+  DeviceClock clock;
   uint64_t hist[HIST_BINS];
-  ~Slab() {
-    if (start) cudaEventDestroy(start);
-    if (stop) cudaEventDestroy(stop);
-  }
 };
 
 void make_slabs(std::vector<Slab> &slabs, const std::vector<SlabPlan> &plans, visfd_ctx *ctx) {
@@ -187,8 +205,8 @@ void vote_to_host(Slab &s, int64_t nx, int64_t ny, int64_t nz, float threshold, 
 // Runs fn(slab) for every slab at once, slab 0 on the calling thread and the others on threads of their own, each
 // on its slab's device.  Returns when all of them have finished, and then throws the error of the first slab that
 // failed.
-template <typename Fn>
-void for_each_slab(const char *name, std::vector<Slab> &slabs, const Fn &fn) {
+template <typename S, typename Fn>
+void for_each_slab(const char *name, std::vector<S> &slabs, const Fn &fn) {
   std::vector<std::string> errors(slabs.size());
   auto run = [&](size_t r) {
     try {
@@ -252,6 +270,45 @@ void release_cache(visfd_ctx *ctx) {
   ctx->trim();
 }
 
+// The budget of a stream call: device_bytes, or for 0 the free memory at entry less a margin.  Releases the cache
+// first: blocks cached by earlier calls count against the budget.
+int64_t stream_budget(visfd_ctx *ctx, int64_t device_bytes) {
+  VCK(cudaSetDevice(ctx->device));
+  drop_pending_stage_events(ctx);
+  release_cache(ctx);
+  if (device_bytes != 0) return device_bytes;
+  // the margin covers what the call needs outside the pool: the allocation granularity of cudaMalloc, code of
+  // kernels loaded on first use, local memory
+  size_t free_b = 0, total_b = 0;
+  VCK(cudaMemGetInfo(&free_b, &total_b));
+  return (int64_t)free_b - (int64_t)(1u << 30);
+}
+
+// The fewest slabs whose every slab fits the budget, 0 if none does; *need: the bytes of the largest slab of the last
+// plan tried.  bytes(plan) is what one slab holds at most.
+template <typename Bytes>
+int fewest_slabs(int64_t nz, int gauss_hw, int tv_hw, int bg_hw, int64_t budget, const Bytes &bytes, size_t *need) {
+  for (int world = 1; world <= max_slabs(nz); world++) {
+    *need = 0;
+    for (const SlabPlan &pl : make_plans(nz, world, gauss_hw, tv_hw, bg_hw)) *need = std::max(*need, bytes(pl));
+    if (*need <= (size_t)std::max<int64_t>(budget, 0)) return world;
+  }
+  return 0;
+}
+
+Error too_small(const std::string &who, const char *what, size_t need, int64_t budget) {
+  return Error(who + ": " + what + " needs " + std::to_string(need) +
+               " bytes of device memory in slabs of 8 planes; the budget is " + std::to_string(budget) + " bytes");
+}
+
+// After a failed stream call: nothing of it stays on the device, and the context takes the next call.
+void reset_after_failure(visfd_ctx *ctx) {
+  if (!ctx) return;
+  cudaStreamSynchronize(ctx->stream);
+  cudaGetLastError();
+  ctx->trim();
+}
+
 // The background of a _background entry point, checked; sigma 0: none (the plain entry points).
 Background background(const std::string &who, const visfd_membrane_params *p, float sigma, int normalize) {
   VREQUIRE(sigma >= 0.0f, who + ": negative background width");   // (NaN fails too)
@@ -282,13 +339,11 @@ int membrane_multi(const char *name, int ndev, const int *devices, int64_t nx, i
     std::lock_guard<std::mutex> lock(g_call_mutex);
     std::vector<Slab> slabs((size_t)world);
     make_slabs(slabs, plans, nullptr);
-    for (int r = 0; r < world; r++) slabs[(size_t)r].ctx = context_for(r, devices[r]);
+    for (int r = 0; r < world; r++) slabs[(size_t)r].ctx = context_for(name, r, devices[r]);
     auto concurrently = [&](const auto &step) { for_each_slab(name, slabs, step); };
 
     for_each_slab(name, slabs, [&](Slab &s) {
-      VCK(cudaEventCreate(&s.start));
-      VCK(cudaEventCreate(&s.stop));
-      VCK(cudaEventRecord(s.start, s.ctx->stream));
+      s.clock.begin(s.ctx->stream);
       upload_and_ridge(s, nx, ny, nz, src_host, mask_host, p, bg);
     });
 
@@ -300,16 +355,12 @@ int membrane_multi(const char *name, int ndev, const int *devices, int64_t nx, i
 
     for_each_slab(name, slabs, [&](Slab &s) {
       vote_to_host(s, nx, ny, nz, threshold, p, out_host);
-      VCK(cudaEventRecord(s.stop, s.ctx->stream));
-      VCK(cudaEventSynchronize(s.stop));
-      float t = 0;
-      VCK(cudaEventElapsedTime(&t, s.start, s.stop));
-      s.ms = t;
+      s.clock.end(s.ctx->stream);
     });
 
     if (threshold_out) *threshold_out = threshold;
     if (device_ms)
-      for (int r = 0; r < ndev; r++) device_ms[r] = r < world ? slabs[(size_t)r].ms : 0.0;
+      for (int r = 0; r < ndev; r++) device_ms[r] = r < world ? slabs[(size_t)r].clock.ms : 0.0;
     return 0;
   } catch (const std::exception &ex) {
     set_last_error(ex.what());
@@ -327,37 +378,16 @@ int membrane_stream(const char *name, visfd_ctx *ctx, int64_t nx, int64_t ny, in
     VREQUIRE(!is_device_pointer(src_host) && !is_device_pointer(out_host) && !is_device_pointer(mask_host),
              who + " takes HOST arrays (use visfd_cuda_membrane for device-resident data)");
     const Background bg = background(who, p, background_sigma, normalize);
-    VCK(cudaSetDevice(ctx->device));
-    drop_pending_stage_events(ctx);
-    release_cache(ctx);   // blocks cached by earlier calls count against the budget
-    int64_t budget = device_bytes;
-    if (budget == 0) {
-      // the margin covers what the call needs outside the pool: the allocation granularity of cudaMalloc, code
-      // of kernels loaded on first use, local memory
-      size_t free_b = 0, total_b = 0;
-      VCK(cudaMemGetInfo(&free_b, &total_b));
-      budget = (int64_t)free_b - (int64_t)(1u << 30);
-    }
+    const int64_t budget = stream_budget(ctx, device_bytes);
     const int gauss_hw = (int)floor(p->sigma * p->truncate_ratio);
     const int tv_hw = p->tv_sigma > 0.0f ? tv_halfwidth(p->tv_sigma, p->tv_cutoff_ratio) : 0;
     const size_t plane = (size_t)nx * (size_t)ny;
     const bool masked = mask_host != nullptr, vote = p->tv_sigma > 0.0f;
 
-    // The fewest slabs whose every slab fits the budget, 0 if none does; *need: the bytes of the largest slab of
-    // the last plan tried.
-    auto fewest_slabs = [&](bool vote_pass, uint64_t voters, size_t *need) {
-      for (int world = 1; world <= max_slabs(nz); world++) {
-        *need = 0;
-        for (const SlabPlan &pl : make_plans(nz, world, gauss_hw, tv_hw, bg.hw))
-          *need = std::max(*need, slab_bytes(pl, nx, ny, masked, p, gauss_hw, bg, vote_pass, voters));
-        if (*need <= (size_t)std::max<int64_t>(budget, 0)) return world;
-      }
-      return 0;
-    };
-    auto too_small = [&](const char *pass, size_t need) {
-      return Error(who + ": " + std::string(pass) + " needs " + std::to_string(need) +
-                   " bytes of device memory in slabs of 8 planes; the budget is " + std::to_string(budget) +
-                   " bytes");
+    auto fewest = [&](bool vote_pass, uint64_t voters, size_t *need) {
+      return fewest_slabs(nz, gauss_hw, tv_hw, bg.hw, budget, [&](const SlabPlan &pl) {
+        return slab_bytes(pl, nx, ny, masked, p, gauss_hw, bg, vote_pass, voters);
+      }, need);
     };
     // Runs step(slab) on every slab in turn, each after step (1) and each released before the next.
     auto one_by_one = [&](std::vector<Slab> &slabs, const auto &step) {
@@ -380,11 +410,11 @@ int membrane_stream(const char *name, visfd_ctx *ctx, int64_t nx, int64_t ny, in
     // The passes before the vote: the cut's rounds, or for an absolute cut one count of the voters when the vote
     // pass would otherwise need more slabs than these passes.  Their slabs are sized without voters.
     size_t need = 0;
-    const int n_cut = fewest_slabs(false, 0, &need);
-    if (n_cut == 0) throw too_small("the upload and ridge step", need);
+    const int n_cut = fewest(false, 0, &need);
+    if (n_cut == 0) throw too_small(who, "the upload and ridge step", need, budget);
     float threshold = p->cut;
     uint64_t voters = UINT64_MAX;   // unknown: every voxel of a slab's voter planes may vote
-    if (p->cut_is_fraction || (vote && fewest_slabs(true, voters, &need) != n_cut)) {
+    if (p->cut_is_fraction || (vote && fewest(true, voters, &need) != n_cut)) {
       std::vector<Slab> slabs((size_t)n_cut);
       make_slabs(slabs, make_plans(nz, n_cut, gauss_hw, tv_hw, bg.hw), ctx);
       auto in_turn = [&](const auto &step) { one_by_one(slabs, step); };
@@ -401,8 +431,8 @@ int membrane_stream(const char *name, visfd_ctx *ctx, int64_t nx, int64_t ny, in
       }
     }
 
-    const int n_vote = fewest_slabs(true, voters, &need);
-    if (n_vote == 0) throw too_small("the vote pass", need);
+    const int n_vote = fewest(true, voters, &need);
+    if (n_vote == 0) throw too_small(who, "the vote pass", need, budget);
     std::vector<Slab> slabs((size_t)n_vote);
     make_slabs(slabs, make_plans(nz, n_vote, gauss_hw, tv_hw, bg.hw), ctx);
     one_by_one(slabs, [&](Slab &s) {
@@ -415,11 +445,210 @@ int membrane_stream(const char *name, visfd_ctx *ctx, int64_t nx, int64_t ny, in
     return 0;
   } catch (const std::exception &ex) {
     set_last_error(ex.what());
-    if (ctx) {
-      cudaStreamSynchronize(ctx->stream);
-      cudaGetLastError();
-      ctx->trim();
+    reset_after_failure(ctx);
+    return 1;
+  }
+}
+
+// ---- BlobDog over Z-slabs ------------------------------------------------------------------------------------
+// A slab needs no collective before the end: it scans its own planes at every scale (blob_dog_device, slab form)
+// and keeps its lists and best scores on the host.  The lists are then concatenated per scale in slab order -- the
+// one-GPU (scale, z, y, x) order -- and the final filter runs once on the best scores of the whole image
+// (feature.hpp:341-344, :369-372).  In ratio mode a slab pre-filters on the device against the best scores of its
+// own earlier scales, a threshold never stricter than the global one, so the final filter decides.
+
+struct BlobArgs {
+  const float *sigmas;
+  int n_sigmas;
+  float delta, truncate_ratio, minima_threshold, maxima_threshold;
+  int use_threshold_ratios;
+};
+
+// The widest LoG half-width over the scales (log_params' arithmetic, as blob_dog_device checks the halo against):
+// a slab's halo is this + 1 planes of raw source.
+int blob_halfwidth(const BlobArgs &a) {
+  int widest = 0;
+  for (int i = 0; i < a.n_sigmas; i++) {
+    const float s3[3] = {a.sigmas[i], a.sigmas[i], a.sigmas[i]};
+    float sa[3], sb[3], scale;
+    int hw[3];
+    log_params(s3, a.delta, a.truncate_ratio, sa, sb, hw, &scale);
+    widest = std::max(widest, hw[2]);
+  }
+  return widest;
+}
+
+// Rows a candidate list of a slab with `own` planes needs for one scale: a strict extremum of its 26 neighbours
+// excludes every one of them, so at most one voxel of each 2x2x2 block is listed.  Lists this long cannot overflow,
+// so blob_dog_device never scans a scale again into larger lists, which would grow the pool past its plan.
+i64 blob_rows(int64_t nx, int64_t ny, int64_t own) { return ((nx + 1) / 2) * ((ny + 1) / 2) * ((own + 1) / 2); }
+
+struct BlobSlab {
+  visfd_ctx *ctx = nullptr;
+  SlabPlan plan;
+  BlobList minima, maxima;
+  float best[2] = {1.0f, -1.0f};
+  DeviceClock clock;
+};
+
+// Uploads the slab's planes, halo included, straight from the caller's arrays and scans its own planes.
+void blob_slab(BlobSlab &s, int64_t nx, int64_t ny, int64_t nz, const float *src_host, const float *mask_host,
+               const BlobArgs &a) {
+  const SlabPlan &pl = s.plan;
+  const size_t plane = (size_t)nx * (size_t)ny;
+  const size_t n = (size_t)(pl.slab1 - pl.slab0) * plane;
+  Scratch<float> src(s.ctx, n), mask;
+  {
+    StageTimer t(s.ctx, "h2d");
+    VCK(cudaMemcpyAsync(src.get(), src_host + (size_t)pl.slab0 * plane, n * sizeof(float), cudaMemcpyHostToDevice,
+                        s.ctx->stream));
+    if (mask_host) {
+      mask.reset(s.ctx, n);
+      VCK(cudaMemcpyAsync(mask.get(), mask_host + (size_t)pl.slab0 * plane, n * sizeof(float),
+                          cudaMemcpyHostToDevice, s.ctx->stream));
     }
+  }
+  blob_dog_device(s.ctx, nx, ny, pl.slab1 - pl.slab0, pl.slab0, nz, pl.own0 - pl.slab0, pl.own1 - pl.slab0,
+                  src.get(), mask.get(), a.sigmas, a.n_sigmas, a.delta, a.truncate_ratio, a.minima_threshold,
+                  a.maxima_threshold, a.use_threshold_ratios, s.minima, s.maxima, false, s.best,
+                  blob_rows(nx, ny, pl.own1 - pl.own0));
+  VCK(cudaStreamSynchronize(s.ctx->stream));
+  resolve_stage_times(s.ctx);
+}
+
+// The device bytes the pool holds at most while a slab of visfd_cuda_blob_dog_stream runs, in the blocks
+// visfd_ctx::alloc takes.  For the whole scan: the uploaded source and mask, the three LoG volumes, the two
+// candidate lists (blob_rows) and their counters.  At every scale dog_device adds the first Gaussian's volume and
+// the separable filter's scratch volume (with a mask also the two volumes of its normalisation), plus one small block
+// of taps and edge profiles at a time.  These come from the cache once the first scale has put them there, except
+// the small blocks: they grow with sigma, so each scale may add up to two new ones (the shared Z sweep's taps and
+// the filter's constants), and a small request that takes a cached volume (visfd_ctx::reuses: tiny volumes) makes
+// the next volume request a new block.
+size_t blob_slab_bytes(const SlabPlan &pl, int64_t nx, int64_t ny, bool masked, int log_hw, int n_sigmas) {
+  const int64_t slab = pl.slab1 - pl.slab0;
+  const size_t vol = visfd_ctx::block_bytes((size_t)slab * (size_t)nx * (size_t)ny * sizeof(float));
+  const size_t lists = 2 * visfd_ctx::block_bytes((size_t)blob_rows(nx, ny, pl.own1 - pl.own0) * 4 * sizeof(float)) +
+                       visfd_ctx::block_bytes(2 * sizeof(unsigned long long));
+  // dog_device's largest small request: both Gaussians' taps and edge profiles
+  const size_t small = visfd_ctx::block_bytes(2 * (size_t)(3 * (2 * log_hw + 1) + nx + ny + slab) * sizeof(float));
+  const size_t scan = (masked ? 5 : 4) * vol + lists;
+  const size_t dog = (masked ? 4 : 2) * vol + 2 * (size_t)n_sigmas * small +
+                     (visfd_ctx::reuses(vol, small) ? vol : 0);
+  return scan + dog;
+}
+
+void check_blob_args(const std::string &who, int64_t nx, int64_t ny, int64_t nz, const float *src_host,
+                     const float *mask_host, const BlobArgs &a, int64_t capacity,
+                     const std::vector<const float *> &outputs) {
+  VREQUIRE(nx > 0 && ny > 0 && nz > 0 && src_host && (a.sigmas || a.n_sigmas == 0) && a.n_sigmas >= 0 &&
+               capacity >= 0,
+           who + ": bad arguments");
+  bool host = !is_device_pointer(src_host) && !is_device_pointer(mask_host);
+  for (const float *o : outputs) host = host && !is_device_pointer(o);
+  VREQUIRE(host, who + " takes HOST arrays (use visfd_cuda_blob_dog_slab for device-resident data)");
+}
+
+// The slabs' lists per scale in slab order, the best scores of the whole image, the final filter, and the first
+// `capacity` rows into the caller's buffers.
+void finish_blobs(const std::vector<BlobSlab> &slabs, const BlobArgs &a, int64_t capacity, float *min_crds,
+                  float *min_sigma, float *min_score, int64_t *n_minima, float *max_crds, float *max_sigma,
+                  float *max_score, int64_t *n_maxima) {
+  auto concat = [&](BlobList BlobSlab::*list) {
+    BlobList out;
+    std::vector<size_t> at(slabs.size(), 0);   // next row of each slab
+    for (int i = 0; i < a.n_sigmas; i++)
+      for (size_t r = 0; r < slabs.size(); r++) {
+        const BlobList &l = slabs[r].*list;
+        const size_t k0 = at[r], k1 = k0 + (size_t)l.scale_rows[(size_t)i];
+        out.crds.insert(out.crds.end(), l.crds.begin() + 3 * k0, l.crds.begin() + 3 * k1);
+        out.sigma.insert(out.sigma.end(), l.sigma.begin() + k0, l.sigma.begin() + k1);
+        out.score.insert(out.score.end(), l.score.begin() + k0, l.score.begin() + k1);
+        at[r] = k1;
+      }
+    return out;
+  };
+  BlobList minima = concat(&BlobSlab::minima), maxima = concat(&BlobSlab::maxima);
+  float gmin = 1.0f, gmax = -1.0f;   // feature.hpp:122-123
+  for (const BlobSlab &s : slabs) {
+    gmin = std::min(gmin, s.best[0]);
+    gmax = std::max(gmax, s.best[1]);
+  }
+  blob_final_filter(minima, maxima, a.minima_threshold, a.maxima_threshold, a.use_threshold_ratios, gmin, gmax);
+  emit_blob_list(minima, capacity, min_crds, min_sigma, min_score, n_minima);
+  emit_blob_list(maxima, capacity, max_crds, max_sigma, max_score, n_maxima);
+}
+
+int blob_multi(const char *name, int ndev, const int *devices, int64_t nx, int64_t ny, int64_t nz,
+               const float *src_host, const float *mask_host, const BlobArgs &a, int64_t capacity, float *min_crds,
+               float *min_sigma, float *min_score, int64_t *n_minima, float *max_crds, float *max_sigma,
+               float *max_score, int64_t *n_maxima, double *device_ms) {
+  try {
+    const std::string who(name);
+    VREQUIRE(ndev >= 1 && devices, who + ": need at least one device");
+    check_blob_args(who, nx, ny, nz, src_host, mask_host, a, capacity,
+                    {min_crds, min_sigma, min_score, max_crds, max_sigma, max_score});
+    const int world = std::min(ndev, max_slabs(nz));
+    const std::vector<SlabPlan> plans = make_plans(nz, world, blob_halfwidth(a), 0, 0);
+
+    std::lock_guard<std::mutex> lock(g_call_mutex);
+    std::vector<BlobSlab> slabs((size_t)world);
+    for (int r = 0; r < world; r++) {
+      slabs[(size_t)r].plan = plans[(size_t)r];
+      slabs[(size_t)r].ctx = context_for(name, r, devices[r]);
+    }
+    for_each_slab(name, slabs, [&](BlobSlab &s) {
+      drop_pending_stage_events(s.ctx);
+      s.clock.begin(s.ctx->stream);
+      blob_slab(s, nx, ny, nz, src_host, mask_host, a);
+      s.clock.end(s.ctx->stream);
+    });
+    finish_blobs(slabs, a, capacity, min_crds, min_sigma, min_score, n_minima, max_crds, max_sigma, max_score,
+                 n_maxima);
+    if (device_ms)
+      for (int r = 0; r < ndev; r++) device_ms[r] = r < world ? slabs[(size_t)r].clock.ms : 0.0;
+    return 0;
+  } catch (const std::exception &ex) {
+    set_last_error(ex.what());
+    return 1;
+  }
+}
+
+int blob_stream(const char *name, visfd_ctx *ctx, int64_t nx, int64_t ny, int64_t nz, const float *src_host,
+                const float *mask_host, const BlobArgs &a, int64_t device_bytes, int64_t capacity, float *min_crds,
+                float *min_sigma, float *min_score, int64_t *n_minima, float *max_crds, float *max_sigma,
+                float *max_score, int64_t *n_maxima, int64_t *n_slabs_out) {
+  try {
+    const std::string who(name);
+    VREQUIRE(ctx != nullptr, who + ": context is NULL");
+    VREQUIRE(device_bytes >= 0, who + ": bad arguments");
+    check_blob_args(who, nx, ny, nz, src_host, mask_host, a, capacity,
+                    {min_crds, min_sigma, min_score, max_crds, max_sigma, max_score});
+    const int64_t budget = stream_budget(ctx, device_bytes);
+    const int log_hw = blob_halfwidth(a);
+    size_t need = 0;
+    const int n = fewest_slabs(nz, log_hw, 0, 0, budget, [&](const SlabPlan &pl) {
+      return blob_slab_bytes(pl, nx, ny, mask_host != nullptr, log_hw, a.n_sigmas);
+    }, &need);
+    if (n == 0) throw too_small(who, "blob detection", need, budget);
+    const std::vector<SlabPlan> plans = make_plans(nz, n, log_hw, 0, 0);
+    std::vector<BlobSlab> slabs((size_t)n);
+    for (size_t r = 0; r < slabs.size(); r++) {
+      slabs[r].ctx = ctx;
+      slabs[r].plan = plans[r];
+      try {
+        blob_slab(slabs[r], nx, ny, nz, src_host, mask_host, a);
+      } catch (const std::exception &ex) {
+        throw Error(who + ", slab " + std::to_string(r) + " of " + std::to_string(n) + ": " + ex.what());
+      }
+      release_cache(ctx);
+    }
+    finish_blobs(slabs, a, capacity, min_crds, min_sigma, min_score, n_minima, max_crds, max_sigma, max_score,
+                 n_maxima);
+    if (n_slabs_out) *n_slabs_out = n;
+    return 0;
+  } catch (const std::exception &ex) {
+    set_last_error(ex.what());
+    reset_after_failure(ctx);
     return 1;
   }
 }
@@ -459,4 +688,28 @@ extern "C" int visfd_cuda_membrane_stream_background(visfd_ctx *ctx, int64_t nx,
   return membrane_stream("visfd_cuda_membrane_stream_background", ctx, nx, ny, nz, src_host, mask_host, p,
                          background_sigma, normalize_near_boundaries, device_bytes, out_host, threshold_out,
                          n_slabs_out);
+}
+
+extern "C" int visfd_cuda_blob_dog_multi(int ndev, const int *devices, int64_t nx, int64_t ny, int64_t nz,
+                                         const float *src_host, const float *mask_host, const float *sigmas,
+                                         int n_sigmas, float delta, float truncate_ratio, float minima_threshold,
+                                         float maxima_threshold, int use_threshold_ratios, int64_t capacity,
+                                         float *min_crds, float *min_sigma, float *min_score, int64_t *n_minima,
+                                         float *max_crds, float *max_sigma, float *max_score, int64_t *n_maxima,
+                                         double *device_ms) {
+  const BlobArgs a{sigmas, n_sigmas, delta, truncate_ratio, minima_threshold, maxima_threshold, use_threshold_ratios};
+  return blob_multi("visfd_cuda_blob_dog_multi", ndev, devices, nx, ny, nz, src_host, mask_host, a, capacity,
+                    min_crds, min_sigma, min_score, n_minima, max_crds, max_sigma, max_score, n_maxima, device_ms);
+}
+
+extern "C" int visfd_cuda_blob_dog_stream(visfd_ctx *ctx, int64_t nx, int64_t ny, int64_t nz, const float *src_host,
+                                          const float *mask_host, const float *sigmas, int n_sigmas, float delta,
+                                          float truncate_ratio, float minima_threshold, float maxima_threshold,
+                                          int use_threshold_ratios, int64_t device_bytes, int64_t capacity,
+                                          float *min_crds, float *min_sigma, float *min_score, int64_t *n_minima,
+                                          float *max_crds, float *max_sigma, float *max_score, int64_t *n_maxima,
+                                          int64_t *n_slabs_out) {
+  const BlobArgs a{sigmas, n_sigmas, delta, truncate_ratio, minima_threshold, maxima_threshold, use_threshold_ratios};
+  return blob_stream("visfd_cuda_blob_dog_stream", ctx, nx, ny, nz, src_host, mask_host, a, device_bytes, capacity,
+                     min_crds, min_sigma, min_score, n_minima, max_crds, max_sigma, max_score, n_maxima, n_slabs_out);
 }

@@ -256,10 +256,13 @@ inline void BlobDog(int const image_size[3], float const *const *const *aaafSour
   for (int attempt = 0; attempt < 2; attempt++) {
     mc.resize(3 * capacity); ms.resize(capacity); msc.resize(capacity);
     xc.resize(3 * capacity); xs.resize(capacity); xsc.resize(capacity);
-    Check(visfd_cuda_blob_dog(Context(), image_size[0], image_size[1], image_size[2], s.data(), m.data(),
-                              blob_sigma.data(), (int)blob_sigma.size(), delta_sigma_over_sigma, truncate_ratio,
-                              minima_threshold, maxima_threshold, use_threshold_ratios ? 1 : 0, capacity, mc.data(),
-                              ms.data(), msc.data(), &nmin, xc.data(), xs.data(), xsc.data(), &nmax));
+    // in Z-slabs within the GPU's free memory: one slab, and the one-GPU lists, when the volume fits; several
+    // slabs, and still the same lists, when it does not
+    Check(visfd_cuda_blob_dog_stream(Context(), image_size[0], image_size[1], image_size[2], s.data(), m.data(),
+                                     blob_sigma.data(), (int)blob_sigma.size(), delta_sigma_over_sigma,
+                                     truncate_ratio, minima_threshold, maxima_threshold, use_threshold_ratios ? 1 : 0,
+                                     0, capacity, mc.data(), ms.data(), msc.data(), &nmin, xc.data(), xs.data(),
+                                     xsc.data(), &nmax, nullptr));
     if (nmin <= capacity && nmax <= capacity) break;
     capacity = std::max(nmin, nmax);
   }
