@@ -527,6 +527,48 @@ int visfd_cuda_blob_dog_stream(visfd_ctx *ctx, int64_t nx, int64_t ny, int64_t n
                                float *max_crds, float *max_sigma, float *max_score, int64_t *n_maxima,
                                int64_t *n_slabs_out);
 
+/* ApplyGauss, ApplyDog and ApplyLog with HOST arrays, in Z-slabs: on several GPUs of one node (multi) or on one GPU
+ * slab after slab within a device-memory budget (stream).  dst_host, *A_out and *B_out are bit-identical to the
+ * one-shot call with the same arguments, for any number of slabs, with or without a mask and in both arithmetic
+ * modes (visfd_cuda_set_fast_gauss):
+ *   VISFD_FILTER_GAUSS  visfd_cuda_apply_gauss(sigma_a, hw_a, normalize)      (*B_out: 0)
+ *   VISFD_FILTER_DOG    visfd_cuda_apply_dog2(sigma_a, sigma_b, hw_a, hw_b)
+ *   VISFD_FILTER_LOG    visfd_cuda_apply_log(sigma_a, delta, truncate_ratio)
+ * The fields a kind does not name are ignored.  src_host, mask_host (may be NULL) and dst_host must be HOST arrays:
+ * a device pointer fails (use the one-shot calls for device-resident data).  dst_host may be src_host, as for the
+ * one-shot host call; the mask must not share memory with dst_host, nor dst_host with src_host unless they are equal.
+ * The volume is cut as visfd_cuda_membrane_multi cuts it, with a halo of (the filter's Z half-width + 1) planes of
+ * raw source, which each slab uploads straight from src_host; each slab filters with the whole volume's borders and
+ * writes its own planes into dst_host.
+ * multi: one slab per entry of devices[] (a device may be listed more than once), all at once; the slabs deliver
+ * only after every slab has uploaded.  It shares its per-entry contexts, and their arithmetic mode
+ * (VISFD_CUDA_FAST_GAUSS), with visfd_cuda_membrane_multi, and one multi call of any kind runs at a time; it
+ * releases the slabs' device memory before it returns.  device_ms (ndev doubles or NULL): device time of each slab,
+ * first upload to delivery.  An error names the slab and its device.
+ * stream: on ctx, in its arithmetic mode; the fewest slabs whose every slab fits device_bytes (0 = the free memory at
+ * entry, less a margin), each released before the next.  A slab holds its source, mask and result and the filter's
+ * scratch: one slab needs what the one-shot call needs.  The call fails, naming the bytes it needs, when slabs of 8
+ * planes do not fit; the context stays usable after any failure.  With dst_host == src_host the raw planes a later
+ * slab still reads are kept in host memory (at most halo + 7 planes) before a slab writes over them.
+ * *n_slabs_out (may be NULL): slabs used. */
+enum { VISFD_FILTER_GAUSS = 0, VISFD_FILTER_DOG = 1, VISFD_FILTER_LOG = 2 };
+typedef struct visfd_filter_params {
+  int kind;              /* VISFD_FILTER_*                                                    */
+  float sigma_a[3];      /* GAUSS: sigma;  DOG: sigma_a;  LOG: sigma                          */
+  float sigma_b[3];      /* DOG only                                                          */
+  int hw_a[3];           /* GAUSS, DOG: half-widths of the (first) Gaussian                   */
+  int hw_b[3];           /* DOG: of the second one (filter_mrc's ApplyDog, apply_dog2)        */
+  int normalize;         /* GAUSS only; DoG and LoG always normalise                          */
+  float delta;           /* LOG: delta_sigma_over_sigma                                       */
+  float truncate_ratio;  /* LOG                                                               */
+} visfd_filter_params;
+int visfd_cuda_filter_multi(int ndev, const int *devices, int64_t nx, int64_t ny, int64_t nz,
+                            const float *src_host, const float *mask_host, const visfd_filter_params *p,
+                            float *dst_host, float *A_out, float *B_out, double *device_ms);
+int visfd_cuda_filter_stream(visfd_ctx *ctx, int64_t nx, int64_t ny, int64_t nz, const float *src_host,
+                             const float *mask_host, const visfd_filter_params *p, int64_t device_bytes,
+                             float *dst_host, float *A_out, float *B_out, int64_t *n_slabs_out);
+
 #ifdef __cplusplus
 }
 #endif

@@ -252,6 +252,56 @@ def blob_dog_multi(devices, src, sigmas, delta=0.02, truncate_ratio=2.5, mask=No
     return dict(minima=minima, maxima=maxima, device_ms=list(ms))
 
 
+class FilterParams(C.Structure):
+    """visfd_filter_params: the filter of filter_multi / Context.filter_stream.  Build it with gauss(), dog() or
+    log(), which take the arguments of Context.apply_gauss, apply_dog and apply_log."""
+    GAUSS, DOG, LOG = 0, 1, 2
+    _fields_ = [("kind", _i), ("sigma_a", _f * 3), ("sigma_b", _f * 3), ("hw_a", _i * 3), ("hw_b", _i * 3),
+                ("normalize", _i), ("delta", _f), ("truncate_ratio", _f)]
+
+    @classmethod
+    def gauss(cls, sigma, hw, normalize=True):
+        return cls(kind=cls.GAUSS, sigma_a=_f3(sigma), hw_a=_i3(hw), normalize=int(normalize))
+
+    @classmethod
+    def dog(cls, sigma_a, sigma_b, hw, hw_b=None):
+        return cls(kind=cls.DOG, sigma_a=_f3(sigma_a), sigma_b=_f3(sigma_b), hw_a=_i3(hw),
+                   hw_b=_i3(hw if hw_b is None else hw_b))
+
+    @classmethod
+    def log(cls, sigma, delta=0.02, truncate_ratio=2.5):
+        return cls(kind=cls.LOG, sigma_a=_f3(sigma), delta=delta, truncate_ratio=truncate_ratio)
+
+
+def _host_filter_args(who, src, mask, out):
+    """numpy host arrays for the filter slab drivers (which refuse device memory); out may be src"""
+    if _is_torch(src) or _is_torch(mask) or _is_torch(out):
+        raise VisfdCudaError(f"{who} takes numpy (host) arrays")
+    src = np.ascontiguousarray(src, np.float32)
+    mask = None if mask is None else np.ascontiguousarray(mask, np.float32)
+    res = out if out is not None else np.empty(src.shape, np.float32)
+    assert isinstance(res, np.ndarray) and res.dtype == np.float32 and res.flags.c_contiguous and res.shape == src.shape
+    return src, mask, res
+
+
+def filter_multi(devices, src, params, mask=None, out=None, lib=None):
+    """visfd_cuda_filter_multi: ApplyGauss / ApplyDog / ApplyLog (params: FilterParams) on several GPUs of this node
+    behind one C call, one Z-slab per entry of devices (a device may appear more than once).  numpy (host) arrays
+    only; out may be src.  -> dict(out, A, B, device_ms), bit-identical to Context.apply_gauss / apply_dog /
+    apply_log."""
+    lib = lib or load_library()
+    src, mask, res = _host_filter_args("visfd_cuda_filter_multi", src, mask, out)
+    devs = (C.c_int * len(devices))(*[int(d) for d in devices])
+    ms = (C.c_double * len(devices))()
+    A, B = _f(), _f()
+    nz, ny, nx = src.shape
+    rc = lib.visfd_cuda_filter_multi(_i(len(devices)), devs, _i64(nx), _i64(ny), _i64(nz), _ptr(src), _ptr(mask),
+                                     C.byref(params), _ptr(res), C.byref(A), C.byref(B), ms)
+    if rc != 0:
+        raise VisfdCudaError(lib.visfd_cuda_last_error().decode())
+    return dict(out=res, A=A.value, B=B.value, device_ms=list(ms))
+
+
 class Context:
     """One context per GPU (visfd_cuda_init)."""
 
@@ -572,6 +622,18 @@ class Context:
                                                          C.byref(p), _i64(int(device_bytes)), _ptr(res), C.byref(thr),
                                                          C.byref(n_slabs)))
         return dict(out=res, threshold=thr.value, n_slabs=n_slabs.value)
+
+    def filter_stream(self, src, params, mask=None, device_bytes=0, out=None):
+        """visfd_cuda_filter_stream: ApplyGauss / ApplyDog / ApplyLog (params: FilterParams) on this context's GPU in
+        Z-slabs run one after another, for volumes that do not fit on it; the device memory the call reserves stays
+        within device_bytes (0: the free memory at entry, less a margin).  numpy (host) arrays only; out may be src.
+        -> dict(out, A, B, n_slabs), bit-identical to apply_gauss / apply_dog / apply_log."""
+        src, mask, res = _host_filter_args("visfd_cuda_filter_stream", src, mask, out)
+        A, B, n_slabs = _f(), _f(), _i64()
+        self._ck(self.lib.visfd_cuda_filter_stream(self.h, *self._dims(src.shape), _ptr(src), _ptr(mask),
+                                                   C.byref(params), _i64(int(device_bytes)), _ptr(res), C.byref(A),
+                                                   C.byref(B), C.byref(n_slabs)))
+        return dict(out=res, A=A.value, B=B.value, n_slabs=n_slabs.value)
 
     # ---- slab stages (device tensors only) -----------------------------------------------------------------
     def ridge_saliency_slab(self, src, z_offset, nz_global, sigma, truncate_ratio, order=DECREASING_EIVALS,

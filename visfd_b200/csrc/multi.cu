@@ -7,7 +7,8 @@
 //     one device, the slabs one after another within a device-memory budget: volumes whose working set does not fit.
 // Their _background forms add `-membrane-background`: both scores multiplied by the peak height
 // source - Gauss(source, background_sigma), as visfd_cuda_membrane_background does on one GPU.
-// visfd_cuda_blob_dog_multi / visfd_cuda_blob_dog_stream do the same for BlobDog, in one pass (see below).
+// visfd_cuda_blob_dog_multi / visfd_cuda_blob_dog_stream do the same for BlobDog, in one pass (see below), and
+// visfd_cuda_filter_multi / visfd_cuda_filter_stream for ApplyGauss, ApplyDog and ApplyLog.
 //
 // The volume is cut into Z-slabs exactly as visfd_b200/slab.py does for the process-per-GPU driver (rank boundaries
 // on multiples of 8 planes, slabs widened by a halo of RAW SOURCE planes, halo = tv_halfwidth + 1 + gauss_halfwidth,
@@ -653,7 +654,266 @@ int blob_stream(const char *name, visfd_ctx *ctx, int64_t nx, int64_t ny, int64_
   }
 }
 
+// ---- ApplyGauss / ApplyDog / ApplyLog over Z-slabs -----------------------------------------------------------
+// A slab uploads its planes, halo included, runs the slab form of gauss_device / dog_device (z_offset = its first
+// plane, nz_global = nz: zero taps, edge profiles and masked denominators are those of the whole volume) and
+// delivers its own planes into the caller's array.  The halo is the filter's Z half-width.
+// dst_host may be src_host, as for the one-shot host call: delivering a slab overwrites raw planes that later slabs
+// read as their lower halo, so multi delivers only once every slab has uploaded, and stream keeps those planes in
+// a host buffer (the carry) before it delivers.
+
+// A checked visfd_filter_params: both Gaussians' sigmas and half-widths (a Gaussian alone: the same one twice).
+struct Filter {
+  int kind = VISFD_FILTER_GAUSS;
+  float sa[3], sb[3];
+  int hwa[3], hwb[3];
+  bool normalize = true;
+  float scale = 1.0f;   // LoG: 1 / delta^2
+  int z_halfwidth() const { return std::max(hwa[2], hwb[2]); }
+};
+
+Filter filter_args(const std::string &who, const visfd_filter_params *p) {
+  VREQUIRE(p != nullptr, who + ": params is NULL");
+  VREQUIRE(p->kind == VISFD_FILTER_GAUSS || p->kind == VISFD_FILTER_DOG || p->kind == VISFD_FILTER_LOG,
+           who + ": unknown filter kind " + std::to_string(p->kind));
+  Filter f;
+  f.kind = p->kind;
+  f.normalize = p->normalize != 0;
+  const bool dog = p->kind == VISFD_FILTER_DOG;
+  if (p->kind == VISFD_FILTER_LOG) {
+    log_params(p->sigma_a, p->delta, p->truncate_ratio, f.sa, f.sb, f.hwa, &f.scale);   // as visfd_cuda_apply_log
+    std::copy(f.hwa, f.hwa + 3, f.hwb);
+  } else {
+    std::copy(p->sigma_a, p->sigma_a + 3, f.sa);
+    std::copy(p->hw_a, p->hw_a + 3, f.hwa);
+    std::copy(dog ? p->sigma_b : p->sigma_a, (dog ? p->sigma_b : p->sigma_a) + 3, f.sb);
+    std::copy(dog ? p->hw_b : p->hw_a, (dog ? p->hw_b : p->hw_a) + 3, f.hwb);
+  }
+  for (int d = 0; d < 3; d++)   // (NaN fails too)
+    VREQUIRE(f.sa[d] >= 0.0f && f.sb[d] >= 0.0f && f.hwa[d] >= 0 && f.hwb[d] >= 0,
+             who + ": negative sigma or half-width");
+  return f;
+}
+
+bool overlap(const float *a, const float *b, size_t n) {
+  const uintptr_t x = (uintptr_t)a, y = (uintptr_t)b, bytes = n * sizeof(float);
+  return x < y + bytes && y < x + bytes;
+}
+
+void check_filter_args(const std::string &who, int64_t nx, int64_t ny, int64_t nz, const float *src_host,
+                       const float *mask_host, const float *dst_host) {
+  VREQUIRE(nx > 0 && ny > 0 && nz > 0 && nx < (1LL << 31) && ny < (1LL << 31) && nz < (1LL << 31) && src_host &&
+               dst_host,
+           who + ": bad arguments");
+  VREQUIRE(!is_device_pointer(src_host) && !is_device_pointer(mask_host) && !is_device_pointer(dst_host),
+           who + " takes HOST arrays (use visfd_cuda_apply_gauss / _dog2 / _log for device-resident data)");
+  const size_t n = (size_t)nx * (size_t)ny * (size_t)nz;
+  VREQUIRE(!mask_host || !overlap(mask_host, dst_host, n), who + ": the mask must not share memory with dst");
+  VREQUIRE(dst_host == src_host || !overlap(src_host, dst_host, n), who + ": dst must be src or apart from it");
+}
+
+struct FilterSlab {
+  visfd_ctx *ctx = nullptr;
+  SlabPlan plan;
+  Scratch<float> out;   // every plane of the slab, filtered
+  float A = 0.0f, B = 0.0f;
+  DeviceClock clock;
+};
+
+// Uploads the slab's planes, halo included, and filters them into s.out.  carry (may be NULL): raw source planes
+// from global plane carry0 up to the slab's own0, which the upload takes instead of the caller's array.
+void filter_slab(FilterSlab &s, const Filter &f, int64_t nx, int64_t ny, int64_t nz, const float *src_host,
+                 const float *mask_host, const float *carry, int64_t carry0) {
+  const SlabPlan &pl = s.plan;
+  const size_t plane = (size_t)nx * (size_t)ny;
+  const int64_t nzl = pl.slab1 - pl.slab0;
+  const size_t n = (size_t)nzl * plane;
+  const int64_t split = carry ? pl.own0 : pl.slab0;   // the planes below it come from the carry
+  Scratch<float> src(s.ctx, n), mask;
+  s.out.reset(s.ctx, n);
+  {
+    StageTimer t(s.ctx, "h2d");
+    if (split > pl.slab0)
+      VCK(cudaMemcpyAsync(src.get(), carry + (size_t)(pl.slab0 - carry0) * plane,
+                          (size_t)(split - pl.slab0) * plane * sizeof(float), cudaMemcpyHostToDevice, s.ctx->stream));
+    VCK(cudaMemcpyAsync(src.get() + (size_t)(split - pl.slab0) * plane, src_host + (size_t)split * plane,
+                        (size_t)(pl.slab1 - split) * plane * sizeof(float), cudaMemcpyHostToDevice, s.ctx->stream));
+    if (mask_host) {
+      mask.reset(s.ctx, n);
+      VCK(cudaMemcpyAsync(mask.get(), mask_host + (size_t)pl.slab0 * plane, n * sizeof(float),
+                          cudaMemcpyHostToDevice, s.ctx->stream));
+    }
+  }
+  if (f.kind == VISFD_FILTER_GAUSS) {
+    s.A = gauss_device(s.ctx, nx, ny, nzl, pl.slab0, nz, src.get(), s.out.get(), mask.get(), f.sa, f.hwa, f.normalize,
+                       nullptr, 1.0f);
+  } else {
+    dog_device(s.ctx, nx, ny, nzl, pl.slab0, nz, src.get(), s.out.get(), mask.get(), f.sa, f.sb, f.hwa, f.scale, &s.A,
+               &s.B, f.hwb);
+    if (f.kind == VISFD_FILTER_LOG) {   // as visfd_cuda_apply_log_slab: the peak heights are scaled as well
+      s.A *= f.scale;
+      s.B *= f.scale;
+    }
+  }
+  // the upload has read the caller's planes once this returns: a delivery may overwrite them
+  VCK(cudaStreamSynchronize(s.ctx->stream));
+  resolve_stage_times(s.ctx);
+}
+
+// Copies the slab's own planes into the caller's array.
+void deliver_slab(FilterSlab &s, int64_t nx, int64_t ny, float *dst_host) {
+  const SlabPlan &pl = s.plan;
+  const size_t plane = (size_t)nx * (size_t)ny;
+  {
+    StageTimer t(s.ctx, "d2h");
+    VCK(cudaMemcpyAsync(dst_host + (size_t)pl.own0 * plane, s.out.get() + (size_t)(pl.own0 - pl.slab0) * plane,
+                        (size_t)(pl.own1 - pl.own0) * plane * sizeof(float), cudaMemcpyDeviceToHost, s.ctx->stream));
+  }
+  VCK(cudaStreamSynchronize(s.ctx->stream));
+  resolve_stage_times(s.ctx);
+}
+
+// The device bytes the pool holds at most while a slab of visfd_cuda_filter_stream runs, in the blocks
+// visfd_ctx::alloc takes: the source (+ mask) and the filtered slab, plus the filter's workspace.  After the trim
+// that precedes every slab the pool cannot hold more than the sum of the filter's requests.  A Gaussian's
+// requests are separable_workspace_bytes.  DoG and LoG add the first Gaussian's volume to one of dog_device's two
+// paths, chosen from the slab's shape (x2_qualifies on ny times its planes), so both are counted: the fused path's
+// block of both filters' taps and edge profiles plus one scratch volume, or the shared Z sweep's taps plus both
+// Gaussians' separable workspaces.
+size_t filter_slab_bytes(const SlabPlan &pl, int64_t nx, int64_t ny, bool masked, const Filter &f) {
+  const int64_t slab = pl.slab1 - pl.slab0;
+  const size_t vol = visfd_ctx::block_bytes((size_t)slab * (size_t)nx * (size_t)ny * sizeof(float));
+  const size_t held = (masked ? 3 : 2) * vol;
+  if (f.kind == VISFD_FILTER_GAUSS) return held + separable_workspace_bytes(nx, ny, slab, f.hwa, masked, f.normalize);
+  const size_t per = (size_t)(2 * f.hwa[0] + 1 + 2 * f.hwa[1] + 1 + 2 * f.hwa[2] + 1 + nx + ny + slab);
+  const size_t fused = visfd_ctx::block_bytes(2 * per * sizeof(float)) + vol;
+  const size_t two_calls = visfd_ctx::block_bytes(2 * (size_t)(2 * f.z_halfwidth() + 1) * sizeof(float)) +
+                           separable_workspace_bytes(nx, ny, slab, f.hwa, masked, true) +
+                           separable_workspace_bytes(nx, ny, slab, f.hwb, masked, true);
+  return held + vol + std::max(fused, two_calls);
+}
+
+int filter_multi(const char *name, int ndev, const int *devices, int64_t nx, int64_t ny, int64_t nz,
+                 const float *src_host, const float *mask_host, const visfd_filter_params *p, float *dst_host,
+                 float *A_out, float *B_out, double *device_ms) {
+  try {
+    const std::string who(name);
+    VREQUIRE(ndev >= 1 && devices, who + ": need at least one device");
+    check_filter_args(who, nx, ny, nz, src_host, mask_host, dst_host);
+    const Filter f = filter_args(who, p);
+    const int world = std::min(ndev, max_slabs(nz));
+    const std::vector<SlabPlan> plans = make_plans(nz, world, f.z_halfwidth(), 0, 0);
+
+    std::lock_guard<std::mutex> lock(g_call_mutex);
+    std::vector<FilterSlab> slabs((size_t)world);
+    for (int r = 0; r < world; r++) {
+      slabs[(size_t)r].plan = plans[(size_t)r];
+      slabs[(size_t)r].ctx = context_for(name, r, devices[r]);
+    }
+    for_each_slab(name, slabs, [&](FilterSlab &s) {
+      drop_pending_stage_events(s.ctx);
+      s.clock.begin(s.ctx->stream);
+      filter_slab(s, f, nx, ny, nz, src_host, mask_host, nullptr, 0);
+    });
+    // every slab has read its planes: delivering cannot overwrite a plane that a slab has still to read
+    for_each_slab(name, slabs, [&](FilterSlab &s) {
+      deliver_slab(s, nx, ny, dst_host);
+      s.out.free();
+      s.clock.end(s.ctx->stream);
+      // a slab's blocks are volume-sized and a later call's slabs may not fit them: cached, they would keep that
+      // memory from every other context on the device
+      release_cache(s.ctx);
+    });
+
+    if (A_out) *A_out = slabs[0].A;   // the peak heights depend on the taps alone
+    if (B_out) *B_out = slabs[0].B;
+    if (device_ms)
+      for (int r = 0; r < ndev; r++) device_ms[r] = r < world ? slabs[(size_t)r].clock.ms : 0.0;
+    return 0;
+  } catch (const std::exception &ex) {
+    set_last_error(ex.what());
+    return 1;
+  }
+}
+
+int filter_stream(const char *name, visfd_ctx *ctx, int64_t nx, int64_t ny, int64_t nz, const float *src_host,
+                  const float *mask_host, const visfd_filter_params *p, int64_t device_bytes, float *dst_host,
+                  float *A_out, float *B_out, int64_t *n_slabs_out) {
+  try {
+    const std::string who(name);
+    check_filter_args(who, nx, ny, nz, src_host, mask_host, dst_host);
+    const Filter f = filter_args(who, p);
+    VREQUIRE(device_bytes >= 0, who + ": negative device_bytes");
+    VREQUIRE(ctx != nullptr, who + ": context is NULL");
+    const int64_t budget = stream_budget(ctx, device_bytes);
+    const int zhw = f.z_halfwidth();
+    size_t need = 0;
+    const int n = fewest_slabs(nz, zhw, 0, 0, budget, [&](const SlabPlan &pl) {
+      return filter_slab_bytes(pl, nx, ny, mask_host != nullptr, f);
+    }, &need);
+    if (n == 0) throw too_small(who, "the filter", need, budget);
+    const std::vector<SlabPlan> plans = make_plans(nz, n, zhw, 0, 0);
+    const size_t plane = (size_t)nx * (size_t)ny;
+    // dst_host == src_host: the raw planes [carry0, own0 of the next slab) that a later slab still reads.  Slab
+    // starts never decrease, so the planes below the next slab's start are dropped: at most halo + 7 planes.
+    const bool aliased = dst_host == src_host;
+    std::vector<float> carry;
+    int64_t carry0 = 0;
+    float A = 0.0f, B = 0.0f;
+    for (int r = 0; r < n; r++) {
+      FilterSlab s;
+      s.ctx = ctx;
+      s.plan = plans[(size_t)r];
+      try {
+        filter_slab(s, f, nx, ny, nz, src_host, mask_host, aliased ? carry.data() : nullptr, carry0);
+        if (aliased && r + 1 < n) {
+          const int64_t keep0 = plans[(size_t)r + 1].slab0, mid = std::max(keep0, s.plan.own0);
+          std::vector<float> next((size_t)(s.plan.own1 - keep0) * plane);
+          if (keep0 < s.plan.own0)
+            std::copy(carry.begin() + (keep0 - carry0) * plane, carry.begin() + (s.plan.own0 - carry0) * plane,
+                      next.begin());
+          std::copy(src_host + (size_t)mid * plane, src_host + (size_t)s.plan.own1 * plane,
+                    next.begin() + (mid - keep0) * plane);
+          carry.swap(next);
+          carry0 = keep0;
+        }
+        deliver_slab(s, nx, ny, dst_host);
+      } catch (const std::exception &ex) {
+        throw Error(who + ", slab " + std::to_string(r) + " of " + std::to_string(n) + ": " + ex.what());
+      }
+      if (r == 0) {   // the peak heights depend on the taps alone
+        A = s.A;
+        B = s.B;
+      }
+      s.out.free();
+      release_cache(ctx);
+    }
+    if (A_out) *A_out = A;
+    if (B_out) *B_out = B;
+    if (n_slabs_out) *n_slabs_out = n;
+    return 0;
+  } catch (const std::exception &ex) {
+    set_last_error(ex.what());
+    reset_after_failure(ctx);
+    return 1;
+  }
+}
+
 }  // namespace
+
+extern "C" int visfd_cuda_filter_multi(int ndev, const int *devices, int64_t nx, int64_t ny, int64_t nz,
+                                       const float *src_host, const float *mask_host, const visfd_filter_params *p,
+                                       float *dst_host, float *A_out, float *B_out, double *device_ms) {
+  return filter_multi("visfd_cuda_filter_multi", ndev, devices, nx, ny, nz, src_host, mask_host, p, dst_host, A_out,
+                      B_out, device_ms);
+}
+
+extern "C" int visfd_cuda_filter_stream(visfd_ctx *ctx, int64_t nx, int64_t ny, int64_t nz, const float *src_host,
+                                        const float *mask_host, const visfd_filter_params *p, int64_t device_bytes,
+                                        float *dst_host, float *A_out, float *B_out, int64_t *n_slabs_out) {
+  return filter_stream("visfd_cuda_filter_stream", ctx, nx, ny, nz, src_host, mask_host, p, device_bytes, dst_host,
+                       A_out, B_out, n_slabs_out);
+}
 
 extern "C" int visfd_cuda_membrane_multi(int ndev, const int *devices, int64_t nx, int64_t ny, int64_t nz,
                                          const float *src_host, const float *mask_host,

@@ -130,16 +130,38 @@ class DenseTensor {
 };
 
 // ---- separable filters (lib/visfd/filter3d.hpp) ---------------------------------------------
+// Every filter runs in Z-slabs within the GPU's free memory: one slab, and the one-shot call's bits, when the volume
+// fits; several slabs, and still the same bits, when it does not.  aaafDest may be aaafSource.
+inline void RunFilter(const int image_size[3], float const *const *const *aaafSource, float ***aaafDest,
+                   float const *const *const *aaafMask, const visfd_filter_params &p, float *pA, float *pB) {
+  Dense3<float, 1> s(image_size, aaafSource, false), m(image_size, aaafMask, false), d(image_size, aaafDest, true);
+  Check(visfd_cuda_filter_stream(Context(), image_size[0], image_size[1], image_size[2], s.data(), m.data(), &p, 0,
+                                 d.data(), pA, pB, nullptr));
+  d.commit();
+}
+inline visfd_filter_params DogParams(const float sigma_a[3], const float sigma_b[3], const int hw_a[3],
+                                     const int hw_b[3]) {
+  visfd_filter_params p{};
+  p.kind = VISFD_FILTER_DOG;
+  std::copy(sigma_a, sigma_a + 3, p.sigma_a);
+  std::copy(sigma_b, sigma_b + 3, p.sigma_b);
+  std::copy(hw_a, hw_a + 3, p.hw_a);
+  std::copy(hw_b, hw_b + 3, p.hw_b);
+  return p;
+}
+
 // ApplyGauss(sigma[3], truncate_halfwidth[3]): filter3d.hpp:1088-1124
 inline float ApplyGauss(const int image_size[3], float const *const *const *aaafSource, float ***aaafDest,
                         float const *const *const *aaafMask, float const sigma[3],
                         const int truncate_halfwidth[3], bool normalize = true,
                         std::ostream *pReportProgress = nullptr) {
-  Dense3<float, 1> s(image_size, aaafSource, false), m(image_size, aaafMask, false), d(image_size, aaafDest, true);
+  visfd_filter_params p{};
+  p.kind = VISFD_FILTER_GAUSS;
+  std::copy(sigma, sigma + 3, p.sigma_a);
+  std::copy(truncate_halfwidth, truncate_halfwidth + 3, p.hw_a);
+  p.normalize = normalize ? 1 : 0;
   float A = 0;
-  Check(visfd_cuda_apply_gauss(Context(), image_size[0], image_size[1], image_size[2], s.data(), d.data(),
-                               m.data(), sigma, truncate_halfwidth, normalize ? 1 : 0, &A));
-  d.commit();
+  RunFilter(image_size, aaafSource, aaafDest, aaafMask, p, &A, nullptr);
   if (pReportProgress) *pReportProgress << " -- Gaussian filter applied on the GPU --\n";
   return A;
 }
@@ -174,10 +196,8 @@ inline void ApplyDog(const int image_size[3], float const *const *const *aaafSou
                      const int truncate_halfwidth[3], float *pA = nullptr, float *pB = nullptr,
                      std::ostream *pReportProgress = nullptr) {
   (void)pReportProgress;
-  Dense3<float, 1> s(image_size, aaafSource, false), m(image_size, aaafMask, false), d(image_size, aaafDest, true);
-  Check(visfd_cuda_apply_dog(Context(), image_size[0], image_size[1], image_size[2], s.data(), d.data(), m.data(),
-                             sigma_a, sigma_b, truncate_halfwidth, pA, pB));
-  d.commit();
+  RunFilter(image_size, aaafSource, aaafDest, aaafMask,
+            DogParams(sigma_a, sigma_b, truncate_halfwidth, truncate_halfwidth), pA, pB);
 }
 
 // ApplyLog: filter3d.hpp:1430-1507
@@ -186,10 +206,12 @@ inline void ApplyLog(const int image_size[3], float const *const *const *aaafSou
                      float delta_sigma_over_sigma = 0.02, float truncate_ratio = 2.5, float *pA = nullptr,
                      float *pB = nullptr, std::ostream *pReportProgress = nullptr) {
   (void)pReportProgress;
-  Dense3<float, 1> s(image_size, aaafSource, false), m(image_size, aaafMask, false), d(image_size, aaafDest, true);
-  Check(visfd_cuda_apply_log(Context(), image_size[0], image_size[1], image_size[2], s.data(), d.data(), m.data(),
-                             sigma, delta_sigma_over_sigma, truncate_ratio, pA, pB));
-  d.commit();
+  visfd_filter_params p{};
+  p.kind = VISFD_FILTER_LOG;
+  std::copy(sigma, sigma + 3, p.sigma_a);
+  p.delta = delta_sigma_over_sigma;
+  p.truncate_ratio = truncate_ratio;
+  RunFilter(image_size, aaafSource, aaafDest, aaafMask, p, pA, pB);
 }
 
 
@@ -204,10 +226,7 @@ inline void ApplyDog(const int image_size[3], float const *const *const *aaafSou
     hwa[d] = visfd_cuda_gauss_halfwidth(sigma_a[d], filter_truncate_ratio, filter_truncate_threshold);
     hwb[d] = visfd_cuda_gauss_halfwidth(sigma_b[d], filter_truncate_ratio, filter_truncate_threshold);
   }
-  Dense3<float, 1> s(image_size, aaafSource, false), m(image_size, aaafMask, false), d(image_size, aaafDest, true);
-  Check(visfd_cuda_apply_dog2(Context(), image_size[0], image_size[1], image_size[2], s.data(), d.data(), m.data(),
-                              sigma_a, sigma_b, hwa, hwb, pA, pB));
-  d.commit();
+  RunFilter(image_size, aaafSource, aaafDest, aaafMask, DogParams(sigma_a, sigma_b, hwa, hwb), pA, pB);
 }
 inline void ApplyLog(const int image_size[3], float const *const *const *aaafSource, float ***aaafDest,
                      float const *const *const *aaafMask, const float sigma[3], float delta_sigma_over_sigma,
