@@ -81,8 +81,8 @@ int64_t visfd_cuda_peak_reserved_bytes(visfd_ctx *ctx);
 void visfd_cuda_reset_peak_reserved_bytes(visfd_ctx *ctx);
 /* Device milliseconds spent in a named stage since the last visfd_cuda_reset_stage_ms,
  * measured with CUDA events on the context's stream around the stage's kernels:
- * "gauss", "ridge", "select", "compact", "tv", "threshold", "blob_scan", "h2d", "d2h".
- * Returns -1 for a stage that has not run. */
+ * "gauss", "ridge", "select", "compact", "tv", "threshold", "blob_scan", "h2d", "d2h"; and "flood", the HOST
+ * milliseconds of LabelConnected's ordered flood.  Returns -1 for a stage that has not run. */
 double visfd_cuda_stage_ms(visfd_ctx *ctx, const char *stage);
 void visfd_cuda_reset_stage_ms(visfd_ctx *ctx);
 
@@ -348,6 +348,54 @@ int visfd_cuda_label_connected(visfd_ctx *ctx, int64_t nx, int64_t ny, int64_t n
                                float threshold_vector_saliency, float threshold_vector_neighbor,
                                float threshold_tensor_saliency, float threshold_tensor_neighbor, int64_t *labels,
                                int64_t *n_clusters, float *cluster_maxima, int64_t maxima_capacity, int64_t *n_maxima);
+
+/* ---- the membrane pipeline and -connect over Z-slabs, one call --------------------------------------------------- */
+/* The thresholds of -connect: threshold_saliency is `-connect T`; the four cosines are those -connect-angle sets
+ * (settings.cpp:3075-3086).  With unsigned dot products a negative vector threshold means "do not test", as in
+ * visfd_cuda_label_connected. */
+typedef struct visfd_connect_params {
+  float threshold_saliency;
+  float threshold_vector_saliency;
+  float threshold_vector_neighbor;
+  float threshold_tensor_saliency;
+  float threshold_tensor_neighbor;
+  int consider_dot_product_sign;
+} visfd_connect_params;
+
+/* HandleTV with `-connect` (handlers.cpp:1932-1970) on volumes of any size: the membrane pipeline of
+ * visfd_cuda_membrane_multi_background / visfd_cuda_membrane_stream_background (background_sigma 0: none), then
+ * LabelConnected on its result and vote tensor, with HOST arrays only.  The vote tensor never leaves the device: each
+ * slab turns the tensor of its own planes into the first eigenvectors and the 16 flag bits of LabelConnected where it
+ * votes, and sends home 2 B of flags per voxel (and the direction if direction_host is given) instead of 24 B of
+ * tensor.  The two planes next to each internal slab boundary take their flags from a small seam step over the four
+ * planes around it (score from out_host, the two tensor planes kept from each side).  The ordered flood then runs on
+ * the calling thread over the flags of the whole image.
+ * The result is bit-identical, for any number of slabs, to
+ *   visfd_cuda_membrane_background(p, background_sigma, normalize_near_boundaries) -> out, *threshold_out, tensor;
+ *   visfd_cuda_label_connected(out, mask, tensor, direction, direction_from_tensor = 1, p->eival_order, ...)
+ * -> labels, *n_clusters, *n_maxima, the first min(n_clusters, maxima_capacity) rows of cluster_maxima (3 floats
+ * each; may be NULL) and direction.  direction_host (N*3 floats) may be NULL: the labels are the same and no direction
+ * is downloaded.  p->tv_sigma <= 0 is refused (-connect clusters the vote tensor).  n_clusters and n_maxima may be
+ * NULL.  The host needs N*2 B for the flags besides the caller's arrays.
+ * multi: one slab per entry of devices[], sharing the contexts of visfd_cuda_membrane_multi and its one call at a time;
+ * device_ms as there.  stream: slabs one after another on ctx within device_bytes (0: the free memory at entry less a
+ * margin); a vote slab also holds its own planes' tensor (24 B), direction (12 B) and flags (2 B) per voxel, so the
+ * same budget may take more slabs than visfd_cuda_membrane_stream; it fails naming the bytes needed when slabs of 8
+ * planes do not fit.  *n_slabs_out (may be NULL): slabs of the vote pass. */
+int visfd_cuda_membrane_connect_multi(int ndev, const int *devices, int64_t nx, int64_t ny, int64_t nz,
+                                      const float *src_host, const float *mask_host, const visfd_membrane_params *p,
+                                      float background_sigma, int normalize_near_boundaries,
+                                      const visfd_connect_params *c, float *out_host, float *threshold_out,
+                                      int64_t *labels_host, float *direction_host, int64_t *n_clusters,
+                                      float *cluster_maxima, int64_t maxima_capacity, int64_t *n_maxima,
+                                      double *device_ms);
+int visfd_cuda_membrane_connect_stream(visfd_ctx *ctx, int64_t nx, int64_t ny, int64_t nz, const float *src_host,
+                                       const float *mask_host, const visfd_membrane_params *p, float background_sigma,
+                                       int normalize_near_boundaries, const visfd_connect_params *c,
+                                       int64_t device_bytes, float *out_host, float *threshold_out,
+                                       int64_t *labels_host, float *direction_host, int64_t *n_clusters,
+                                       float *cluster_maxima, int64_t maxima_capacity, int64_t *n_maxima,
+                                       int64_t *n_slabs_out);
 
 /* ---- oriented point cloud of a detected surface ---------------------------------------
  * The block of HandleTV that runs when `-normals-file` is given (bin/filter_mrc/handlers.cpp:2039-2309; the

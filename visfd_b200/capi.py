@@ -207,6 +207,61 @@ def membrane_multi(devices, src, sigma, truncate_ratio, order, cut, cut_is_fract
     return dict(out=res, threshold=thr.value, device_ms=list(ms))
 
 
+class ConnectParams(C.Structure):
+    """visfd_connect_params: the thresholds of `-connect T -connect-angle A`."""
+    _fields_ = [("threshold_saliency", _f), ("threshold_vector_saliency", _f), ("threshold_vector_neighbor", _f),
+                ("threshold_tensor_saliency", _f), ("threshold_tensor_neighbor", _f),
+                ("consider_dot_product_sign", _i)]
+
+
+_CONNECT_MAXIMA = 1 << 16   # rows of cluster maxima returned, as Context.label_connected
+
+
+def _connect_args(who, src, mask, threshold_saliency, angle_deg, thresholds, consider_dot_product_sign,
+                  want_direction):
+    """numpy host arrays and outputs for the membrane + -connect slab drivers (which refuse device memory)
+    -> (src, mask, out, labels, direction or None, ConnectParams, maxima buffer)"""
+    if _is_torch(src) or _is_torch(mask):
+        raise VisfdCudaError(f"{who} takes numpy (host) arrays")
+    src = np.ascontiguousarray(src, np.float32)
+    mask = None if mask is None else np.ascontiguousarray(mask, np.float32)
+    c = float(np.float32(np.cos(angle_deg * np.pi / 180.0)))   # as Context.label_connected
+    tvs, tvn, tts, ttn = thresholds if thresholds is not None else (c, c, c, c)
+    params = ConnectParams(threshold_saliency, tvs, tvn, tts, ttn, int(consider_dot_product_sign))
+    direction = np.zeros(src.shape + (3,), np.float32) if want_direction else None
+    return (src, mask, np.empty(src.shape, np.float32), np.zeros(src.shape, np.int64), direction, params,
+            np.zeros((_CONNECT_MAXIMA, 3), np.float32))
+
+
+def membrane_connect_multi(devices, src, sigma, truncate_ratio, order, cut, cut_is_fraction, tv_sigma, tv_exponent,
+                           tv_cutoff_ratio, threshold_saliency, angle_deg=15.0, mask=None, want_direction=False,
+                           consider_dot_product_sign=False, thresholds=None, background_sigma=0.0, normalize=True,
+                           lib=None):
+    """visfd_cuda_membrane_connect_multi: membrane_multi followed by `-connect` (LabelConnected on the result and the
+    vote tensor, which stays on the GPUs), one Z-slab per entry of devices (a device may appear more than once).
+    numpy (host) arrays only.  -> dict(out, threshold, labels, n_clusters, n_maxima, maxima, direction, device_ms),
+    equal to Context.membrane(..., want_tensor=True) followed by Context.label_connected on its out and tensor."""
+    lib = lib or load_library()
+    who = "visfd_cuda_membrane_connect_multi"
+    src, mask, res, labels, direction, cp, maxima = _connect_args(who, src, mask, threshold_saliency, angle_deg,
+                                                                  thresholds, consider_dot_product_sign,
+                                                                  want_direction)
+    p = MembraneParams(sigma, truncate_ratio, order, cut, int(cut_is_fraction), tv_sigma, tv_exponent, tv_cutoff_ratio)
+    devs = (C.c_int * len(devices))(*[int(d) for d in devices])
+    ms = (C.c_double * len(devices))()
+    thr, ncl, nmax = _f(), _i64(), _i64()
+    nz, ny, nx = src.shape
+    rc = lib.visfd_cuda_membrane_connect_multi(_i(len(devices)), devs, _i64(nx), _i64(ny), _i64(nz), _ptr(src),
+                                               _ptr(mask), C.byref(p), _f(background_sigma), _i(int(normalize)),
+                                               C.byref(cp), _ptr(res), C.byref(thr), _p(labels.ctypes.data),
+                                               _ptr(direction), C.byref(ncl), _ptr(maxima), _i64(len(maxima)),
+                                               C.byref(nmax), ms)
+    if rc != 0:
+        raise VisfdCudaError(lib.visfd_cuda_last_error().decode())
+    return dict(out=res, threshold=thr.value, labels=labels, n_clusters=ncl.value, n_maxima=nmax.value,
+                maxima=maxima[:min(ncl.value, len(maxima))].copy(), direction=direction, device_ms=list(ms))
+
+
 def _blob_buffers(capacity):
     return [np.zeros((capacity, 3), np.float32), np.zeros(capacity, np.float32), np.zeros(capacity, np.float32),
             np.zeros((capacity, 3), np.float32), np.zeros(capacity, np.float32), np.zeros(capacity, np.float32)]
@@ -622,6 +677,29 @@ class Context:
                                                          C.byref(p), _i64(int(device_bytes)), _ptr(res), C.byref(thr),
                                                          C.byref(n_slabs)))
         return dict(out=res, threshold=thr.value, n_slabs=n_slabs.value)
+
+    def membrane_connect_stream(self, src, sigma, truncate_ratio, order, cut, cut_is_fraction, tv_sigma, tv_exponent,
+                                tv_cutoff_ratio, threshold_saliency, angle_deg=15.0, mask=None, want_direction=False,
+                                consider_dot_product_sign=False, thresholds=None, background_sigma=0.0,
+                                normalize=True, device_bytes=0):
+        """visfd_cuda_membrane_connect_stream: membrane_stream followed by `-connect` (LabelConnected on the result
+        and the vote tensor, which never leaves the GPU), slab after slab within device_bytes (0: the free memory at
+        entry, less a margin).  numpy (host) arrays only.  -> dict(out, threshold, labels, n_clusters, n_maxima,
+        maxima, direction, n_slabs), equal to membrane(..., want_tensor=True) followed by label_connected."""
+        who = "visfd_cuda_membrane_connect_stream"
+        src, mask, res, labels, direction, cp, maxima = _connect_args(who, src, mask, threshold_saliency, angle_deg,
+                                                                      thresholds, consider_dot_product_sign,
+                                                                      want_direction)
+        p = MembraneParams(sigma, truncate_ratio, order, cut, int(cut_is_fraction), tv_sigma, tv_exponent,
+                           tv_cutoff_ratio)
+        thr, ncl, nmax, n_slabs = _f(), _i64(), _i64(), _i64()
+        self._ck(self.lib.visfd_cuda_membrane_connect_stream(
+            self.h, *self._dims(src.shape), _ptr(src), _ptr(mask), C.byref(p), _f(background_sigma),
+            _i(int(normalize)), C.byref(cp), _i64(int(device_bytes)), _ptr(res), C.byref(thr),
+            _p(labels.ctypes.data), _ptr(direction), C.byref(ncl), _ptr(maxima), _i64(len(maxima)), C.byref(nmax),
+            C.byref(n_slabs)))
+        return dict(out=res, threshold=thr.value, labels=labels, n_clusters=ncl.value, n_maxima=nmax.value,
+                    maxima=maxima[:min(ncl.value, len(maxima))].copy(), direction=direction, n_slabs=n_slabs.value)
 
     def filter_stream(self, src, params, mask=None, device_bytes=0, out=None):
         """visfd_cuda_filter_stream: ApplyGauss / ApplyDog / ApplyLog (params: FilterParams) on this context's GPU in

@@ -34,6 +34,7 @@
 // mask keep the internal marker n_maxima + 1 (connect.hpp:1398-1401 skips them).
 // Not offered: must-link constraints (connect.hpp:830-1040), sorting by value, voxel weights.
 #include <algorithm>
+#include <chrono>
 #include <cmath>
 #include <queue>
 
@@ -57,9 +58,11 @@ enum : uint16_t {
 __constant__ int c_nbr[6][3] = {{0, 0, -1}, {0, -1, 0}, {-1, 0, 0}, {1, 0, 0}, {0, 1, 0}, {0, 0, 1}};
 static const int h_nbr[6][3] = {{0, 0, -1}, {0, -1, 0}, {-1, 0, 0}, {1, 0, 0}, {0, 1, 0}, {0, 0, 1}};
 
+// The arrays hold nz planes starting at global plane z_offset of a volume of nz_global planes: the stencil clamp and
+// the neighbour bounds are those of the whole volume, so a slab computes the flags of the undivided image.
 struct ConnArgs {
   const float *sal, *mask, *tensor, *dir;
-  int nx, ny, nz;
+  int nx, ny, nz, z_offset, nz_global;
   float thr_sal, thr_vs, thr_vn, thr_ts, thr_tn;
   int order, signed_dot;
   uint16_t *state;
@@ -131,7 +134,7 @@ __global__ void __launch_bounds__(256) connect_predicates_kernel(ConnArgs g, int
     // ---- saliency vs tensor / vector at this voxel (connect.hpp:462-578) ----
     bool discard = false;
     if (g.tensor || g.dir) {
-      Stencil sten = make_stencil(g.sal, g.nx, g.ny, 0, g.nz, ix, iy, iz);
+      Stencil sten = make_stencil(g.sal, g.nx, g.ny, g.z_offset, g.nz_global, ix, iy, iz);
       float h[6];
       fd_hessian(sten, 1.0f, h);
       // tensor positive definite near the target and clusters start at maxima: the Hessian changes sign (:487-492)
@@ -163,7 +166,7 @@ __global__ void __launch_bounds__(256) connect_predicates_kernel(ConnArgs g, int
 #pragma unroll
   for (int k = 0; k < 6; k++) {
     const int jx = ix + c_nbr[k][0], jy = iy + c_nbr[k][1], jz = iz + c_nbr[k][2];
-    if (jx < 0 || jx >= g.nx || jy < 0 || jy >= g.ny || jz < 0 || jz >= g.nz) continue;
+    if (jx < 0 || jx >= g.nx || jy < 0 || jy >= g.ny || jz + g.z_offset < 0 || jz + g.z_offset >= g.nz_global) continue;
     const i64 j = jz * sz + jy * sy + jx;
     if (g.mask && __ldg(g.mask + j) == 0.0f) continue;
     const float sj = __ldg(g.sal + j);
@@ -184,21 +187,35 @@ __global__ void __launch_bounds__(256) connect_predicates_kernel(ConnArgs g, int
   g.state[i] = st;
 }
 
-void connect_predicates_device(visfd_ctx *ctx, i64 nx, i64 ny, i64 nz, const float *sal, const float *mask,
-                               const float *tensor, const float *dir, int eival_order, int signed_dot, float thr_sal,
-                               float thr_vs, float thr_vn, float thr_ts, float thr_tn, uint16_t *state) {
-  VREQUIRE(nx >= 3 && ny >= 3 && nz >= 3, "LabelConnected needs an image at least 3 voxels wide (finite-difference Hessian)");
+void connect_predicates_device(visfd_ctx *ctx, i64 nx, i64 ny, i64 nz_local, i64 z_offset, i64 nz_global, i64 z0,
+                               i64 z1, const float *sal, const float *mask, const float *tensor, const float *dir,
+                               int eival_order, int signed_dot, float thr_sal, float thr_vs, float thr_vn, float thr_ts,
+                               float thr_tn, uint16_t *state) {
+  VREQUIRE(nx >= 3 && ny >= 3 && nz_global >= 3, "LabelConnected needs an image at least 3 voxels wide (finite-difference Hessian)");
   VREQUIRE(!tensor || dir, "tensors without directions");
-  ConnArgs g{sal, mask, tensor, dir, (int)nx, (int)ny, (int)nz, thr_sal, thr_vs, thr_vn, thr_ts, thr_tn,
-             eival_order, signed_dot, state};
+  // the clamped stencil and the neighbours of planes [z0, z1) must lie in the slab
+  const i64 lo = std::max<i64>(0, std::min(z_offset + z0 - 1, nz_global - 3));
+  const i64 hi = std::min(nz_global, std::max<i64>(z_offset + z1 + 1, 3));
+  VREQUIRE(0 <= z0 && z0 <= z1 && z1 <= nz_local && z_offset >= 0 && z_offset + nz_local <= nz_global &&
+               (z1 == z0 || (lo >= z_offset && hi <= z_offset + nz_local)),
+           "connect: the slab lacks the planes next to the planes it computes");
+  ConnArgs g{sal, mask, tensor, dir, (int)nx, (int)ny, (int)nz_local, (int)z_offset, (int)nz_global, thr_sal, thr_vs,
+             thr_vn, thr_ts, thr_tn, eival_order, signed_dot, state};
   StageTimer t(ctx, "connect_predicates");
   dim3 block(64, 4, 1);
-  for (i64 z0 = 0; z0 < nz; z0 += 65535) {
-    dim3 grid(div_up(nx, 64), div_up(ny, 4), (unsigned)std::min<i64>(65535, nz - z0));
-    connect_predicates_kernel<<<grid, block, 0, ctx->stream>>>(g, (int)z0);
+  for (i64 zc = z0; zc < z1; zc += 65535) {
+    dim3 grid(div_up(nx, 64), div_up(ny, 4), (unsigned)std::min<i64>(65535, z1 - zc));
+    connect_predicates_kernel<<<grid, block, 0, ctx->stream>>>(g, (int)zc);
     VCK(cudaGetLastError());
     ctx->count_launch();
   }
+}
+
+void first_eigenvectors_device(visfd_ctx *ctx, i64 n, const float *tensor, const float *mask, int eival_order,
+                               float *dir) {
+  // handlers.cpp:1933-1950: the first eigenvector of every vote tensor (masked voxels: left as they are -> zero here)
+  VCK(cudaMemsetAsync(dir, 0, 3 * (size_t)n * sizeof(float), ctx->stream));
+  tensor_score_device(ctx, n, tensor, mask, eival_order, 0, 1, nullptr, nullptr, dir);
 }
 
 // ---------------------------------------------------------------------------------------------------
@@ -463,14 +480,10 @@ extern "C" int visfd_cuda_label_connected(visfd_ctx *ctx, int64_t nx, int64_t ny
       dir_tmp.reset(ctx, 3 * N);
       dir_dev = dir_tmp.get();
     }
-    if (compute_dir) {
-      // handlers.cpp:1933-1950: the first eigenvector of every vote tensor (masked voxels: left as they are -> zero here)
-      VCK(cudaMemsetAsync(dir_dev, 0, 3 * N * sizeof(float), ctx->stream));
-      tensor_score_device(ctx, (i64)N, t.get(), m.get(), eival_order, 0, 1, nullptr, nullptr, dir_dev);
-    }
+    if (compute_dir) first_eigenvectors_device(ctx, (i64)N, t.get(), m.get(), eival_order, dir_dev);
     Scratch<uint16_t> state(ctx, N);
     // the Hessian of the saliency is diagonalised with DECREASING eigenvalues (clusters start at maxima, connect.hpp:173-177)
-    connect_predicates_device(ctx, nx, ny, nz, s.get(), m.get(), t.get(), dir_dev, 1, consider_dot_product_sign != 0,
+    connect_predicates_device(ctx, nx, ny, nz, 0, nz, 0, nz, s.get(), m.get(), t.get(), dir_dev, 1, consider_dot_product_sign != 0,
                               threshold_saliency, threshold_vector_saliency, threshold_vector_neighbor,
                               threshold_tensor_saliency, threshold_tensor_neighbor, state.get());
     // ---- to the host: flags, saliency (if it was on the device), directions (if they are wanted back) ----
@@ -504,8 +517,10 @@ extern "C" int visfd_cuda_label_connected(visfd_ctx *ctx, int64_t nx, int64_t ny
     }
     std::vector<float> maxima;
     i64 n_max = 0;
+    const auto t0 = std::chrono::steady_clock::now();
     const i64 nc = connect_flood_host(nx, ny, nz, h_sal, h_state.data(), h_dir, consider_dot_product_sign == 0,
                                       threshold_saliency, h_lab, &maxima, &n_max);
+    const double flood_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
     if (h_lab != labels) VCK(cudaMemcpyAsync(labels, h_lab, N * sizeof(int64_t), cudaMemcpyHostToDevice, ctx->stream));
     if (direction && !host)
       VCK(cudaMemcpyAsync(direction, h_dir, 3 * N * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
@@ -515,6 +530,7 @@ extern "C" int visfd_cuda_label_connected(visfd_ctx *ctx, int64_t nx, int64_t ny
       memcpy(cluster_maxima, maxima.data(), sizeof(float) * 3 * (size_t)std::min<i64>(nc, maxima_capacity));
     VCK(cudaStreamSynchronize(ctx->stream));
     resolve_stage_times(ctx);
+    ctx->stage_ms["flood"] += flood_ms;   // host time of the ordered flood
     return 0;
   } catch (const std::exception &ex) {
     set_last_error(ex.what());

@@ -95,6 +95,21 @@ bool tv_device(visfd_ctx *ctx, i64 nx, i64 ny, i64 nz_local, i64 z_offset, i64 n
 size_t tv_workspace_bytes(i64 nx, i64 ny, i64 nz_local, i64 own_planes, uint64_t n_voters);
 int tv_halfwidth(float sigma, float cutoff_ratio);
 
+// ---- connect.cu -------------------------------------------------------------------
+// LabelConnected's 16 flag bits for planes [z0, z1) of a slab of nz_local planes that starts at global plane z_offset
+// of nz_global (the whole image: 0, nz, 0, nz).  The slab must hold the planes the clamped stencil and the neighbour
+// tests of those planes read; every array is indexed like the slab.
+void connect_predicates_device(visfd_ctx *ctx, i64 nx, i64 ny, i64 nz_local, i64 z_offset, i64 nz_global, i64 z0,
+                               i64 z1, const float *sal, const float *mask, const float *tensor, const float *dir,
+                               int eival_order, int signed_dot, float thr_sal, float thr_vs, float thr_vn, float thr_ts,
+                               float thr_tn, uint16_t *state);
+// dir (n*3) = the first eigenvector of each tensor, zero where the mask is 0 (handlers.cpp:1933-1950).
+void first_eigenvectors_device(visfd_ctx *ctx, i64 n, const float *tensor, const float *mask, int eival_order,
+                               float *dir);
+// The ordered flood over the flags of the whole image (host arrays) -> the number of clusters.
+i64 connect_flood_host(i64 nx, i64 ny, i64 nz, const float *sal, const uint16_t *state, float *dir, bool unsigned_dot,
+                       float thr_sal, i64 *labels, std::vector<float> *cluster_maxima, i64 *n_maxima_out);
+
 // ---- api.cu -----------------------------------------------------------------------
 // visfd_cuda_vote_slab_host without its API frame (the slab drivers of multi.cu).  peak (optional, nz_local*ny*nx
 // floats like saliency): the voted score is multiplied by the peak height (tv_device); without voting the saliency

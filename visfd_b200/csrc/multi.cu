@@ -9,6 +9,8 @@
 // source - Gauss(source, background_sigma), as visfd_cuda_membrane_background does on one GPU.
 // visfd_cuda_blob_dog_multi / visfd_cuda_blob_dog_stream do the same for BlobDog, in one pass (see below), and
 // visfd_cuda_filter_multi / visfd_cuda_filter_stream for ApplyGauss, ApplyDog and ApplyLog.
+// visfd_cuda_membrane_connect_multi / visfd_cuda_membrane_connect_stream add `-connect` (LabelConnected) to the
+// membrane drivers, with the vote tensor kept on the device (see "-connect over Z-slabs" below).
 //
 // The volume is cut into Z-slabs exactly as visfd_b200/slab.py does for the process-per-GPU driver (rank boundaries
 // on multiples of 8 planes, slabs widened by a halo of RAW SOURCE planes, halo = tv_halfwidth + 1 + gauss_halfwidth,
@@ -31,6 +33,8 @@
 // before the step of the pass, since nothing stays on the device from one slab to the next (Gaussian + ridge are
 // under 1 % of a C4 step).  Its slab count is the smallest whose slabs fit the budget by slab_bytes.
 #include <algorithm>
+#include <chrono>
+#include <memory>
 #include <mutex>
 #include <thread>
 
@@ -129,6 +133,7 @@ struct Slab {
   Scratch<float> peak;   // with the background: the peak height of every plane of the slab, until the vote ends
   DeviceClock clock;
   uint64_t hist[HIST_BINS];
+  std::vector<float> tensor_lo, tensor_hi;   // -connect: the vote tensor of the first / last two own planes (seams)
 };
 
 void make_slabs(std::vector<Slab> &slabs, const std::vector<SlabPlan> &plans, visfd_ctx *ctx) {
@@ -241,8 +246,11 @@ void for_each_slab(const char *name, std::vector<S> &slabs, const Fn &fn) {
 // With the background both steps also hold the slab's whole peak height.  In step (1) the background Gaussian runs
 // first, beside the same volumes; its scratch goes back to the pool, where the smoothing's scratch, which has at least
 // as many volumes, takes them again, so only its block of taps may stay cached next to the smoothing's.
+// With -connect (vote_and_flag) the vote also holds the own planes' tensor; then everything but the mask, the output
+// and the tensor goes back to the device, and the flags step adds the own planes' directions and flags.  A seam step
+// holds the same blocks for 4 planes: never more than a slab of at least 8 own planes.
 size_t slab_bytes(const SlabPlan &pl, int64_t nx, int64_t ny, bool masked, const visfd_membrane_params *p,
-                  int gauss_hw, const Background &bg, bool vote, uint64_t voters) {
+                  int gauss_hw, const Background &bg, bool vote, uint64_t voters, bool connect) {
   const size_t plane = (size_t)nx * (size_t)ny;
   const int64_t slab = pl.slab1 - pl.slab0;
   const size_t vol = visfd_ctx::block_bytes((size_t)slab * plane * sizeof(float));
@@ -251,8 +259,10 @@ size_t slab_bytes(const SlabPlan &pl, int64_t nx, int64_t ny, bool masked, const
   const size_t bg_taps = bg.on() ? separable_workspace_bytes(nx, ny, slab, hw_bg, false, false) - vol : 0;
   const size_t ridge = (masked ? 4 : 3) * vol + peak + separable_workspace_bytes(nx, ny, slab, hw, masked, true) + bg_taps;
   if (!vote) return ridge + visfd_ctx::block_bytes(HIST_BINS * sizeof(uint64_t));
-  size_t voting = (masked ? 3 : 2) * vol + peak +
-                  visfd_ctx::block_bytes((size_t)(pl.own1 - pl.own0) * plane * sizeof(float));
+  const size_t own = (size_t)(pl.own1 - pl.own0) * plane;
+  const size_t out = visfd_ctx::block_bytes(own * sizeof(float));
+  const size_t tensor = connect ? visfd_ctx::block_bytes(own * 6 * sizeof(float)) : 0;
+  size_t voting = (masked ? 3 : 2) * vol + peak + out + tensor;
   if (p->tv_sigma > 0.0f) {
     // visfd_cuda_vote_slab_host widens the voter planes down to a global multiple of 8: up to 7 more planes, whose
     // saliency may be incomplete, so they may add up to 7 planes of voters to the count of the whole volume
@@ -261,7 +271,10 @@ size_t slab_bytes(const SlabPlan &pl, int64_t nx, int64_t ny, bool masked, const
     const uint64_t n = voters < vox ? std::min(vox, voters + 7 * (uint64_t)plane) : vox;
     voting += tv_workspace_bytes(nx, ny, vplanes, pl.own1 - pl.own0, n);
   }
-  return std::max(ridge, voting);
+  const size_t flags = connect ? (masked ? vol : 0) + out + tensor + visfd_ctx::block_bytes(own * 3 * sizeof(float)) +
+                                     visfd_ctx::block_bytes(own * sizeof(uint16_t))
+                               : 0;
+  return std::max({ridge, voting, flags});
 }
 
 // The ridge step's scratch and every block a finished slab leaves behind go back to the device, so that the next
@@ -320,10 +333,162 @@ Background background(const std::string &who, const visfd_membrane_params *p, fl
   return bg;
 }
 
+// ---- -connect over Z-slabs -------------------------------------------------------------------------------------
+// LabelConnected's per-voxel predicates read the post-vote score, the vote tensor, its first eigenvector and the mask
+// within +-1 plane only (2 planes at the global ends, where the stencil is clamped), and the host flood reads only the
+// 16-bit flags, the score and the directions.  So a slab computes, right after its vote, the flags of every own plane
+// whose neighbours it holds, and sends 2 B per voxel home instead of the 24 B of the tensor.  Slab boundaries lie on
+// multiples of 8 planes with at least 8 own planes per slab, so the two planes next to an internal boundary b are
+// inner planes of the volume: a seam step computes their flags from planes b-2 .. b+1 (score and mask from the
+// caller's arrays, the two tensor planes each side kept on the host by the slabs).  Receivers are not voted again:
+// a receiver is bit-exact only inside whole 4-plane patches of its slab.
+
+// The arguments and outputs of a connect call; flags: the whole image's, filled by the slabs and the seams.
+struct Connect {
+  visfd_connect_params c;   // thresholds as LabelConnected takes them (negative vector cosines clamped)
+  int64_t *labels = nullptr;
+  float *direction = nullptr;
+  int64_t *n_clusters = nullptr, *n_maxima = nullptr;
+  float *maxima = nullptr;
+  int64_t capacity = 0;
+  std::unique_ptr<uint16_t[]> flags;
+};
+
+Connect connect_args(const std::string &who, int64_t nx, int64_t ny, int64_t nz, const float *src_host,
+                     const visfd_membrane_params *p, float background_sigma, const visfd_connect_params *c,
+                     float *out_host, int64_t *labels, float *direction, int64_t capacity) {
+  VREQUIRE(src_host && p && c && out_host && labels && capacity >= 0, who + ": bad arguments");
+  VREQUIRE(p->tv_sigma > 0.0f, who + ": -connect clusters the vote tensor: tv_sigma must be positive");
+  VREQUIRE(background_sigma >= 0.0f, who + ": negative background width");   // (NaN fails too)
+  VREQUIRE(nx >= 3 && ny >= 3 && nz >= 3, who + ": LabelConnected needs an image at least 3 voxels wide");
+  VREQUIRE(nx < (1LL << 31) && ny < (1LL << 31) && nz < (1LL << 31), who + ": bad image dimensions");
+  VREQUIRE(!is_device_pointer(labels) && !is_device_pointer(direction), who + " takes HOST arrays");
+  Connect cn;
+  cn.c = *c;
+  if (!c->consider_dot_product_sign) {   // connect.hpp:190-205, as visfd_cuda_label_connected
+    cn.c.threshold_vector_saliency = std::max(cn.c.threshold_vector_saliency, 0.0f);
+    cn.c.threshold_vector_neighbor = std::max(cn.c.threshold_vector_neighbor, 0.0f);
+  }
+  cn.labels = labels;
+  cn.direction = direction;
+  cn.capacity = capacity;
+  return cn;
+}
+
+// Flags of `planes` planes [z0, z1) of arrays that start at global plane z_offset, into cn.flags.
+void flag_planes(visfd_ctx *ctx, int64_t nx, int64_t ny, int64_t nz, int64_t planes, int64_t z_offset, int64_t z0,
+                 int64_t z1, const float *score, const float *mask, const float *tensor,
+                 const visfd_membrane_params *p, Connect &cn, float *direction_host) {
+  const size_t plane = (size_t)nx * (size_t)ny, n = (size_t)planes * plane;
+  Scratch<float> dir(ctx, 3 * n);
+  Scratch<uint16_t> state(ctx, n);
+  first_eigenvectors_device(ctx, (i64)n, tensor, mask, p->eival_order, dir.get());
+  const visfd_connect_params &c = cn.c;
+  // the Hessian of the score is diagonalised with DECREASING eigenvalues, as visfd_cuda_label_connected does
+  connect_predicates_device(ctx, nx, ny, planes, z_offset, nz, z0, z1, score, mask, tensor, dir.get(), 1,
+                            c.consider_dot_product_sign != 0, c.threshold_saliency, c.threshold_vector_saliency,
+                            c.threshold_vector_neighbor, c.threshold_tensor_saliency, c.threshold_tensor_neighbor,
+                            state.get());
+  {
+    StageTimer t(ctx, "d2h");
+    VCK(cudaMemcpyAsync(cn.flags.get() + (size_t)(z_offset + z0) * plane, state.get() + (size_t)z0 * plane,
+                        (size_t)(z1 - z0) * plane * sizeof(uint16_t), cudaMemcpyDeviceToHost, ctx->stream));
+    if (direction_host)
+      VCK(cudaMemcpyAsync(direction_host, dir.get(), 3 * n * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
+  }
+  VCK(cudaStreamSynchronize(ctx->stream));
+}
+
+// Step (3) with -connect: voting on the own planes, delivered into the caller's array, with their tensor kept on the
+// device; then the flags of the own planes whose neighbours the slab holds, the directions, and the tensor planes the
+// seams need.
+void vote_and_flag(Slab &s, int64_t nx, int64_t ny, int64_t nz, float threshold, const visfd_membrane_params *p,
+                   float *out_host, Connect &cn) {
+  const SlabPlan &pl = s.plan;
+  const size_t plane = (size_t)nx * (size_t)ny;
+  const int64_t own = pl.own1 - pl.own0;
+  Scratch<float> out(s.ctx, (size_t)own * plane), tensor(s.ctx, (size_t)own * plane * 6);
+  vote_slab_device(s.ctx, nx, ny, pl.slab1 - pl.slab0, pl.slab0, nz, pl.own0 - pl.slab0, pl.own1 - pl.slab0,
+                   pl.vote0 - pl.slab0, pl.vote1 - pl.slab0, s.saliency.get(), s.smoothed.get(), s.mask.get(),
+                   threshold, p, out.get(), tensor.get(), out_host + (size_t)pl.own0 * plane, s.peak.get());
+  // the voting workspace and the volumes only the vote read go back to the device
+  s.smoothed.free();
+  s.saliency.free();
+  s.peak.free();
+  release_cache(s.ctx);
+  const float *mask = s.mask.get() ? s.mask.get() + (size_t)(pl.own0 - pl.slab0) * plane : nullptr;
+  flag_planes(s.ctx, nx, ny, nz, own, pl.own0, pl.own0 > 0 ? 1 : 0, pl.own1 < nz ? own - 1 : own, out.get(), mask,
+              tensor.get(), p, cn, cn.direction ? cn.direction + 3 * (size_t)pl.own0 * plane : nullptr);
+  const size_t two = 2 * plane * 6;
+  if (pl.own0 > 0) {
+    s.tensor_lo.resize(two);
+    VCK(cudaMemcpyAsync(s.tensor_lo.data(), tensor.get(), two * sizeof(float), cudaMemcpyDeviceToHost, s.ctx->stream));
+  }
+  if (pl.own1 < nz) {
+    s.tensor_hi.resize(two);
+    VCK(cudaMemcpyAsync(s.tensor_hi.data(), tensor.get() + (size_t)(own - 2) * plane * 6, two * sizeof(float),
+                        cudaMemcpyDeviceToHost, s.ctx->stream));
+  }
+  VCK(cudaStreamSynchronize(s.ctx->stream));
+  resolve_stage_times(s.ctx);
+}
+
+// The boundary between two slabs: planes b-2, b-1 belong to the slab below, b, b+1 to the one above.
+struct Seam {
+  visfd_ctx *ctx = nullptr;
+  int64_t b = 0;
+  const float *tensor_below = nullptr, *tensor_above = nullptr;   // two planes each
+};
+
+std::vector<Seam> seams_of(const std::vector<Slab> &slabs) {
+  std::vector<Seam> seams(slabs.size() - 1);
+  for (size_t r = 0; r + 1 < slabs.size(); r++)
+    seams[r] = {slabs[r].ctx, slabs[r].plan.own1, slabs[r].tensor_hi.data(), slabs[r + 1].tensor_lo.data()};
+  return seams;
+}
+
+// The flags of planes b-1 and b, from the result already in the caller's array.
+void seam_flags(const Seam &sm, int64_t nx, int64_t ny, int64_t nz, const float *out_host, const float *mask_host,
+                const visfd_membrane_params *p, Connect &cn) {
+  const size_t plane = (size_t)nx * (size_t)ny, n = 4 * plane, first = (size_t)(sm.b - 2) * plane;
+  Scratch<float> score(sm.ctx, n), mask, tensor(sm.ctx, 6 * n);
+  {
+    StageTimer t(sm.ctx, "h2d");
+    VCK(cudaMemcpyAsync(score.get(), out_host + first, n * sizeof(float), cudaMemcpyHostToDevice, sm.ctx->stream));
+    if (mask_host) {
+      mask.reset(sm.ctx, n);
+      VCK(cudaMemcpyAsync(mask.get(), mask_host + first, n * sizeof(float), cudaMemcpyHostToDevice, sm.ctx->stream));
+    }
+    VCK(cudaMemcpyAsync(tensor.get(), sm.tensor_below, 3 * n * sizeof(float), cudaMemcpyHostToDevice,
+                        sm.ctx->stream));
+    VCK(cudaMemcpyAsync(tensor.get() + 3 * n, sm.tensor_above, 3 * n * sizeof(float), cudaMemcpyHostToDevice,
+                        sm.ctx->stream));
+  }
+  flag_planes(sm.ctx, nx, ny, nz, 4, sm.b - 2, 1, 3, score.get(), mask.get(), tensor.get(), p, cn, nullptr);
+  resolve_stage_times(sm.ctx);
+}
+
+// The ordered flood over the flags of the whole image, on the calling thread, and the outputs of the call.  Its host
+// time goes to ctx's stage "flood".
+void connect_flood(Connect &cn, visfd_ctx *ctx, int64_t nx, int64_t ny, int64_t nz, const float *out_host) {
+  std::vector<float> maxima;
+  i64 n_max = 0;
+  const auto t0 = std::chrono::steady_clock::now();
+  const i64 nc = connect_flood_host(nx, ny, nz, out_host, cn.flags.get(), cn.direction,
+                                    cn.c.consider_dot_product_sign == 0, cn.c.threshold_saliency, cn.labels, &maxima,
+                                    &n_max);
+  ctx->stage_ms["flood"] += std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+  if (cn.n_clusters) *cn.n_clusters = nc;
+  if (cn.n_maxima) *cn.n_maxima = n_max;
+  if (cn.maxima && cn.capacity > 0)
+    std::copy(maxima.begin(), maxima.begin() + 3 * std::min<i64>(nc, cn.capacity), cn.maxima);
+}
+
+// cn: -connect, or NULL for the membrane pipeline alone.
 int membrane_multi(const char *name, int ndev, const int *devices, int64_t nx, int64_t ny, int64_t nz,
                    const float *src_host, const float *mask_host, const visfd_membrane_params *p,
                    float background_sigma, int normalize, float *out_host, float *threshold_out,
-                   double *device_ms) {
+                   double *device_ms, Connect *cn = nullptr) {
   try {
     const std::string who(name);
     VREQUIRE(ndev >= 1 && devices, who + ": need at least one device");
@@ -354,10 +519,18 @@ int membrane_multi(const char *name, int ndev, const int *devices, int64_t nx, i
         summed_own_hist(slabs, concurrently, plane, mask_host != nullptr, prefix, prefix_bits, hist);
       });
 
+    if (cn) cn->flags.reset(new uint16_t[plane * (size_t)nz]);
     for_each_slab(name, slabs, [&](Slab &s) {
-      vote_to_host(s, nx, ny, nz, threshold, p, out_host);
+      if (cn) vote_and_flag(s, nx, ny, nz, threshold, p, out_host, *cn);
+      else vote_to_host(s, nx, ny, nz, threshold, p, out_host);
       s.clock.end(s.ctx->stream);
     });
+    if (cn) {
+      std::vector<Seam> seams = seams_of(slabs);
+      if (!seams.empty())
+        for_each_slab(name, seams, [&](Seam &sm) { seam_flags(sm, nx, ny, nz, out_host, mask_host, p, *cn); });
+      connect_flood(*cn, slabs[0].ctx, nx, ny, nz, out_host);
+    }
 
     if (threshold_out) *threshold_out = threshold;
     if (device_ms)
@@ -371,7 +544,8 @@ int membrane_multi(const char *name, int ndev, const int *devices, int64_t nx, i
 
 int membrane_stream(const char *name, visfd_ctx *ctx, int64_t nx, int64_t ny, int64_t nz, const float *src_host,
                     const float *mask_host, const visfd_membrane_params *p, float background_sigma, int normalize,
-                    int64_t device_bytes, float *out_host, float *threshold_out, int64_t *n_slabs_out) {
+                    int64_t device_bytes, float *out_host, float *threshold_out, int64_t *n_slabs_out,
+                    Connect *cn = nullptr) {
   try {
     const std::string who(name);
     VREQUIRE(ctx != nullptr, who + ": context is NULL");
@@ -387,7 +561,7 @@ int membrane_stream(const char *name, visfd_ctx *ctx, int64_t nx, int64_t ny, in
 
     auto fewest = [&](bool vote_pass, uint64_t voters, size_t *need) {
       return fewest_slabs(nz, gauss_hw, tv_hw, bg.hw, budget, [&](const SlabPlan &pl) {
-        return slab_bytes(pl, nx, ny, masked, p, gauss_hw, bg, vote_pass, voters);
+        return slab_bytes(pl, nx, ny, masked, p, gauss_hw, bg, vote_pass, voters, cn && vote_pass);
       }, need);
     };
     // Runs step(slab) on every slab in turn, each after step (1) and each released before the next.
@@ -436,10 +610,19 @@ int membrane_stream(const char *name, visfd_ctx *ctx, int64_t nx, int64_t ny, in
     if (n_vote == 0) throw too_small(who, "the vote pass", need, budget);
     std::vector<Slab> slabs((size_t)n_vote);
     make_slabs(slabs, make_plans(nz, n_vote, gauss_hw, tv_hw, bg.hw), ctx);
+    if (cn) cn->flags.reset(new uint16_t[plane * (size_t)nz]);
     one_by_one(slabs, [&](Slab &s) {
       release_cache(ctx);   // the ridge step's scratch
-      vote_to_host(s, nx, ny, nz, threshold, p, out_host);
+      if (cn) vote_and_flag(s, nx, ny, nz, threshold, p, out_host, *cn);
+      else vote_to_host(s, nx, ny, nz, threshold, p, out_host);
     });
+    if (cn) {
+      for (const Seam &sm : seams_of(slabs)) {
+        seam_flags(sm, nx, ny, nz, out_host, mask_host, p, *cn);
+        release_cache(ctx);
+      }
+      connect_flood(*cn, ctx, nx, ny, nz, out_host);
+    }
 
     if (threshold_out) *threshold_out = threshold;
     if (n_slabs_out) *n_slabs_out = n_vote;
@@ -948,6 +1131,54 @@ extern "C" int visfd_cuda_membrane_stream_background(visfd_ctx *ctx, int64_t nx,
   return membrane_stream("visfd_cuda_membrane_stream_background", ctx, nx, ny, nz, src_host, mask_host, p,
                          background_sigma, normalize_near_boundaries, device_bytes, out_host, threshold_out,
                          n_slabs_out);
+}
+
+extern "C" int visfd_cuda_membrane_connect_multi(int ndev, const int *devices, int64_t nx, int64_t ny, int64_t nz,
+                                                 const float *src_host, const float *mask_host,
+                                                 const visfd_membrane_params *p, float background_sigma,
+                                                 int normalize_near_boundaries, const visfd_connect_params *c,
+                                                 float *out_host, float *threshold_out, int64_t *labels_host,
+                                                 float *direction_host, int64_t *n_clusters, float *cluster_maxima,
+                                                 int64_t maxima_capacity, int64_t *n_maxima, double *device_ms) {
+  const char *name = "visfd_cuda_membrane_connect_multi";
+  try {
+    VREQUIRE(ndev >= 1 && devices, std::string(name) + ": need at least one device");
+    Connect cn = connect_args(name, nx, ny, nz, src_host, p, background_sigma, c, out_host, labels_host,
+                              direction_host, maxima_capacity);
+    cn.n_clusters = n_clusters;
+    cn.n_maxima = n_maxima;
+    cn.maxima = cluster_maxima;
+    return membrane_multi(name, ndev, devices, nx, ny, nz, src_host, mask_host, p, background_sigma,
+                          normalize_near_boundaries, out_host, threshold_out, device_ms, &cn);
+  } catch (const std::exception &ex) {
+    set_last_error(ex.what());
+    return 1;
+  }
+}
+
+extern "C" int visfd_cuda_membrane_connect_stream(visfd_ctx *ctx, int64_t nx, int64_t ny, int64_t nz,
+                                                  const float *src_host, const float *mask_host,
+                                                  const visfd_membrane_params *p, float background_sigma,
+                                                  int normalize_near_boundaries, const visfd_connect_params *c,
+                                                  int64_t device_bytes, float *out_host, float *threshold_out,
+                                                  int64_t *labels_host, float *direction_host, int64_t *n_clusters,
+                                                  float *cluster_maxima, int64_t maxima_capacity, int64_t *n_maxima,
+                                                  int64_t *n_slabs_out) {
+  const char *name = "visfd_cuda_membrane_connect_stream";
+  try {
+    // the arguments are checked before the context is used
+    Connect cn = connect_args(name, nx, ny, nz, src_host, p, background_sigma, c, out_host, labels_host,
+                              direction_host, maxima_capacity);
+    VREQUIRE(device_bytes >= 0, std::string(name) + ": negative device_bytes");
+    cn.n_clusters = n_clusters;
+    cn.n_maxima = n_maxima;
+    cn.maxima = cluster_maxima;
+    return membrane_stream(name, ctx, nx, ny, nz, src_host, mask_host, p, background_sigma, normalize_near_boundaries,
+                           device_bytes, out_host, threshold_out, n_slabs_out, &cn);
+  } catch (const std::exception &ex) {
+    set_last_error(ex.what());
+    return 1;
+  }
 }
 
 extern "C" int visfd_cuda_blob_dog_multi(int ndev, const int *devices, int64_t nx, int64_t ny, int64_t nz,
